@@ -19,8 +19,12 @@ the samples are independent systems on a replicated mesh).
   cpu_baseline  oracle/fem_port.c (C restatement, OpenMP over samples) on a bounded sample, rank 0, N=1
   --impl reference  times that CPU port alone (the reference is pure Python and cannot run n=1e5:
              dense K would be 80 GB — BASELINE.md §2)
+  --dump-outputs DIR  after the timed steps, write what the last timed step returned to its caller as DIR/<name>.npy
+             (float64, at most 64 MB in all; see dump_outputs).  The inputs are seeded, so two builds run with the same
+             arguments can be compared file by file.
 
 Inputs per array are 3.28 GB (>> 126 MB L2), so no L2 flush is needed between iterations.
+bench.py writes nothing into the source tree (it may be read-only): it loads the library build() compiled.
 """
 from __future__ import annotations
 
@@ -37,6 +41,7 @@ import numpy as np
 
 ROOT = pathlib.Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True            # no __pycache__ for the project modules imported below: the tree stays untouched
 
 WORKLOADS = {
     # name: (n_elements, batch per rank, kappa layout, scaling)
@@ -70,7 +75,14 @@ def parse():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-sweep", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float64, at most 64 MB in all)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    return args
 
 
 def measured_peak():
@@ -375,11 +387,37 @@ def parity_block_small2d(mesh, rows, f, kappa, gbar, u, gf):
             "tolerance": 1e-9, "oracle": "oracle/oracle.py (sparse LU + refinement of the same float64 system)"}
 
 
-def time_sweep(args, rank, world, dev, n_el, B_total, steps, warmup):
+DUMP_BYTES = 64 * 10 ** 6                   # --dump-outputs: all files together, .npy headers included
+
+
+def dump_outputs(out_dir, whole, batched=None):
+    """--dump-outputs: write the arrays the last timed step returned to its caller as <out_dir>/<name>.npy (float64).
+
+    `whole` arrays are written entire.  `batched` arrays hold one row per sample; when they do not fit the budget left by
+    `whole`, every one of them keeps the same rows: as many as fit, drawn with a fixed seed and sorted ascending.  The
+    sample depends on the shapes alone, so runs with the same arguments write the same rows.  Only rank 0 dumps."""
+    import torch
+
+    out = {k: v.detach().double().cpu().numpy() for k, v in whole.items()}
+    if batched:
+        B = next(iter(batched.values())).shape[0]
+        room = DUMP_BYTES - sum(a.nbytes for a in out.values()) - 4096 * (len(out) + len(batched))   # 4 KiB per header
+        n = min(B, room // sum(8 * (v.numel() // B) for v in batched.values()))
+        rows = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+        idx = torch.from_numpy(rows).to(next(iter(batched.values())).device)
+        out.update({k: v.detach()[idx].double().cpu().numpy() for k, v in batched.items()})
+    d = pathlib.Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for k, a in out.items():
+        np.save(d / f"{k}.npy", a)
+
+
+def time_sweep(args, rank, world, dev, n_el, B_total, steps, warmup, dump_dir=None):
     """BASELINE config 5a as SURVEY §8(d) defines it: 65 536 samples on line(16384), shared kappa, sharded over the
     ranks (strong scaling); per step  forward -> fused misfit adjoint (gbar = 2 (u - u_data) / n formed in the kernel,
     [sum dL/dkappa, sum loss] written into the persistent reduction buffer) -> ONE NCCL all-reduce of 16 bytes -> Adam
-    step replicated on every rank (examples/poisson_1d_demo.py:104-110, batched)."""
+    step replicated on every rank (examples/poisson_1d_demo.py:104-110, batched).  With `dump_dir`, the last step's
+    loss, dL/dkappa and updated kappa go there (dump_outputs)."""
     import torch
     import torch.distributed as dist
 
@@ -426,6 +464,8 @@ def time_sweep(args, rank, world, dev, n_el, B_total, steps, warmup):
         barrier()
     ms_total = e0.elapsed_time(e1)
     ksum = kt.summary()
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, {"loss": last, "grad_kappa": kappa.grad, "kappa": kappa})
     if world > 1:
         t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -472,7 +512,9 @@ def run_b200(args):
     if world > 1:
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=dev)
-    _native.build()
+    if _native.needs_build():
+        print("bench.py: libdfe_b200.so is older than its sources; run __graft_entry__.build() to rebuild it", file=sys.stderr)
+    _native.lib()
 
     w = dict(WORKLOADS[args.workload])
     if w.get("small"):
@@ -534,6 +576,10 @@ def run_b200(args):
         ms_total = float(t[0])
     ms_step = ms_total / args.steps
     value = B * world * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        whole, batched = {}, {"u": keep["u"], "grad_f": f.grad}
+        (batched if per_elem else whole)["grad_kappa"] = keep["gk"]
+        dump_outputs(args.dump_outputs, whole, batched)
 
     # ---------------- parity of the timed output (rank 0): rows from the first / a middle / the last pipeline iteration
     parity = None
@@ -689,7 +735,8 @@ def run_b200_sweep(args, w, rank, local_rank, world, dev):
 
     sampler = ClockSampler(local_rank)
     sampler.start()
-    r = time_sweep(args, rank, world, dev, args.n_elements or w["n_elements"], args.batch or w["batch"], args.steps, args.warmup)
+    r = time_sweep(args, rank, world, dev, args.n_elements or w["n_elements"], args.batch or w["batch"], args.steps, args.warmup,
+                   dump_dir=args.dump_outputs)
     clocks = sampler.stop()
     peak, peak_src = measured_peak()
     cpu = None
@@ -781,6 +828,8 @@ def run_b200_2d(args, w, rank, local_rank, world, dev):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms_total = float(t[0])
     ms_step = ms_total / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"u": its["u"], "grad_kappa": its["gk"]})
     parity = None
     if rank == 0 and not args.no_parity:
         try:
@@ -928,7 +977,7 @@ def run_b200_small2d(args, w, rank, local_rank, world, dev):
     with KernelTimer() as kt:
         e0.record()
         for _ in range(args.steps):
-            step()
+            gk_last = step()
         e1.record()
         barrier()
     clocks = sampler.stop()
@@ -940,6 +989,8 @@ def run_b200_small2d(args, w, rank, local_rank, world, dev):
         ms_total = float(t[0])
     ms_step = ms_total / args.steps
     value = B * world * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"grad_kappa": gk_last}, {"u": its["u"], "grad_f": f.grad})
     parity = None
     u_last = its.pop("u", None)
     if rank == 0 and not args.no_parity and u_last is not None:

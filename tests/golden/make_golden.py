@@ -1,10 +1,10 @@
 """Generate golden vectors by running the UNMODIFIED reference implementation.
 
-Run in the build container only (needs /root/reference, which does not exist on
-the GPU box):
+Needs a checkout of the original DiffFE-Physics-Lab (the directory that holds its ``diffhe`` package); the tests
+only read the stored vectors:
 
-    python tests/golden/make_golden.py            # small cases  (~1-2 min)
-    python tests/golden/make_golden.py --big      # + 2D 64x64 / 128x128 forward (~3 min, ~7 GB RAM)
+    python tests/golden/make_golden.py --reference DIR          # small cases  (~1-2 min)
+    python tests/golden/make_golden.py --reference DIR --big    # + 2D 64x64 / 128x128 forward (~3 min, ~7 GB RAM)
 
 Outputs ``tests/golden/ref_small.npz`` and ``tests/golden/ref_big.npz``.  Every
 array is float64/int64 stored bit-exactly.  Keys are ``<case>/<field>``.
@@ -18,8 +18,11 @@ import sys
 import numpy as np
 import torch
 
-REF = "/root/reference"
-sys.path.insert(0, REF)
+ap = argparse.ArgumentParser()
+ap.add_argument("--reference", required=True, help="checkout of the original DiffFE-Physics-Lab")
+ap.add_argument("--big", action="store_true")
+a = ap.parse_args()
+sys.path.insert(0, a.reference)
 from diffhe.mesh import FEMesh  # noqa: E402  (reference)
 from diffhe.solver import DifferentiableFESolver  # noqa: E402  (reference)
 
@@ -153,9 +156,6 @@ def big():
 
 
 if __name__ == "__main__":
-    ap = argparse.ArgumentParser()
-    ap.add_argument("--big", action="store_true")
-    a = ap.parse_args()
     if a.big:
         big()
     else:

@@ -9,7 +9,9 @@ pytestmark = pytest.mark.gpu
 
 
 @pytest.fixture(scope="module", autouse=True)
-def _built():
+def _need_gpu():
+    if not torch.cuda.is_available():
+        pytest.skip("no CUDA device")
     _native.build()
 
 
