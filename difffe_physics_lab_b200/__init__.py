@@ -9,6 +9,7 @@ from .mesh import FEMesh
 from .solver import DifferentiableFESolver, assemble_sparse
 from .loss import PhysicsLoss
 from .neural import NeuralPDE
+from .timestepping import DifferentiableHeatSolver
 
 __version__ = "0.1.0"
-__all__ = ["FEMesh", "DifferentiableFESolver", "PhysicsLoss", "NeuralPDE", "assemble_sparse"]
+__all__ = ["FEMesh", "DifferentiableFESolver", "PhysicsLoss", "NeuralPDE", "assemble_sparse", "DifferentiableHeatSolver"]

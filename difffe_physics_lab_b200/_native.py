@@ -20,7 +20,7 @@ PKG = pathlib.Path(__file__).resolve().parent
 ROOT = PKG.parent
 LIB_PATH = PKG / "libdfe_b200.so"
 SOURCES = ["dfe_mesh.cu", "dfe_1d.cu", "dfe_1d_split.cu", "dfe_1d_pipe.cu", "dfe_general.cu", "dfe_pcg.cu", "dfe_mg.cu",
-           "dfe_batch.cu"]
+           "dfe_batch.cu", "dfe_heat.cu"]
 HEADERS = [PKG / "csrc" / "dfe_internal.h", PKG / "csrc" / "dfe_1d_common.cuh", PKG / "csrc" / "dfe_gridsync.cuh", PKG / "csrc" / "dfe_exact.cuh",
            PKG / "csrc" / "dfe_p2.cuh", PKG / "csrc" / "dfe_mg_kernel.cuh", ROOT / "include" / "dfe.h"]
 
@@ -39,6 +39,8 @@ SYMBOLS = [
     "dfe_batch_supported", "dfe_batch_fwd", "dfe_batch_bwd",
     "dfe_band_supported", "dfe_band_factor_bytes", "dfe_band_workspace_bytes", "dfe_band_factor", "dfe_band_fwd", "dfe_band_bwd",
     "dfe_band_npad", "dfe_band_solve",
+    "dfe_heat_supported", "dfe_heat_warps", "dfe_heat_grad_bytes", "dfe_heat_fwd", "dfe_heat_adj", "dfe_heat_grad",
+    "dfe_heat_grad_sum",
 ]
 
 
@@ -211,6 +213,20 @@ def lib() -> C.CDLL:
     L.dfe_band_npad.argtypes = [vp]
     L.dfe_band_solve.restype = ci
     L.dfe_band_solve.argtypes = [vp, i64, vp, vp, vp]
+    L.dfe_heat_supported.restype = ci
+    L.dfe_heat_supported.argtypes = [vp]
+    L.dfe_heat_warps.restype = ci
+    L.dfe_heat_warps.argtypes = [vp, i64]
+    L.dfe_heat_grad_bytes.restype = sz
+    L.dfe_heat_grad_bytes.argtypes = [vp, i64, i64]
+    L.dfe_heat_fwd.restype = ci
+    L.dfe_heat_fwd.argtypes = [vp, i64, i64, vp, i64, vp, vp, vp, vp, vp, i64, i64, ci, vp, vp]
+    L.dfe_heat_adj.restype = ci
+    L.dfe_heat_adj.argtypes = [vp, i64, i64, i64, vp, i64, i64, i64, vp, vp, vp, vp, vp, ci, vp, vp]
+    L.dfe_heat_grad.restype = ci
+    L.dfe_heat_grad.argtypes = [vp, i64, i64, i64, i64, vp, i64, i64, vp, vp, sz, vp]
+    L.dfe_heat_grad_sum.restype = ci
+    L.dfe_heat_grad_sum.argtypes = [vp, i64, i64, dbl, ci, vp, vp, sz, vp]
     if L.dfe_abi_version() != 1:
         raise RuntimeError("libdfe_b200.so ABI version mismatch")
     _lib = L

@@ -1156,7 +1156,7 @@ __global__ void __launch_bounds__(128) k_band_solve(int npad, long long B, const
 // operands agree: k-step (tile nt', half j) is DEFINED to cover the columns 8nt' + 2(t%4) + j, which are exactly the
 // accumulator registers the thread already holds.  The B fragments are stored with the matching permutation, and the
 // result of one block row feeds the next one without a single shuffle or shared-memory round trip.
-constexpr int FRAGD = 2048;   // doubles per block row and direction: H fragments (1024), then -S fragments (1024)
+constexpr int FRAGD = dfe::BAND_FRAGD;   // doubles per block row and direction: H fragments (1024), then -S fragments (1024)
 constexpr int MMA_W = 8;      // warps per CTA of the solve kernel
 constexpr int MMA_S = 16;     // samples per warp (two m8 tiles)
 
@@ -1684,6 +1684,12 @@ bool band_fused_io() {
   return !off;
 }
 }  // namespace
+
+void dfe::band_frags(const dfe_mesh* m, const void* factor, const double** Ff, const double** Bf) {
+  const BandPtrs p = band_ptrs(m, const_cast<void*>(factor));
+  *Ff = p.Ff;
+  *Bf = p.Bf;
+}
 
 // K_free = L L^T from the assembled matrix (dfe_assemble); `factor` holds dfe_band_factor_bytes(m) bytes.  The status
 // word (0 ok, 5 = a pivot <= 0: K_free is not SPD) is the int at the end of the buffer; *status_dev (optional, device)

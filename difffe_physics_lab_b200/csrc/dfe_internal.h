@@ -71,6 +71,11 @@ struct Misfit1D {
 int poison1d_launch(const dfe_mesh* m, double* out, long long ldo, long long B, int nn, double* gk, long long ngk,
                     double* loss, long long nloss, cudaStream_t st);
 
+// banded factor of dfe_band_factor (dfe_batch.cu): the DMMA B-operand fragments of the block TRSM, BAND_FRAGD doubles per
+// block row — Ff (forward: H_k, then -S_k) and Bf (backward: H_k^T, then -S_{k+1}^T), both 16-byte aligned
+constexpr int BAND_FRAGD = 2048;
+void band_frags(const dfe_mesh* m, const void* factor, const double** Ff, const double** Bf);
+
 }  // namespace dfe
 
 struct dfe_mesh {

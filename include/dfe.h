@@ -249,6 +249,46 @@ int dfe_band_bwd(const dfe_mesh* m, int64_t B, const double* gbar, int64_t ldg, 
 int64_t dfe_band_npad(const dfe_mesh* m);
 int dfe_band_solve(const dfe_mesh* m, int64_t B, double* X, const void* factor, void* stream);
 
+/* ---------------------------------------------------------------- differentiable heat-equation rollouts
+ * Backward Euler with the lumped mass, (M_L + dt K) u^{n+1} = M_L u^n + dt F, Dirichlet nodes held at the mesh's values,
+ * for B states sharing one factor of A = M_L + dt K (dfe_band_factor), and its discrete adjoint.  In free numbering,
+ *   forward   A_ff x_{n+1} = m * x_n + c                     m = M_L[free], c = dt F_free - (A g)_free
+ *   adjoint   A_ff lambda_n = gbar_n + m * lambda_{n+1}        lambda_{N+1} = 0
+ *   dL/du0[free] = m * lambda_1,   dL/dkappa_e = -dt sum_n sum_b lam~_n^T K0_e u_n,   dL/df = W^T (dt sum_n sum_b lam~_n)
+ * (lam~: lambda with zeros on the Dirichlet nodes; W: the load operator, dfe_grad's gf).  Each rollout call is ONE launch
+ * of a block-TRSM kernel (FP64 tensor cores) with the time loop inside; results do not depend on `warps`.
+ *   dfe_heat_supported   1 for 2-D P1 meshes with dfe_band_supported and a gradient kernel that fits shared memory
+ *   dfe_heat_warps       warps per CTA (16 states each) the rollout kernels choose for B states (0 if unsupported)
+ *   dfe_heat_fwd         n_steps steps.  u0 (B, .) node layout with row stride ldu0, or NULL: X already holds x_0.
+ *                        X (B, npad) free-layout carry (dfe_band_npad), holds x_{n_steps} on return; the state after step
+ *                        j (0-based) is written to traj + b * ld_b + j * ld_t in node layout, Dirichlet values included.
+ *                        m_free / c_free: (npad), zero beyond n_free.
+ *   dfe_heat_adj         steps n0 + n_steps down to n0 + 1.  X (B, npad) carries lambda_{n+1} in and lambda_{n0+1} out
+ *                        (zero it before step N); gbar (B, R, n_nodes)-like with strides ldg_b / ldg_t holds dL/du_n for
+ *                        n % g_every == 0 at slot n / g_every - 1 (NULL: no loss term in this range); lam (n_steps, B, npad)
+ *                        receives lambda_{n0+1+j} at slot j; lam_sum (B, npad) += lambda_n in step order.
+ *   dfe_heat_grad        per-step partial sums of lam~^T K0_e u for steps n0+1 .. n0+n_seg (u: state of step n0+1+j of
+ *                        sample b at u + b * ld_b + j * ld_t; lam as written by dfe_heat_adj) into ws, which holds
+ *                        dfe_heat_grad_bytes(m, B, n_total) bytes for the whole rollout of n_total steps.
+ *   dfe_heat_grad_sum    dL/dkappa from the partials of all n_total steps, added in a fixed step order (independent of how
+ *                        the rollout was split): PER_ELEMENT -> gkappa[n_el], SCALAR -> gkappa[1].
+ *   fault (device int32): set to 1 if a bounded wait inside a rollout kernel expired; the outputs are then invalid.
+ * X, m_free, c_free, lam and lam_sum must be 16-byte aligned.  All calls are asynchronous on `stream`.
+ */
+int dfe_heat_supported(const dfe_mesh* m);
+int dfe_heat_warps(const dfe_mesh* m, int64_t B);
+size_t dfe_heat_grad_bytes(const dfe_mesh* m, int64_t B, int64_t n_total);
+int dfe_heat_fwd(const dfe_mesh* m, int64_t B, int64_t n_steps, const double* u0, int64_t ldu0, const void* factor,
+                 const double* m_free, const double* c_free, double* X, double* traj, int64_t ld_b, int64_t ld_t,
+                 int warps, int32_t* fault, void* stream);
+int dfe_heat_adj(const dfe_mesh* m, int64_t B, int64_t n0, int64_t n_steps, const double* gbar, int64_t ldg_b,
+                 int64_t ldg_t, int64_t g_every, const void* factor, const double* m_free, double* X, double* lam,
+                 double* lam_sum, int warps, int32_t* fault, void* stream);
+int dfe_heat_grad(const dfe_mesh* m, int64_t B, int64_t n0, int64_t n_seg, int64_t n_total, const double* u, int64_t ld_b,
+                  int64_t ld_t, const double* lam, void* ws, size_t ws_bytes, void* stream);
+int dfe_heat_grad_sum(const dfe_mesh* m, int64_t B, int64_t n_total, double dt, int kappa_mode, double* gkappa, void* ws,
+                      size_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
