@@ -22,7 +22,8 @@ LIB_PATH = PKG / "libdfe_b200.so"
 SOURCES = ["dfe_mesh.cu", "dfe_1d.cu", "dfe_1d_split.cu", "dfe_1d_pipe.cu", "dfe_general.cu", "dfe_pcg.cu", "dfe_mg.cu",
            "dfe_batch.cu", "dfe_heat.cu"]
 HEADERS = [PKG / "csrc" / "dfe_internal.h", PKG / "csrc" / "dfe_1d_common.cuh", PKG / "csrc" / "dfe_gridsync.cuh", PKG / "csrc" / "dfe_exact.cuh",
-           PKG / "csrc" / "dfe_p2.cuh", PKG / "csrc" / "dfe_mg_kernel.cuh", ROOT / "include" / "dfe.h"]
+           PKG / "csrc" / "dfe_p2.cuh", PKG / "csrc" / "dfe_mg_kernel.cuh", PKG / "csrc" / "dfe_band_mma.cuh",
+           ROOT / "include" / "dfe.h"]
 
 OK, ERR_INVALID, ERR_CUDA, ERR_UNSUPPORTED, ERR_NOT_CONVERGED, ERR_BREAKDOWN, ERR_WORKSPACE = range(7)
 KAPPA_SCALAR, KAPPA_PER_SAMPLE, KAPPA_PER_ELEMENT, KAPPA_PER_SAMPLE_ELEMENT = range(4)

@@ -20,6 +20,7 @@ namespace {
 
 using dfe::MeshDev;
 #include "dfe_1d_common.cuh"        // mbarrier / 1-D TMA bulk copy wrappers (used by the tensor-core band solve)
+#include "dfe_band_mma.cuh"         // block-row step of the tensor-core band solve and its fragment layout
 #include "dfe_exact.cuh"            // div3: correctly rounded x / 3.0 without the division instruction
 
 constexpr double AREA_EPS = 1e-15;  // solver.py:120
@@ -315,16 +316,13 @@ __global__ void __launch_bounds__(BT, (RPT <= 4 ? 2 : 1)) k_batch(const BArgs A)
 // =====================================================================================================================
 // Banded direct solver for the same job when the half bandwidth of K_free is <= 32 (rectangle(nx, ny) with nx <= 32
 // in the reference's node numbering): K_free = L L^T once per call (the batch shares the matrix), then two banded
-// triangular solves per sample.  That is ~13x fewer flops than ~120 Jacobi-PCG iterations at 961 unknowns and has
-// no reductions: a WARP owns BS samples, lane k holds the pending right-hand side of the rows = k (mod 32) of the
-// sliding 32-row window, and a step is  y = W[head] / L_ii  (one shuffle),  W -= L[.., i] y  (one coalesced 256 B
-// load of the column shared by the BS samples, one fma per sample).  Replaces solver.py:174 (LU with partial
+// triangular solves per sample (a block TRSM on the FP64 tensor cores, k_band_solve_mma).  That is ~13x fewer flops
+// than ~120 Jacobi-PCG iterations at 961 unknowns and has no reductions.  Replaces solver.py:174 (LU with partial
 // pivoting on the dense K_free) more literally than PCG does.
-constexpr int BW = 32;   // half bandwidth supported: one lane per sub-diagonal
-constexpr int BS = 8;    // samples per warp (the factor is loaded once per BS samples: its L2 -> SM traffic is the bound)
+constexpr int BW = 32;   // half bandwidth supported
 
 // Lower band of K_free, Ab[r * 33 + k] = K_free[r][r - k] (k = 0..32), scattered from the assembled matrix in parallel.
-// Rows n_free .. n_free + 34 are zero (the factor kernel prefetches past the end).
+// Rows n_free and beyond are zero.
 __global__ void k_band_gather(const MeshDev M, const double* __restrict__ vals_full, double* __restrict__ Ab) {
   const int r = blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= M.n_free) return;
@@ -334,90 +332,19 @@ __global__ void k_band_gather(const MeshDev M, const double* __restrict__ vals_f
   }
 }
 
-// One CTA: right-looking banded Cholesky with the active (BW+1) x (BW+1) window in shared memory; the row that enters
-// the window at step j is prefetched from Ab two steps earlier (one global latency per step would otherwise be the
-// critical path of the whole factorisation).
-//   invd[i] = 1 / L_ii,  Lc[i*32 + d-1] = L[i+d][i],  Lr[i*32 + d-1] = L[i][i-d]   (d = 1..32; rows >= n: identity)
-__global__ void __launch_bounds__(256) k_band_factor(int n, int npad, const double* __restrict__ Ab,
-                                                     double* __restrict__ invd, double* __restrict__ Lc,
-                                                     double* __restrict__ Lr, int* __restrict__ status) {
-  __shared__ double sA[BW + 1][BW + 2];   // sA[r % 33][k] = A[r][r-k], rows j..j+32 of the trailing matrix
-  __shared__ double sl[BW + 1];
-  __shared__ double sd0[BW + 1];          // diagonal entries of the window's rows before elimination
-  __shared__ int sbad;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  for (int i = n + tid; i < npad; i += 256) invd[i] = 1.0;
-  if (tid == 0) sbad = 0;
-  for (int q = tid; q < (BW + 1) * (BW + 1); q += 256) {   // rows 0..32
-    const int r = q / (BW + 1), k = q - r * (BW + 1);
-    const double v = Ab[static_cast<size_t>(r) * (BW + 1) + k];
-    sA[r][k] = v;
-    if (k == 0) sd0[r] = v;
-  }
-  // warp 0 keeps the next two incoming rows in registers (lane k holds entry k, lane 0 also entry 32)
-  double pa = 0.0, pa32 = 0.0, pb = 0.0, pb32 = 0.0;
-  if (warp == 0) {
-    pa = Ab[static_cast<size_t>(BW + 1) * (BW + 1) + lane];
-    pb = Ab[static_cast<size_t>(BW + 2) * (BW + 1) + lane];
-    if (lane == 0) {
-      pa32 = Ab[static_cast<size_t>(BW + 1) * (BW + 1) + BW];
-      pb32 = Ab[static_cast<size_t>(BW + 2) * (BW + 1) + BW];
-    }
-  }
-  __syncthreads();
-  for (int j = 0; j < n; ++j) {
-    const int sj = j % (BW + 1);
-    const double d = sA[sj][0];
-    // SPD check: a pivot that lost 12 digits against its diagonal entry means K_free is (numerically) singular — the
-    // reference returns garbage silently there (SURVEY §5), this library reports a breakdown
-    const bool ok = d > 1e-12 * sd0[sj];
-    const double inv = ok ? rsqrt(d) : 1.0;
-    if (!ok && tid == 0) sbad = 1;
-    if (tid == 0) invd[j] = inv;
-    double pc = 0.0, pc32 = 0.0;
-    if (warp == 0) {   // prefetch row j + 35 (consumed at step j + 2)
-      pc = Ab[static_cast<size_t>(j + BW + 3) * (BW + 1) + lane];
-      if (lane == 0) pc32 = Ab[static_cast<size_t>(j + BW + 3) * (BW + 1) + BW];
-    }
-    if (tid >= 1 && tid <= BW) {
-      const int a = tid, r = j + a;
-      const double l = r < n ? sA[r % (BW + 1)][a] * inv : 0.0;
-      sl[a] = l;
-      Lc[static_cast<size_t>(j) * BW + a - 1] = l;
-      if (r < n) Lr[static_cast<size_t>(r) * BW + a - 1] = l;
-    }
-    __syncthreads();
-    // warps 1..7: A[j+a][j+b] -= l_a l_b, 1 <= b <= a <= 32; warp 0 meanwhile puts row j+33 into the slot of row j
-    // (whose pivot was read before the barrier; the update never touches that slot)
-    if (warp == 0) {
-      sA[sj][lane] = pa;
-      if (lane == 0) { sA[sj][BW] = pa32; sd0[sj] = pa; }
-      pa = pb; pa32 = pb32;
-      pb = pc; pb32 = pc32;
-    } else {
-      for (int q = tid - 32; q < BW * BW; q += 224) {
-        const int a = (q >> 5) + 1, b = (q & 31) + 1;
-        if (b <= a && j + a < n) sA[(j + a) % (BW + 1)][a - b] -= sl[a] * sl[b];
-      }
-    }
-    __syncthreads();
-  }
-  if (tid == 0) *status = sbad ? 5 : 0;
-}
-
-// Blocked variant of the factorisation (default).  k_band_factor above pays ~1500 cycles for each of its n dependent
-// pivot steps (two CTA barriers, a shared-memory round trip and a double-precision rsqrt per step: 0.72 ms at 961 unknowns —
-// 18 % of a config-5b step and, replicated on every rank, the part that does not scale over GPUs).  With 32 x 32 blocks the
-// band is block tridiagonal:
+// K_free = L L^T in ONE CTA, blocked.  (Round 1 factored row by row: ~1500 cycles for each of the n dependent pivot steps
+// — two CTA barriers, a shared-memory round trip and a double-precision rsqrt per step: 0.72 ms at 961 unknowns, 18 % of a
+// config-5b step and, replicated on every rank, the part that does not scale over GPUs.)  With 32 x 32 blocks the band is
+// block tridiagonal:
 //     L_kk L_kk^T = A_kk - L_{k,k-1} L_{k,k-1}^T,      L_{k+1,k} = A_{k+1,k} L_kk^{-T}.
 // The dense Cholesky of a diagonal block runs in ONE warp out of registers (lane i holds row i; pivots and multipliers
 // move by shuffles with compile-time register indices, no barrier and no shared-memory latency in the pivot chain), the
 // triangular solve for L_{k+1,k} in the same warp (lane a holds row a; L_kk is read from shared memory as broadcasts),
-// and the rank-32 update of the next diagonal block by the whole CTA — three CTA barriers per BLOCK instead of two per row.
-// Same outputs and the same pivot test as k_band_factor.
+// and the rank-32 update of the next diagonal block by the whole CTA — three CTA barriers per BLOCK.
+//   invd[i] = 1 / L_ii,  Lr[i*32 + d-1] = L[i][i-d]   (d = 1..32; rows >= n: identity)
 __global__ void __launch_bounds__(256) k_band_factor_blk(int n, int npad, const double* __restrict__ Ab,
-                                                         double* __restrict__ invd, double* __restrict__ Lc,
-                                                         double* __restrict__ Lr, int* __restrict__ status) {
+                                                         double* __restrict__ invd, double* __restrict__ Lr,
+                                                         int* __restrict__ status) {
   __shared__ double Ls[32][33];   // L_kk (lower triangle, diagonal included)
   __shared__ double Xs[32][33];   // L_{k+1,k}: Xs[a][b] = L[32(k+1)+a][32k+b] (zero for b < a)
   __shared__ double Ns[2][32][33];   // diagonal blocks k / k+1 (ping-pong): raw, then minus the rank-32 update (lower triangle)
@@ -499,13 +426,9 @@ __global__ void __launch_bounds__(256) k_band_factor_blk(int n, int npad, const 
       // ---- meanwhile: the factor entries inside the diagonal block
       for (int q = tid - 32; q < 1024; q += 224) {
         const int i = q >> 5, j = q & 31;
-        const size_t gi = static_cast<size_t>(32 * k + i), gj = static_cast<size_t>(32 * k + j);
+        const size_t gi = static_cast<size_t>(32 * k + i);
         if (i == j) invd[gi] = sinv[i];
-        if (i > j) {
-          const double l = Ls[i][j];
-          Lc[gj * BW + (i - j) - 1] = l;
-          Lr[gi * BW + (i - j) - 1] = l;
-        }
+        if (i > j) Lr[gi * BW + (i - j) - 1] = Ls[i][j];
       }
     }
     __syncthreads();   // [B3] Xs ready
@@ -518,12 +441,8 @@ __global__ void __launch_bounds__(256) k_band_factor_blk(int n, int npad, const 
           for (int c = 0; c < 32; ++c) acc = fma(-Xs[aa][c], Xs[b][c], acc);
           Ns[cur ^ 1][aa][b] = acc;
         }
-        if (b >= aa) {   // factor entries that cross the block boundary: row 32(k+1)+aa, column 32k+b
-          const double l = Xs[aa][b];
-          const size_t gr = static_cast<size_t>(32 * (k + 1) + aa), gc = static_cast<size_t>(32 * k + b);
-          Lc[gc * BW + (32 + aa - b) - 1] = l;
-          Lr[gr * BW + (32 + aa - b) - 1] = l;
-        }
+        if (b >= aa)   // factor entries that cross the block boundary: row 32(k+1)+aa, column 32k+b
+          Lr[static_cast<size_t>(32 * (k + 1) + aa) * BW + (32 + aa - b) - 1] = Xs[aa][b];
       }
     }
   }
@@ -560,15 +479,6 @@ __global__ void k_band_geom(const MeshDev M, double* __restrict__ geom) {
 }
 
 // right-hand sides of the whole batch, (B, npad) row-major, rows >= n_free zero.
-// adjoint: gbar restricted to the free rows (SURVEY A7)
-__global__ void k_band_rhs_bwd(const MeshDev M, long long B, int npad, const double* __restrict__ gbar, long long ldg,
-                               double* __restrict__ X) {
-  const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
-  if (idx >= B * npad) return;
-  const long long b = idx / npad;
-  const int r = static_cast<int>(idx - b * npad);
-  X[idx] = r < M.n_free ? gbar[b * ldg + M.free_nodes[r]] : 0.0;
-}
 // forward: one CTA per sample — f_b and the per-element terms (area/3) * (f_i+f_j+f_k)/3 (solver.py:143-145) in shared
 // memory, then every free row adds the terms of its adjacent elements in ascending element order and applies the
 // lifting in dict order (solver.py:165-169): the arithmetic of k_assemble / k_eliminate, bit for bit
@@ -928,19 +838,19 @@ __global__ void __launch_bounds__(512) k_band_rhs_fwd3(const MeshDev M, long lon
   cp_async_wait<0>();
 }
 
-// GF: dL/df = M_F lambda (streams the lambda rows);  GK: per-warp partials of lambda^T K^0 u (streams u and lambda rows).
-// Both in one kernel cost 96 registers at 576 threads (one CTA per SM, 0.86 ms at config 5b); as two kernels each half keeps
-// the weights of ONE stencil in registers and two CTAs fit an SM, but the lambda rows are streamed twice (0.54 + 0.39 ms):
-// the fused form is the default, an adjoint without dL/df launches the GK half only.
-template <bool GF, bool GK, int SPI, int NG>
-__global__ void __launch_bounds__(SBT_MAX, (GF && GK) ? 1 : 2) k_band_grad3(const MeshDev M, long long B, int npad, int nnp,
+// Per-warp partials of lambda^T K^0 u (streams the u and lambda rows) and, with GF, dL/df = M_F lambda in the same pass.
+// With GF the kernel costs 96 registers at 576 threads (one CTA per SM, 0.86 ms at config 5b); as two kernels each half
+// kept the weights of ONE stencil in registers and two CTAs fit an SM, but the lambda rows were streamed twice
+// (0.54 + 0.39 ms).  An adjoint without dL/df launches it without GF.
+template <bool GF, int SPI, int NG>
+__global__ void __launch_bounds__(SBT_MAX, GF ? 1 : 2) k_band_grad3(const MeshDev M, long long B, int npad, int nnp,
                                                         const double* __restrict__ X, const double* __restrict__ ufull,
                                                         long long ldu, const double* __restrict__ ellK,
                                                         const double* __restrict__ ellMr, const unsigned* __restrict__ ellc,
                                                         double* __restrict__ gkpart, double* __restrict__ gf, long long ldgf) {
-  extern __shared__ __align__(16) double sg[];   // [NG][SPI][(nnp + 2) + npad]: u row (GK only), lambda row (free numbering)
+  extern __shared__ __align__(16) double sg[];   // [NG][SPI][(nnp + 2) + npad]: u row, lambda row (free numbering)
   const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, warp = tid >> 5, nw = nt >> 5;
-  const int uoff = GK ? nnp + 2 : 0;       // u row (with room for its 16-byte phase) | lambda row
+  const int uoff = nnp + 2;                // u row (with room for its 16-byte phase) | lambda row
   const int pitch = uoff + npad;
   double wk[SR][SW], wm[SR][SW];
   unsigned c[SR][SW];
@@ -952,7 +862,7 @@ __global__ void __launch_bounds__(SBT_MAX, (GF && GK) ? 1 : 2) k_band_grad3(cons
     rk[k] = ex ? M.free_rank[p] : -1;
 #pragma unroll
     for (int j = 0; j < SW; ++j) {
-      wk[k][j] = (GK && ex) ? ellK[static_cast<size_t>(j) * nnp + p] : 0.0;
+      wk[k][j] = ex ? ellK[static_cast<size_t>(j) * nnp + p] : 0.0;
       wm[k][j] = (GF && ex) ? ellMr[static_cast<size_t>(j) * nnp + p] : 0.0;
       c[k][j] = ex ? ellc[static_cast<size_t>(j) * nnp + p] : 0u;
     }
@@ -967,7 +877,7 @@ __global__ void __launch_bounds__(SBT_MAX, (GF && GK) ? 1 : 2) k_band_grad3(cons
       const long long bb = b_in + s * bs;
       if (bb < B) {
         const uint32_t du = sg32 + 8u * ((st_in * SPI + s) * pitch);
-        if (GK) row_to_smem(du, ufull + bb * ldu, M.n_nodes, tid, nt);
+        row_to_smem(du, ufull + bb * ldu, M.n_nodes, tid, nt);
         const double* sl = X + bb * npad;      // 16-byte aligned rows (npad is a multiple of 32)
         for (int q = tid; q < (npad >> 1); q += nt) cp_async16_u32(du + 8u * uoff + 16u * q, sl + 2 * q);
       }
@@ -991,18 +901,16 @@ __global__ void __launch_bounds__(SBT_MAX, (GF && GK) ? 1 : 2) k_band_grad3(cons
 #pragma unroll
       for (int s = 0; s < SPI; ++s) {
         const long long bb = b + s * bs;
-        const double* ub = sg + (st * SPI + s) * pitch + (GK ? ((reinterpret_cast<uintptr_t>(ufull + bb * ldu) >> 3) & 1) : 0);
+        const double* ub = sg + (st * SPI + s) * pitch + ((reinterpret_cast<uintptr_t>(ufull + bb * ldu) >> 3) & 1);
         const double* lb = sg + (st * SPI + s) * pitch + uoff;
-        if (GK) {
-          double uv[SW];
+        double uv[SW];
 #pragma unroll
-          for (int j = 0; j < SW; ++j) uv[j] = ub[c[k][j] & 0xffffu];
-          const double lam = rk[k] >= 0 ? lb[rk[k]] : 0.0;
-          double ku = 0.0;
+        for (int j = 0; j < SW; ++j) uv[j] = ub[c[k][j] & 0xffffu];
+        const double lam = rk[k] >= 0 ? lb[rk[k]] : 0.0;
+        double ku = 0.0;
 #pragma unroll
-          for (int j = 0; j < SW; ++j) ku = fma(wk[k][j], uv[j], ku);
-          part[s] = fma(lam, ku, part[s]);
-        }
+        for (int j = 0; j < SW; ++j) ku = fma(wk[k][j], uv[j], ku);
+        part[s] = fma(lam, ku, part[s]);
         if (GF) {
           double lv[SW];
 #pragma unroll
@@ -1014,16 +922,14 @@ __global__ void __launch_bounds__(SBT_MAX, (GF && GK) ? 1 : 2) k_band_grad3(cons
         }
       }
     }
-    if (GK) {
 #pragma unroll
-      for (int d = 16; d > 0; d >>= 1)
+    for (int d = 16; d > 0; d >>= 1)
 #pragma unroll
-        for (int s = 0; s < SPI; ++s) part[s] += __shfl_xor_sync(0xffffffffu, part[s], d);
-      if (lane == 0)
+      for (int s = 0; s < SPI; ++s) part[s] += __shfl_xor_sync(0xffffffffu, part[s], d);
+    if (lane == 0)
 #pragma unroll
-        for (int s = 0; s < SPI; ++s)
-          if (b + s * bs < B) gkpart[(b + s * bs) * nw + warp] = part[s];
-    }
+      for (int s = 0; s < SPI; ++s)
+        if (b + s * bs < B) gkpart[(b + s * bs) * nw + warp] = part[s];
     st = st + 1 == NG ? 0 : st + 1;
   }
   cp_async_wait<0>();
@@ -1059,106 +965,15 @@ bool band_reg_fits(const dfe_mesh* m) {
          m->dev.n_nodes > 0 && m->n_lift <= 8192 && m->max_adj <= ADJ6;
 }
 
-// L y = b, then L^T x = y, in place on X; one warp per BS samples.
-// Lane k holds two pending right-hand sides per sample: C = row k of the current 32-row block, N = row k of the next
-// one.  Step q (row i = 32 t + q): y = C[lane q] / L_ii (one shuffle, one multiply), then every lane subtracts
-// L[row][i] * y from the row it holds at distance d = 1..32 — lanes k > q from C (same block), lanes k <= q from N
-// (next block) — one coalesced 256 B load of column i for all BS samples.  C[lane q] is never touched after step q,
-// so the block's 32 results are C * (1 / L_ii) at the end of the block: no per-step capture.
-__global__ void __launch_bounds__(128) k_band_solve(int npad, long long B, const double* __restrict__ invd,
-                                                    const double* __restrict__ Lc, const double* __restrict__ Lr,
-                                                    double* __restrict__ X) {
-  const int lane = threadIdx.x & 31;
-  const long long b0 = (blockIdx.x * static_cast<long long>(blockDim.x >> 5) + (threadIdx.x >> 5)) * BS;
-  if (b0 >= B) return;
-  double* x[BS];
-  bool valid[BS];
-#pragma unroll
-  for (int s = 0; s < BS; ++s) {
-    valid[s] = b0 + s < B;
-    x[s] = X + (valid[s] ? b0 + s : b0) * npad;
-  }
-  const int nb = npad >> 5;
-  double C[BS], N[BS];
-  // ---- forward substitution, rows ascending
-#pragma unroll
-  for (int s = 0; s < BS; ++s) C[s] = x[s][lane];
-  for (int t = 0; t < nb; ++t) {
-#pragma unroll
-    for (int s = 0; s < BS; ++s) N[s] = t + 1 < nb ? x[s][32 * (t + 1) + lane] : 0.0;
-    const double invl = invd[32 * t + lane];
-#pragma unroll
-    for (int q = 0; q < 32; ++q) {
-      const int i = 32 * t + q;
-      const double inv = invd[i];                                                    // uniform
-      const double lc = Lc[static_cast<size_t>(i) * BW + ((lane - q - 1) & 31)];   // L[i+d][i], d = ((lane-q-1)&31)+1
-      // the coefficient is routed once per step (shared by the BS samples): two unconditional fmas per sample, one of
-      // which subtracts an exact zero
-      const double lcC = lane > q ? -lc : 0.0, lcN = lane > q ? 0.0 : -lc;
-#pragma unroll
-      for (int s = 0; s < BS; ++s) {
-        const double y = __shfl_sync(0xffffffffu, C[s], q) * inv;
-        C[s] = fma(lcC, y, C[s]);
-        N[s] = fma(lcN, y, N[s]);
-      }
-    }
-#pragma unroll
-    for (int s = 0; s < BS; ++s) {
-      if (valid[s]) x[s][32 * t + lane] = C[s] * invl;
-      C[s] = N[s];
-    }
-  }
-  __syncwarp();
-  // ---- backward substitution, rows descending (N = the block below)
-#pragma unroll
-  for (int s = 0; s < BS; ++s) C[s] = x[s][32 * (nb - 1) + lane];
-  for (int t = nb - 1; t >= 0; --t) {
-#pragma unroll
-    for (int s = 0; s < BS; ++s) N[s] = t > 0 ? x[s][32 * (t - 1) + lane] : 0.0;
-    const double invl = invd[32 * t + lane];
-#pragma unroll
-    for (int q = 31; q >= 0; --q) {
-      const int i = 32 * t + q;
-      const double inv = invd[i];
-      const double lr = Lr[static_cast<size_t>(i) * BW + ((q - lane - 1) & 31)];   // L[i][i-d], d = ((q-lane-1)&31)+1
-      const double lrC = lane < q ? -lr : 0.0, lrN = lane < q ? 0.0 : -lr;
-#pragma unroll
-      for (int s = 0; s < BS; ++s) {
-        const double xv = __shfl_sync(0xffffffffu, C[s], q) * inv;
-        C[s] = fma(lrC, xv, C[s]);
-        N[s] = fma(lrN, xv, N[s]);
-      }
-    }
-#pragma unroll
-    for (int s = 0; s < BS; ++s) {
-      if (valid[s]) x[s][32 * t + lane] = C[s] * invl;
-      C[s] = N[s];
-    }
-  }
-}
-
 // ---------------------------------------------------------------------------------------------------------------------
-// The same two triangular solves as a BLOCK-banded TRSM on the FP64 tensor cores (DMMA m8n8k4).
-//
-// With 32 x 32 blocks the band of L is block-bidiagonal: L y = b reads  y_k = H_k (b_k - S_k y_{k-1})  with
-// H_k = L_kk^{-1} (lower triangular) and S_k = L_{k,k-1} (UPPER triangular: the band is 32 wide), and L^T x = y reads
-// x_k = H_k^T (y_k - S_{k+1}^T x_{k+1}) — two TRIANGULAR 32 x 32 products per block row and right-hand side instead of 32
-// dependent shuffle / fma steps, i.e. a contraction: the one place of this library where tensor cores apply (the scalar
-// kernel above runs at ~2 TFLOP/s because every step waits for the previous one).  k_band_blocks builds H once per
-// factorisation (one CTA per block row) and stores H, -S and their transposes in the register layout of the DMMA B
-// operand.  (Round 2 first used y_k = H_k b_k + G_k y_{k-1} with the full block G_k = -H_k S_k: 26 non-zero 8 x 8 tiles per
-// block row; the two triangular factors have 20, and the kernel is bound by the FP64 MMA pipe.)
-//
-// The solve works on the transposed problem (samples x rows), Y_k^T = (B_k^T - Y_{k-1}^T S_k^T) H_k^T, so that a warp's
-// 16 samples are the M dimension (two 8-row tiles) and the previous block's result is the A operand of the next
-// product.  The accumulator layout of m8n8k4 (thread t holds row t/4, columns 2(t%4), 2(t%4)+1 of an 8 x 8 tile) differs
-// from the A layout (row t/4, column t%4) — but a contraction may enumerate its k index in any order as long as both
-// operands agree: k-step (tile nt', half j) is DEFINED to cover the columns 8nt' + 2(t%4) + j, which are exactly the
-// accumulator registers the thread already holds.  The B fragments are stored with the matching permutation, and the
-// result of one block row feeds the next one without a single shuffle or shared-memory round trip.
-constexpr int FRAGD = dfe::BAND_FRAGD;   // doubles per block row and direction: H fragments (1024), then -S fragments (1024)
+// The two triangular solves as a BLOCK-banded TRSM on the FP64 tensor cores (the block-row step and the fragment layout
+// are in dfe_band_mma.cuh): two TRIANGULAR 32 x 32 products per block row and right-hand side instead of 32 dependent
+// shuffle / fma steps (~2 TFLOP/s: every step waits for the previous one), i.e. a contraction: the one place of this library
+// where tensor cores apply.  k_band_blocks builds H once per factorisation (one CTA per block row) and stores H, -S and
+// their transposes in the register layout of the DMMA B operand.  (Round 2 first used y_k = H_k b_k + G_k y_{k-1} with the
+// full block G_k = -H_k S_k: 26 non-zero 8 x 8 tiles per block row; the two triangular factors have 20, and the kernel is
+// bound by the FP64 MMA pipe.)
 constexpr int MMA_W = 8;      // warps per CTA of the solve kernel
-constexpr int MMA_S = 16;     // samples per warp (two m8 tiles)
 
 __global__ void __launch_bounds__(256) k_band_blocks(int npad, const double* __restrict__ invd, const double* __restrict__ Lr,
                                                      double* __restrict__ Ff, double* __restrict__ Bf) {
@@ -1174,7 +989,7 @@ __global__ void __launch_bounds__(256) k_band_blocks(int npad, const double* __r
     H[a][b] = 0.0;
   }
   __syncthreads();
-  if (tid < 32) {   // column tid of H = L_kk^{-1} by forward substitution (same pivots 1 / L_ii as the scalar solve)
+  if (tid < 32) {   // column tid of H = L_kk^{-1} by forward substitution (pivots 1 / L_ii)
     const int c = tid;
     double h[32];
 #pragma unroll
@@ -1197,9 +1012,8 @@ __global__ void __launch_bounds__(256) k_band_blocks(int npad, const double* __r
   double* ff = Ff + static_cast<size_t>(k) * FRAGD;
   double* bf = Bf + static_cast<size_t>(k) * FRAGD;
   for (int q = tid; q < 1024; q += 256) {
-    const int f = q >> 5, t = q & 31;
-    const int nt = f & 3, j = (f >> 2) & 1, ntp = f >> 3;
-    const int cc = 8 * ntp + 2 * (t & 3) + j, rr = 8 * nt + (t >> 2);
+    int rr, cc;
+    frag_rc(q, rr, cc);
     ff[q] = H[rr][cc];            // forward:  out[s][r] += in[s][c] H[r][c]          (zero for c > r)
     ff[1024 + q] = -S[rr][cc];    //           t[s][r]   += y_prev[s][c] (-S[r][c])    (zero for c < r)
     bf[q] = H[cc][rr];            // backward: out[s][r] += in[s][c] H[c][r]          (zero for c < r)
@@ -1207,16 +1021,10 @@ __global__ void __launch_bounds__(256) k_band_blocks(int npad, const double* __r
   }
 }
 
-__device__ __forceinline__ void dmma884(double& d0, double& d1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};"
-               : "+d"(d0), "+d"(d1)
-               : "d"(a), "d"(b));
-}
-
 // GIN: the right-hand sides are gathered from a (B, n_nodes) array in node numbering (gsrc[b * ldg + free_nodes[r]], the
 // adjoint's gbar restricted to the free rows) instead of being read from X; SOUT: the solution is scattered straight into
-// u (u[b * ldu + free_nodes[r]], solver.py:180-181) instead of being written back to X.  Either removes a pass over the
-// batch (k_band_rhs_bwd / k_band_scatter: 0.25 + 0.27 ms of pure copies at config 5b); X still holds y between the passes.
+// u (u[b * ldu + free_nodes[r]], solver.py:177-181, with the Dirichlet values) instead of being written back to X.  Either
+// saves a pass over the batch (0.25 + 0.27 ms of pure copies at config 5b); X still holds y between the passes.
 template <bool GIN, bool SOUT>
 __global__ void __launch_bounds__(32 * MMA_W, 2) k_band_solve_mma(int npad, long long B, const double* __restrict__ Ff,
                                                                   const double* __restrict__ Bf, double* __restrict__ X,
@@ -1244,11 +1052,13 @@ __global__ void __launch_bounds__(32 * MMA_W, 2) k_band_solve_mma(int npad, long
     grow[mt] = GIN ? gsrc + sc * ldg : nullptr;
     urow[mt] = SOUT ? uout + sc * ldu : nullptr;
   }
-  // right-hand side of block row kb, columns 8 nt + 2 q + {0, 1}: from X, or gathered through the free-node table
-  auto load_rhs = [&](int kb, double (&Rr)[2][4][2]) {
+  // right-hand side of block row kb: from X, or gathered through the free-node table
+  auto load_rhs = [&](int kb, Blk& Rr) {
+    if (!GIN) {
+      ld_block(row, kb, Rr);
+    } else {
 #pragma unroll
-    for (int nt = 0; nt < 4; ++nt) {
-      if (GIN) {
+      for (int nt = 0; nt < 4; ++nt) {
         const int c0 = 32 * kb + 8 * nt + 2 * q;
         const int n0 = c0 < nfree ? fnode[c0] : -1, n1 = c0 + 1 < nfree ? fnode[c0 + 1] : -1;
 #pragma unroll
@@ -1256,120 +1066,36 @@ __global__ void __launch_bounds__(32 * MMA_W, 2) k_band_solve_mma(int npad, long
           Rr[mt][nt][0] = n0 >= 0 ? grow[mt][n0] : 0.0;
           Rr[mt][nt][1] = n1 >= 0 ? grow[mt][n1] : 0.0;
         }
-      } else {
-#pragma unroll
-        for (int mt = 0; mt < 2; ++mt) {
-          const double2 v = *reinterpret_cast<const double2*>(row[mt] + 32 * kb + 8 * nt);
-          Rr[mt][nt][0] = v.x;
-          Rr[mt][nt][1] = v.y;
-        }
       }
     }
   };
-  auto frag_src = [&](int step) { return step < nb ? Ff + static_cast<size_t>(step) * FRAGD : Bf + static_cast<size_t>(nsteps - 1 - step) * FRAGD; };
   if (tid == 0) {
     mbar_init_raw(&bar[0], 1);
     mbar_init_raw(&bar[1], 1);
     fence_mbar_init();
     mbar_arrive_expect_tx(&bar[0], FRAGD * 8u);
-    bulk_g2s(stg[0], frag_src(0), FRAGD * 8u, &bar[0]);
+    bulk_g2s(stg[0], frag_src(Ff, Bf, nb, 0), FRAGD * 8u, &bar[0]);
   }
-  double R[2][4][2], P[2][4][2], acc[2][4][2];
+  Blk R, P = {}, acc;
   load_rhs(0, R);
-#pragma unroll
-  for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt) P[mt][nt][0] = P[mt][nt][1] = 0.0;
   for (int step = 0; step < nsteps; ++step) {
-    const int k = step < nb ? step : nsteps - 1 - step;
+    const int k = band_block(step, nb);
     __syncthreads();   // every warp has finished step - 1: the other stage is free (and, at step 0, the barriers exist)
     if (tid == 0 && step + 1 < nsteps) {
       mbar_arrive_expect_tx(&bar[(step + 1) & 1], FRAGD * 8u);
-      bulk_g2s(stg[(step + 1) & 1], frag_src(step + 1), FRAGD * 8u, &bar[(step + 1) & 1]);
+      bulk_g2s(stg[(step + 1) & 1], frag_src(Ff, Bf, nb, step + 1), FRAGD * 8u, &bar[(step + 1) & 1]);
     }
     mbar_wait(&bar[step & 1], (step >> 1) & 1);
-    const double* sH = stg[step & 1];
-    const double* sG = sH + 1024;
-    // ---- stage 1: t = rhs of this block - S y_prev (forward) / - S_next^T x_next (backward).  The right-hand side is already
-    // in the accumulator layout; S is triangular: 10 of its 16 8 x 8 tiles are non-zero.
-    double t[2][4][2];
-#pragma unroll
-    for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-      for (int nt = 0; nt < 4; ++nt) {
-        t[mt][nt][0] = R[mt][nt][0];
-        t[mt][nt][1] = R[mt][nt][1];
-      }
-    // ---- the right-hand side of the next step is in flight while the two products run
-    const int knext = step + 1 < nb ? step + 1 : nsteps - 2 - step;   // block of step + 1 (== k at the turn-around)
+    Blk t;
+    blk_copy(t, R);
+    const int knext = band_block(step + 1, nb);   // == k at the turn-around
+    // the right-hand side of the next step is in flight while the two products run: the next block of b (forward pass)
+    // or of y (backward pass)
     if (step + 1 < nsteps && knext != k) {
-      if (GIN && step + 1 < nb) {
-        load_rhs(knext, R);               // forward pass: the next block of the gathered right-hand side
-      } else {
-#pragma unroll
-        for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-          for (int nt = 0; nt < 4; ++nt) {
-            const double2 v = *reinterpret_cast<const double2*>(row[mt] + 32 * knext + 8 * nt);
-            R[mt][nt][0] = v.x;
-            R[mt][nt][1] = v.y;
-          }
-      }
+      if (GIN && step + 1 < nb) load_rhs(knext, R);
+      else ld_block(row, knext, R);
     }
-    if (step != 0 && step != nb) {   // first block of a pass: nothing above / below it
-      if (step < nb) {
-#pragma unroll
-        for (int ntp = 0; ntp < 4; ++ntp)
-#pragma unroll
-          for (int j = 0; j < 2; ++j)
-#pragma unroll
-            for (int nt = 0; nt <= ntp; ++nt) {     // t[s][r] += y_prev[s][c] (-S[r][c]), zero for c < r
-              const double b = sG[((ntp * 2 + j) * 4 + nt) * 32 + lane];
-              dmma884(t[0][nt][0], t[0][nt][1], P[0][ntp][j], b);
-              dmma884(t[1][nt][0], t[1][nt][1], P[1][ntp][j], b);
-            }
-      } else {
-#pragma unroll
-        for (int ntp = 0; ntp < 4; ++ntp)
-#pragma unroll
-          for (int j = 0; j < 2; ++j)
-#pragma unroll
-            for (int nt = ntp; nt < 4; ++nt) {      // t[s][r] += x_next[s][c] (-U[c][r]), zero for c > r
-              const double b = sG[((ntp * 2 + j) * 4 + nt) * 32 + lane];
-              dmma884(t[0][nt][0], t[0][nt][1], P[0][ntp][j], b);
-              dmma884(t[1][nt][0], t[1][nt][1], P[1][ntp][j], b);
-            }
-      }
-    }
-    // ---- stage 2: H_k (forward; lower triangular) or H_k^T (backward; upper triangular) applied to t — the accumulators of
-    // stage 1 are the A operand (see above); 10 non-zero tiles
-#pragma unroll
-    for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-      for (int nt = 0; nt < 4; ++nt) acc[mt][nt][0] = acc[mt][nt][1] = 0.0;
-    if (step < nb) {
-#pragma unroll
-      for (int ntp = 0; ntp < 4; ++ntp)
-#pragma unroll
-        for (int j = 0; j < 2; ++j)
-#pragma unroll
-          for (int nt = ntp; nt < 4; ++nt) {      // out[s][r] += t[s][c] H[r][c], zero for c > r
-            const double b = sH[((ntp * 2 + j) * 4 + nt) * 32 + lane];
-            dmma884(acc[0][nt][0], acc[0][nt][1], t[0][ntp][j], b);
-            dmma884(acc[1][nt][0], acc[1][nt][1], t[1][ntp][j], b);
-          }
-    } else {
-#pragma unroll
-      for (int ntp = 0; ntp < 4; ++ntp)
-#pragma unroll
-        for (int j = 0; j < 2; ++j)
-#pragma unroll
-          for (int nt = 0; nt <= ntp; ++nt) {     // out[s][r] += t[s][c] H[c][r], zero for c < r
-            const double b = sH[((ntp * 2 + j) * 4 + nt) * 32 + lane];
-            dmma884(acc[0][nt][0], acc[0][nt][1], t[0][ntp][j], b);
-            dmma884(acc[1][nt][0], acc[1][nt][1], t[1][ntp][j], b);
-          }
-    }
+    band_step(step, nb, stg[step & 1], lane, t, P, acc);
 #pragma unroll
     for (int mt = 0; mt < 2; ++mt)
 #pragma unroll
@@ -1395,18 +1121,6 @@ __global__ void __launch_bounds__(32 * MMA_W, 2) k_band_solve_mma(int npad, long
         if (s0 + sidx < B) uout[(s0 + sidx) * ldu + node] = gv;
     }
   }
-}
-
-// forward: u = 0; u[d] = g; u[free] = x   (solver.py:177-181)
-__global__ void k_band_scatter(const MeshDev M, long long B, int npad, const double* __restrict__ X, double* __restrict__ u,
-                               long long ldu) {
-  const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
-  const int per = M.n_free + M.n_dir;
-  if (idx >= B * per) return;
-  const long long b = idx / per;
-  const int r = static_cast<int>(idx - b * per);
-  if (r < M.n_free) u[b * ldu + M.free_nodes[r]] = X[b * npad + r];
-  else u[b * ldu + M.dir_idx[r - M.n_free]] = M.dir_val[r - M.n_free];
 }
 
 // adjoint: dL/dkappa (per element, or summed per sample in a fixed order) and dL/df from lambda = X (0 on Dirichlet
@@ -1615,7 +1329,7 @@ extern "C" size_t dfe_band_factor_bytes(const dfe_mesh* m) {
   if (!m) return 0;
   const size_t np = static_cast<size_t>(band_npad(m));
   const size_t nnp = (static_cast<size_t>(m->dev.n_nodes) + 1) & ~static_cast<size_t>(1);
-  return (np + 2 * np * BW + 12 * static_cast<size_t>(m->dev.n_el) + static_cast<size_t>(m->n_lift) + (np + 40) * (BW + 1) +
+  return (np + np * BW + 12 * static_cast<size_t>(m->dev.n_el) + static_cast<size_t>(m->n_lift) + (np + 40) * (BW + 1) +
           2 * (np / 32) * FRAGD + 8 + (3 * SW + SW / 2 + 1) * nnp + np) * sizeof(double) + 512;
 }
 extern "C" size_t dfe_band_workspace_bytes(const dfe_mesh* m, int64_t B) {
@@ -1625,7 +1339,7 @@ extern "C" size_t dfe_band_workspace_bytes(const dfe_mesh* m, int64_t B) {
 
 namespace {
 struct BandPtrs {
-  double *invd, *Lc, *Lr, *geom, *geom2, *liftp, *Ab, *Ff, *Bf, *ellK, *ellM, *ellMr, *liftc;
+  double *invd, *Lr, *geom, *geom2, *liftp, *Ab, *Ff, *Bf, *ellK, *ellM, *ellMr, *liftc;
   unsigned* ellc;
   int nnp;
   int* status;
@@ -1634,8 +1348,7 @@ BandPtrs band_ptrs(const dfe_mesh* m, void* factor) {
   const size_t np = static_cast<size_t>(band_npad(m));
   BandPtrs p;
   p.invd = static_cast<double*>(factor);
-  p.Lc = p.invd + np;
-  p.Lr = p.Lc + np * BW;
+  p.Lr = p.invd + np;
   p.geom = p.Lr + np * BW;
   p.geom2 = p.geom + 8 * static_cast<size_t>(m->dev.n_el);
   p.liftp = p.geom2 + 4 * static_cast<size_t>(m->dev.n_el);
@@ -1671,17 +1384,10 @@ int band_enter(const dfe_mesh* m, const char* who, int* prev) {
 }
 inline unsigned nblk(long long n, int t) { return static_cast<unsigned>((n + t - 1) / t > 0 ? (n + t - 1) / t : 1); }
 
-// L y = b, L^T x = y for the whole batch, in place on X: block TRSM on the FP64 tensor cores (default), or the scalar
-// warp-shuffle kernel (DFE_BAND_SCALAR=1: the bit-reference of the tensor-core path and an A/B switch)
+// L y = b, L^T x = y for the whole batch, in place on X: block TRSM on the FP64 tensor cores
 void band_solve(int np, long long B, const BandPtrs& p, double* X, cudaStream_t st) {
-  static const bool scalar = getenv("DFE_BAND_SCALAR") != nullptr;
-  if (scalar) k_band_solve<<<nblk((B + BS - 1) / BS, 4), 128, 0, st>>>(np, B, p.invd, p.Lc, p.Lr, X);
-  else k_band_solve_mma<false, false><<<nblk(B, MMA_W * MMA_S), 32 * MMA_W, 0, st>>>(np, B, p.Ff, p.Bf, X, nullptr, 0, nullptr, 0, nullptr, 0, nullptr, nullptr, 0);
-}
-// the fused variants exist for the tensor-core kernel only
-bool band_fused_io() {
-  static const bool off = getenv("DFE_BAND_SCALAR") != nullptr || getenv("DFE_BAND_NOFUSE") != nullptr;
-  return !off;
+  k_band_solve_mma<false, false><<<nblk(B, MMA_W * MMA_S), 32 * MMA_W, 0, st>>>(np, B, p.Ff, p.Bf, X, nullptr, 0, nullptr, 0,
+                                                                                nullptr, 0, nullptr, nullptr, 0);
 }
 }  // namespace
 
@@ -1705,15 +1411,13 @@ extern "C" int dfe_band_factor(const dfe_mesh* m, const double* vals_full, void*
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const BandPtrs p = band_ptrs(m, factor);
     const size_t np = static_cast<size_t>(band_npad(m));
-    // invd | Lc | Lr zeroed (rows >= n_free and entries outside the band stay zero), Ab zeroed, then gathered
-    cudaError_t e = cudaMemsetAsync(p.invd, 0, (np + 2 * np * BW) * sizeof(double), st);
+    // invd | Lr zeroed (rows >= n_free and entries outside the band stay zero), Ab zeroed, then gathered
+    cudaError_t e = cudaMemsetAsync(p.invd, 0, (np + np * BW) * sizeof(double), st);
     if (e == cudaSuccess) e = cudaMemsetAsync(p.Ab, 0, (np + 40) * (BW + 1) * sizeof(double), st);
     k_band_gather<<<nblk(m->dev.n_free, 128), 128, 0, st>>>(m->dev, vals_full, p.Ab);
     // (running the Cholesky chain on a second stream under the load-vector kernel of dfe_band_fwd was measured: no gain —
     // the one-CTA factorisation is latency-bound and slows down under a bandwidth-bound neighbour as much as it overlaps)
-    static const bool unblocked = getenv("DFE_BAND_FACTOR_ROWS") != nullptr;   // A/B switch: the row-by-row kernel
-    if (unblocked) k_band_factor<<<1, 256, 0, st>>>(m->dev.n_free, band_npad(m), p.Ab, p.invd, p.Lc, p.Lr, p.status);
-    else k_band_factor_blk<<<1, 256, 0, st>>>(m->dev.n_free, band_npad(m), p.Ab, p.invd, p.Lc, p.Lr, p.status);
+    k_band_factor_blk<<<1, 256, 0, st>>>(m->dev.n_free, band_npad(m), p.Ab, p.invd, p.Lr, p.status);
     k_band_blocks<<<static_cast<unsigned>(np / 32), 256, 0, st>>>(band_npad(m), p.invd, p.Lr, p.Ff, p.Bf);
     if (e == cudaSuccess && status_dev) e = cudaMemcpyAsync(status_dev, p.status, sizeof(int), cudaMemcpyDeviceToDevice, st);
     k_band_geom<<<nblk(m->dev.n_el, 128), 128, 0, st>>>(m->dev, p.geom);
@@ -1751,9 +1455,7 @@ extern "C" int dfe_band_fwd(const dfe_mesh* m, int64_t B, const double* f, int64
     const int np = band_npad(m);
     const BandPtrs p = band_ptrs(m, const_cast<void*>(factor));
     double* X = static_cast<double*>(ws);
-    static const bool old_kernels = getenv("DFE_BAND_OLD") != nullptr;   // A/B switch: general per-sample kernels
-    static const bool reg_kernels = getenv("DFE_BAND_REG") != nullptr;   // A/B switch: no stencil-form kernels
-    if (band_stencil_fits(m) && !old_kernels && !reg_kernels) {
+    if (band_stencil_fits(m)) {
       const int nt = ((np + SR - 1) / SR + 31) & ~31;
       const size_t row = static_cast<size_t>(p.nnp + 2) * sizeof(double);
       auto launch_rhs = [&](auto kern, int rows) {
@@ -1777,14 +1479,9 @@ extern "C" int dfe_band_fwd(const dfe_mesh* m, int64_t B, const double* f, int64
       if (rgrid > B) rgrid = B;
       k_band_rhs_fwd<<<static_cast<unsigned>(rgrid), BT, rsm, st>>>(m->dev, B, np, f, ldf, vals_full, p.geom, X);
     }
-    if (band_fused_io()) {
-      k_band_solve_mma<false, true><<<nblk(B, MMA_W * MMA_S), 32 * MMA_W, 0, st>>>(np, B, p.Ff, p.Bf, X, m->dev.free_nodes,
-                                                                                   m->dev.n_free, nullptr, 0, u, ldu,
-                                                                                   m->dev.dir_idx, m->dev.dir_val, m->dev.n_dir);
-    } else {
-      band_solve(np, B, p, X, st);
-      k_band_scatter<<<nblk(B * (m->dev.n_free + m->dev.n_dir), 256), 256, 0, st>>>(m->dev, B, np, X, u, ldu);
-    }
+    k_band_solve_mma<false, true><<<nblk(B, MMA_W * MMA_S), 32 * MMA_W, 0, st>>>(np, B, p.Ff, p.Bf, X, m->dev.free_nodes,
+                                                                                 m->dev.n_free, nullptr, 0, u, ldu,
+                                                                                 m->dev.dir_idx, m->dev.dir_val, m->dev.n_dir);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) {
       dfe::set_error("dfe_band_fwd: kernel launch failed: %s", cudaGetErrorString(e));
@@ -1815,20 +1512,13 @@ extern "C" int dfe_band_bwd(const dfe_mesh* m, int64_t B, const double* gbar, in
     const int np = band_npad(m);
     const BandPtrs p = band_ptrs(m, const_cast<void*>(factor));
     double* X = static_cast<double*>(ws);
-    if (band_fused_io()) {
-      k_band_solve_mma<true, false><<<nblk(B, MMA_W * MMA_S), 32 * MMA_W, 0, st>>>(np, B, p.Ff, p.Bf, X, m->dev.free_nodes,
-                                                                                   m->dev.n_free, gbar, ldg, nullptr, 0, nullptr, nullptr, 0);
-    } else {
-      k_band_rhs_bwd<<<nblk(B * np, 256), 256, 0, st>>>(m->dev, B, np, gbar, ldg, X);
-      band_solve(np, B, p, X, st);
-    }
+    k_band_solve_mma<true, false><<<nblk(B, MMA_W * MMA_S), 32 * MMA_W, 0, st>>>(np, B, p.Ff, p.Bf, X, m->dev.free_nodes,
+                                                                                 m->dev.n_free, gbar, ldg, nullptr, 0, nullptr, nullptr, 0);
     const size_t gsm = (2 * static_cast<size_t>(m->dev.n_nodes) + m->dev.n_el + 2 * BNW) * sizeof(double);
-    static const bool old_kernels = getenv("DFE_BAND_OLD") != nullptr;
-    static const bool reg_kernels = getenv("DFE_BAND_REG") != nullptr;
-    if (kappa_mode == DFE_KAPPA_SCALAR && band_stencil_fits(m) && !old_kernels && !reg_kernels) {
+    if (kappa_mode == DFE_KAPPA_SCALAR && band_stencil_fits(m)) {
       const int nt = ((m->dev.n_nodes + SR - 1) / SR + 31) & ~31;
       double* gkpart = X + static_cast<size_t>(B) * np;
-      auto launch_half = [&](auto kern, size_t sm3, double* gfp) {
+      auto launch_grad = [&](auto kern, size_t sm3, double* gfp) {
         cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(sm3));
         int occ = 1;
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, nt, sm3);
@@ -1836,26 +1526,22 @@ extern "C" int dfe_band_bwd(const dfe_mesh* m, int64_t B, const double* gbar, in
         if (grid > B) grid = B;
         kern<<<static_cast<unsigned>(grid), nt, sm3, st>>>(m->dev, B, np, p.nnp, X, u, ldu, p.ellK, p.ellMr, p.ellc, gkpart, gfp, ldgf);
       };
-      // both halves in one kernel when dL/df is wanted (measured: 0.86 ms vs 0.54 + 0.39 ms as two kernels — the second
-      // pass over the lambda rows costs more than the lower occupancy); DFE_BAND_GRAD_SPLIT=1 is the A/B switch
-      static const bool split = getenv("DFE_BAND_GRAD_SPLIT") != nullptr;
-      const size_t row2 = static_cast<size_t>(p.nnp + 2 + np) * sizeof(double), row1 = static_cast<size_t>(np) * sizeof(double);
-      if (gf && !split) {
-        switch (band_spi(row2)) {
-          case 4: launch_half(k_band_grad3<true, true, 4, 3>, 12 * row2, gf); break;
-          case 2: launch_half(k_band_grad3<true, true, 2, 4>, 8 * row2, gf); break;
-          default: launch_half(k_band_grad3<true, true, 1, NST_G>, NST_G * row2, gf); break;
+      const size_t row = static_cast<size_t>(p.nnp + 2 + np) * sizeof(double);
+      if (gf) {
+        switch (band_spi(row)) {
+          case 4: launch_grad(k_band_grad3<true, 4, 3>, 12 * row, gf); break;
+          case 2: launch_grad(k_band_grad3<true, 2, 4>, 8 * row, gf); break;
+          default: launch_grad(k_band_grad3<true, 1, NST_G>, NST_G * row, gf); break;
         }
       } else {
-        switch (band_spi(2 * row2)) {   // two CTAs per SM for this half
-          case 4: launch_half(k_band_grad3<false, true, 4, 3>, 12 * row2, nullptr); break;
-          case 2: launch_half(k_band_grad3<false, true, 2, 4>, 8 * row2, nullptr); break;
-          default: launch_half(k_band_grad3<false, true, 1, NST_G>, NST_G * row2, nullptr); break;
+        switch (band_spi(2 * row)) {   // two CTAs per SM without dL/df
+          case 4: launch_grad(k_band_grad3<false, 4, 3>, 12 * row, nullptr); break;
+          case 2: launch_grad(k_band_grad3<false, 2, 4>, 8 * row, nullptr); break;
+          default: launch_grad(k_band_grad3<false, 1, NST_G>, NST_G * row, nullptr); break;
         }
-        if (gf) launch_half(k_band_grad3<true, false, 1, NST_G>, NST_G * row1, gf);
       }
       k_band_gksum<<<nblk(B, 256), 256, 0, st>>>(B, nt / 32, gkpart, gkappa);
-    } else if (band_reg_fits(m) && !old_kernels) {
+    } else if (band_reg_fits(m)) {
       const int nnp = (m->dev.n_nodes + 1) & ~1;
       const size_t gsm2 = (4 * static_cast<size_t>(nnp) + m->dev.n_el + 4 + 2 * BNW) * sizeof(double);
       cudaFuncSetAttribute(k_band_grad2, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(gsm2));

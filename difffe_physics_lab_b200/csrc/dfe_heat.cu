@@ -10,7 +10,7 @@
 // (lam~ = lambda scattered with zeros on the Dirichlet nodes, u_n the full state: the kappa-dependence of the lifting is
 // included because lam~ vanishes on the Dirichlet rows).  dL/df is W^T (dt sum_n sum_b lam~_n): dfe_grad's gf.
 //
-// k_heat_roll   the whole time loop in ONE launch.  It is the tensor-core block TRSM of k_band_solve_mma (dfe_batch.cu) with
+// k_heat_roll   the whole time loop in ONE launch.  It runs the block-row step of k_band_solve_mma (dfe_band_mma.cuh) with
 //               a time loop around the substitution loop: a warp owns 16 samples for the whole rollout and every lane reads
 //               back exactly the row positions it wrote, so consecutive time steps need no synchronisation beyond the
 //               per-block-row stage barrier.  The right-hand side is formed at load time (fma(m, x_n, c) forward,
@@ -32,10 +32,9 @@ namespace {
 
 using dfe::MeshDev;
 #include "dfe_1d_common.cuh"   // mbarrier / 1-D TMA bulk copy wrappers
+#include "dfe_band_mma.cuh"     // block-row step of the tensor-core band solve and its fragment layout
 
 constexpr double AREA_EPS = 1e-15;          // solver.py:120
-constexpr int FRAGD = dfe::BAND_FRAGD;
-constexpr int HS = 16;                      // samples per warp (two m8 tiles of the DMMA M dimension)
 constexpr long long WAIT_POLLS = 1LL << 24; // try_wait polls before a fragment stage counts as lost (raises the fault word)
 constexpr int GT = 256;                     // threads of the gradient kernel
 constexpr int GNST = 3;                     // cp.async ring stages of the gradient kernel
@@ -65,12 +64,6 @@ struct RollArgs {
   int* fault;                       // set to 1 when a fragment stage was lost
 };
 
-__device__ __forceinline__ void dmma884(double& d0, double& d1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};"
-               : "+d"(d0), "+d"(d1)
-               : "d"(a), "d"(b));
-}
-
 __device__ __forceinline__ bool mbar_wait_bounded(uint64_t* bar, uint32_t parity) {
   for (long long i = 0; i < WAIT_POLLS; ++i) {
     uint32_t ok;
@@ -94,7 +87,7 @@ __global__ void __launch_bounds__(32 * W, 16 / W) k_heat_roll(const RollArgs a) 
   const int g = lane >> 2, q = lane & 3;
   const int npad = a.npad, nb = npad >> 5, nsub = 2 * nb, nfree = a.nfree;
   const long long B = a.B;
-  const long long s0 = (blockIdx.x * static_cast<long long>(W) + warp) * HS;
+  const long long s0 = (blockIdx.x * static_cast<long long>(W) + warp) * MMA_S;
   long long sid[2];
   bool valid[2];
   double* row[2];
@@ -127,19 +120,8 @@ __global__ void __launch_bounds__(32 * W, 16 / W) k_heat_roll(const RollArgs a) 
       }
     }
   }
-  // the carry of block kb (columns 32 kb + 8 nt + 2 q + {0, 1}, the accumulator layout)
-  auto load_carry = [&](int kb, double (&R)[2][4][2]) {
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-      for (int mt = 0; mt < 2; ++mt) {
-        const double2 v = *reinterpret_cast<const double2*>(row[mt] + 32 * kb + 8 * nt);
-        R[mt][nt][0] = v.x;
-        R[mt][nt][1] = v.y;
-      }
-  };
   // carry -> right-hand side in place: fma(m, x_n, c) (forward) / fma(m, lambda_{n+1}, gbar_n[free]) (adjoint)
-  auto form_rhs = [&](int kb, double (&R)[2][4][2]) {
+  auto form_rhs = [&](int kb, Blk& R) {
 #pragma unroll
     for (int nt = 0; nt < 4; ++nt) {
       const int c0 = 32 * kb + 8 * nt + 2 * q;
@@ -162,115 +144,43 @@ __global__ void __launch_bounds__(32 * W, 16 / W) k_heat_roll(const RollArgs a) 
       }
     }
   };
-  auto frag_src = [&](int step) { return step < nb ? a.Ff + static_cast<size_t>(step) * FRAGD : a.Bf + static_cast<size_t>(nsub - 1 - step) * FRAGD; };
   if (tid == 0) {
     mbar_init_raw(&bar[0], 1);
     mbar_init_raw(&bar[1], 1);
     fence_mbar_init();
     mbar_arrive_expect_tx(&bar[0], FRAGD * 8u);
-    bulk_g2s(stg[0], frag_src(0), FRAGD * 8u, &bar[0]);
+    bulk_g2s(stg[0], frag_src(a.Ff, a.Bf, nb, 0), FRAGD * 8u, &bar[0]);
   }
-  double R[2][4][2], P[2][4][2], acc[2][4][2];
+  Blk R, P = {}, acc;
   set_gbar(0);
-  load_carry(0, R);
+  ld_block(row, 0, R);
   form_rhs(0, R);
-#pragma unroll
-  for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt) P[mt][nt][0] = P[mt][nt][1] = 0.0;
   bool lost = false;
   long long G = 0;   // stage counter over the whole rollout: fragment slot G & 1, barrier parity (G >> 1) & 1
   for (int it = 0; it < a.nt; ++it) {
     for (int step = 0; step < nsub; ++step, ++G) {
-      const int k = step < nb ? step : nsub - 1 - step;
+      const int k = band_block(step, nb);
       __syncthreads();   // every warp has finished stage G - 1: the other slot is free (and, at G = 0, the barriers exist)
       if (tid == 0 && !(it + 1 == a.nt && step + 1 == nsub)) {   // the fragment sequence repeats every time step
         const int ns = step + 1 < nsub ? step + 1 : 0;
         mbar_arrive_expect_tx(&bar[(G + 1) & 1], FRAGD * 8u);
-        bulk_g2s(stg[(G + 1) & 1], frag_src(ns), FRAGD * 8u, &bar[(G + 1) & 1]);
+        bulk_g2s(stg[(G + 1) & 1], frag_src(a.Ff, a.Bf, nb, ns), FRAGD * 8u, &bar[(G + 1) & 1]);
       }
       if (!mbar_wait_bounded(&bar[G & 1], static_cast<uint32_t>((G >> 1) & 1))) lost = true;
-      const double* sH = stg[G & 1];
-      const double* sG = sH + 1024;
-      double t[2][4][2];
-#pragma unroll
-      for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-        for (int nt = 0; nt < 4; ++nt) {
-          t[mt][nt][0] = R[mt][nt][0];
-          t[mt][nt][1] = R[mt][nt][1];
-        }
-      // the right-hand side of the next block is in flight while the two products run
-      const int knext = step + 1 < nb ? step + 1 : nsub - 2 - step;
+      Blk t;
+      blk_copy(t, R);
+      const int knext = band_block(step + 1, nb);   // == k at the turn-around
+      // the right-hand side of the next block is in flight while the two products run.  (One load per branch, and the
+      // redundant step + 1 < nsub test of the turn-around below: the merged forms spill at 128 registers.)
       if (step + 1 < nsub && knext != k) {
         if (step + 1 < nb) {
-          load_carry(knext, R);
+          ld_block(row, knext, R);
           form_rhs(knext, R);
         } else {
-#pragma unroll
-          for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-            for (int nt = 0; nt < 4; ++nt) {
-              const double2 v = *reinterpret_cast<const double2*>(row[mt] + 32 * knext + 8 * nt);
-              R[mt][nt][0] = v.x;
-              R[mt][nt][1] = v.y;
-            }
+          ld_block(row, knext, R);
         }
       }
-      // stage 1: t -= S y_prev (forward pass) / S_next^T x_next (backward pass); 10 non-zero 8 x 8 tiles
-      if (step != 0 && step != nb) {
-        if (step < nb) {
-#pragma unroll
-          for (int ntp = 0; ntp < 4; ++ntp)
-#pragma unroll
-            for (int j = 0; j < 2; ++j)
-#pragma unroll
-              for (int nt = 0; nt <= ntp; ++nt) {
-                const double b = sG[((ntp * 2 + j) * 4 + nt) * 32 + lane];
-                dmma884(t[0][nt][0], t[0][nt][1], P[0][ntp][j], b);
-                dmma884(t[1][nt][0], t[1][nt][1], P[1][ntp][j], b);
-              }
-        } else {
-#pragma unroll
-          for (int ntp = 0; ntp < 4; ++ntp)
-#pragma unroll
-            for (int j = 0; j < 2; ++j)
-#pragma unroll
-              for (int nt = ntp; nt < 4; ++nt) {
-                const double b = sG[((ntp * 2 + j) * 4 + nt) * 32 + lane];
-                dmma884(t[0][nt][0], t[0][nt][1], P[0][ntp][j], b);
-                dmma884(t[1][nt][0], t[1][nt][1], P[1][ntp][j], b);
-              }
-        }
-      }
-      // stage 2: H_k (forward pass) or H_k^T (backward pass) applied to t; 10 non-zero tiles
-#pragma unroll
-      for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-        for (int nt = 0; nt < 4; ++nt) acc[mt][nt][0] = acc[mt][nt][1] = 0.0;
-      if (step < nb) {
-#pragma unroll
-        for (int ntp = 0; ntp < 4; ++ntp)
-#pragma unroll
-          for (int j = 0; j < 2; ++j)
-#pragma unroll
-            for (int nt = ntp; nt < 4; ++nt) {
-              const double b = sH[((ntp * 2 + j) * 4 + nt) * 32 + lane];
-              dmma884(acc[0][nt][0], acc[0][nt][1], t[0][ntp][j], b);
-              dmma884(acc[1][nt][0], acc[1][nt][1], t[1][ntp][j], b);
-            }
-      } else {
-#pragma unroll
-        for (int ntp = 0; ntp < 4; ++ntp)
-#pragma unroll
-          for (int j = 0; j < 2; ++j)
-#pragma unroll
-            for (int nt = 0; nt <= ntp; ++nt) {
-              const double b = sH[((ntp * 2 + j) * 4 + nt) * 32 + lane];
-              dmma884(acc[0][nt][0], acc[0][nt][1], t[0][ntp][j], b);
-              dmma884(acc[1][nt][0], acc[1][nt][1], t[1][ntp][j], b);
-            }
-      }
+      band_step(step, nb, stg[G & 1], lane, t, P, acc);
       const int jslot = a.nt - 1 - it;   // adjoint: lambda_{n0 + 1 + jslot} is this time step's result
 #pragma unroll
       for (int mt = 0; mt < 2; ++mt)
@@ -312,13 +222,7 @@ __global__ void __launch_bounds__(32 * W, 16 / W) k_heat_roll(const RollArgs a) 
     }
     if (it + 1 < a.nt) {   // block 0 of the carry is in acc: the first right-hand side block of the next step, from registers
       set_gbar(it + 1);
-#pragma unroll
-      for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-        for (int nt = 0; nt < 4; ++nt) {
-          R[mt][nt][0] = acc[mt][nt][0];
-          R[mt][nt][1] = acc[mt][nt][1];
-        }
+      blk_copy(R, acc);
       form_rhs(0, R);
     }
   }
@@ -459,7 +363,7 @@ int grad_nchunk(long long B) { return static_cast<int>((B + grad_cs(B) - 1) / gr
 // warps per CTA of the rollout kernels: the largest of 8 and 4 whose grid still covers every SM, else 2
 int roll_warps(const dfe_mesh* m, long long B) {
   for (int w = 8; w > 2; w >>= 1)
-    if ((B + HS * w - 1) / (HS * w) >= m->sm_count) return w;
+    if ((B + MMA_S * w - 1) / (MMA_S * w) >= m->sm_count) return w;
   return 2;
 }
 
@@ -498,7 +402,7 @@ int roll_launch(const dfe_mesh* m, int warps, RollArgs a, const void* factor, cu
   a.dir_idx = m->dev.dir_idx;
   a.dir_val = m->dev.dir_val;
   dfe::band_frags(m, factor, &a.Ff, &a.Bf);
-  const unsigned grid = nblk(a.B, HS * warps);
+  const unsigned grid = nblk(a.B, MMA_S * warps);
   switch (warps) {
     case 8: k_heat_roll<ADJ, 8><<<grid, 256, 0, st>>>(a); break;
     case 4: k_heat_roll<ADJ, 4><<<grid, 128, 0, st>>>(a); break;

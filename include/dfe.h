@@ -223,7 +223,7 @@ int dfe_batch_bwd(const dfe_mesh* m, int64_t B, const double* gbar, int64_t ldg,
 /* ---------------------------------------------------------------- the same batch, banded direct solver
  * When the half bandwidth of K_free is <= 32 (dfe_band_supported; e.g. FEMesh.rectangle(nx, ny) with nx <= 32 in the
  * reference's node numbering) the shared matrix is factored ONCE per call, K_free = L L^T, and every sample costs two
- * banded triangular solves (a warp owns 8 samples) — ~13x fewer flops than Jacobi-PCG at 961 unknowns and no
+ * banded triangular solves (a warp owns 16 samples) — ~13x fewer flops than Jacobi-PCG at 961 unknowns and no
  * reductions.  This is the closest replacement of solver.py:174 (dense LU) for config 5b.
  *   dfe_band_factor   vals_full from dfe_assemble; factor: dfe_band_factor_bytes(m) bytes of device memory;
  *                     status_dev (optional, device int32): 0 ok, 5 = pivot <= 0 (K_free not SPD)
@@ -234,8 +234,8 @@ int dfe_batch_bwd(const dfe_mesh* m, int64_t B, const double* gbar, int64_t ldg,
  *                     = free node dfe_mesh_free_nodes_host()[r]; entries r >= n_free must be 0 and stay 0), in place, with
  *                     a factor from dfe_band_factor.  `vals_full` given to dfe_band_factor may be ANY symmetric positive
  *                     definite matrix on the pattern of K (e.g. M + dt K): this is the operator-reuse entry point for
- *                     time stepping (reference README.md:139-143 roadmap: heat equation; examples/heat_2d.py).  Default:
- *                     block TRSM on the FP64 tensor cores (mma.sync m8n8k4.f64), DFE_BAND_SCALAR=1: warp-shuffle kernel.
+ *                     time stepping (reference README.md:139-143 roadmap: heat equation; examples/heat_2d.py).  Block TRSM
+ *                     on the FP64 tensor cores (mma.sync m8n8k4.f64).
  */
 int dfe_band_supported(const dfe_mesh* m);
 size_t dfe_band_factor_bytes(const dfe_mesh* m);
