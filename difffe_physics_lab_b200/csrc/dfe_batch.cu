@@ -760,6 +760,9 @@ __device__ __forceinline__ void cp_async16_u32(uint32_t dst, const double* gsrc)
 }
 // Copy the n doubles at src (8-byte aligned) to shared memory so that element p lands at dst16 + 8 * (mis + p), where
 // mis = 0 / 1 is the 16-byte phase of src and dst16 is 16-byte aligned: one 8-byte head / tail, 16-byte pairs between.
+// Thread 0 issues both: it exists in every CTA, one-warp CTAs included (npad <= 64 / n_nodes <= 64).  (Giving the tail to
+// thread 32 instead left it uncopied in a one-warp CTA; thread nt - 1 or a thread of the second warp costs k_band_rhs_fwd3
+// up to 10 registers more.)
 // Returns mis (the reader's row starts at element `mis` of the stage).
 __device__ __forceinline__ int row_to_smem(uint32_t dst16, const double* src, int n, int tid, int nt) {
   const int mis = static_cast<int>((reinterpret_cast<uintptr_t>(src) >> 3) & 1);
@@ -768,7 +771,7 @@ __device__ __forceinline__ int row_to_smem(uint32_t dst16, const double* src, in
   const uint32_t d2 = dst16 + 16u * mis;
   for (int q = tid; q < npair; q += nt) cp_async16_u32(d2 + 16u * q, s2 + 2 * q);
   if (tid == 0 && mis) cp_async8_u32(dst16 + 8u, src);
-  if (tid == 32 && ((n - mis) & 1)) cp_async8_u32(dst16 + 8u * (mis + n - 1), src + n - 1);
+  if (tid == 0 && ((n - mis) & 1)) cp_async8_u32(dst16 + 8u * (mis + n - 1), src + n - 1);
   return mis;
 }
 
@@ -1444,8 +1447,8 @@ extern "C" int dfe_band_fwd(const dfe_mesh* m, int64_t B, const double* f, int64
   int prev;
   int rc = band_enter(m, "dfe_band_fwd", &prev);
   if (rc) return rc;
-  if (!f || !vals_full || !factor || !u || !ws || B < 1) {
-    dfe::set_error("dfe_band_fwd: null / invalid argument");
+  if (!f || !vals_full || !factor || !u || !ws || B < 1 || ldf < m->dev.n_nodes || ldu < m->dev.n_nodes) {
+    dfe::set_error("dfe_band_fwd: null / invalid argument (row strides must be >= n_nodes)");
     rc = DFE_ERR_INVALID;
   } else if (ws_bytes < dfe_band_workspace_bytes(m, B)) {
     dfe::set_error("dfe_band_fwd: workspace %zu bytes < required %zu", ws_bytes, dfe_band_workspace_bytes(m, B));
@@ -1498,8 +1501,9 @@ extern "C" int dfe_band_bwd(const dfe_mesh* m, int64_t B, const double* gbar, in
   int prev;
   int rc = band_enter(m, "dfe_band_bwd", &prev);
   if (rc) return rc;
-  if (!gbar || !u || !factor || !gkappa || !ws || B < 1) {
-    dfe::set_error("dfe_band_bwd: null / invalid argument");
+  if (!gbar || !u || !factor || !gkappa || !ws || B < 1 || ldg < m->dev.n_nodes || ldu < m->dev.n_nodes ||
+      (gf && ldgf < m->dev.n_nodes)) {
+    dfe::set_error("dfe_band_bwd: null / invalid argument (row strides must be >= n_nodes)");
     rc = DFE_ERR_INVALID;
   } else if (kappa_mode != DFE_KAPPA_SCALAR && kappa_mode != DFE_KAPPA_PER_ELEMENT) {
     dfe::set_error("dfe_band_bwd: kappa_mode must be SCALAR or PER_ELEMENT (the batch shares one matrix)");

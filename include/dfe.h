@@ -229,6 +229,8 @@ int dfe_batch_bwd(const dfe_mesh* m, int64_t B, const double* gbar, int64_t ldg,
  *                     status_dev (optional, device int32): 0 ok, 5 = pivot <= 0 (K_free not SPD)
  *   dfe_band_fwd/bwd  like dfe_batch_fwd/bwd with `factor` instead of the SELL matrix;
  *                     ws: dfe_band_workspace_bytes(m, B) bytes.  All calls are asynchronous on `stream`.
+ *                     Row strides ldf / ldu / ldg / ldgf are >= n_nodes (else DFE_ERR_INVALID); the rows of f, u, gbar
+ *                     and gf need only the 8-byte alignment of a double (odd strides and offsets are fine).
  *   dfe_band_npad     leading dimension of a block of right-hand sides in free numbering (n_free rounded up to 32)
  *   dfe_band_solve    X <- A_free^{-1} X for B right-hand sides, X (B, npad) row-major in FREE numbering (row r of a sample
  *                     = free node dfe_mesh_free_nodes_host()[r]; entries r >= n_free must be 0 and stay 0), in place, with
