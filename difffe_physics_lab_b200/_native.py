@@ -20,10 +20,10 @@ PKG = pathlib.Path(__file__).resolve().parent
 ROOT = PKG.parent
 LIB_PATH = PKG / "libdfe_b200.so"
 SOURCES = ["dfe_mesh.cu", "dfe_1d.cu", "dfe_1d_split.cu", "dfe_1d_pipe.cu", "dfe_general.cu", "dfe_pcg.cu", "dfe_mg.cu",
-           "dfe_batch.cu", "dfe_heat.cu"]
+           "dfe_batch.cu", "dfe_band_ps.cu", "dfe_heat.cu"]
 HEADERS = [PKG / "csrc" / "dfe_internal.h", PKG / "csrc" / "dfe_1d_common.cuh", PKG / "csrc" / "dfe_gridsync.cuh", PKG / "csrc" / "dfe_exact.cuh",
            PKG / "csrc" / "dfe_p2.cuh", PKG / "csrc" / "dfe_mg_kernel.cuh", PKG / "csrc" / "dfe_band_mma.cuh",
-           ROOT / "include" / "dfe.h"]
+           PKG / "csrc" / "dfe_assemble_row.cuh", ROOT / "include" / "dfe.h"]
 
 OK, ERR_INVALID, ERR_CUDA, ERR_UNSUPPORTED, ERR_NOT_CONVERGED, ERR_BREAKDOWN, ERR_WORKSPACE = range(7)
 KAPPA_SCALAR, KAPPA_PER_SAMPLE, KAPPA_PER_ELEMENT, KAPPA_PER_SAMPLE_ELEMENT = range(4)
@@ -40,6 +40,7 @@ SYMBOLS = [
     "dfe_batch_supported", "dfe_batch_fwd", "dfe_batch_bwd",
     "dfe_band_supported", "dfe_band_factor_bytes", "dfe_band_workspace_bytes", "dfe_band_factor", "dfe_band_fwd", "dfe_band_bwd",
     "dfe_band_npad", "dfe_band_solve",
+    "dfe_band_ps_supported", "dfe_band_ps_factor_bytes", "dfe_band_ps_workspace_bytes", "dfe_band_ps_fwd", "dfe_band_ps_bwd",
     "dfe_heat_supported", "dfe_heat_warps", "dfe_heat_grad_bytes", "dfe_heat_fwd", "dfe_heat_adj", "dfe_heat_grad",
     "dfe_heat_grad_sum",
 ]
@@ -214,6 +215,16 @@ def lib() -> C.CDLL:
     L.dfe_band_npad.argtypes = [vp]
     L.dfe_band_solve.restype = ci
     L.dfe_band_solve.argtypes = [vp, i64, vp, vp, vp]
+    L.dfe_band_ps_supported.restype = ci
+    L.dfe_band_ps_supported.argtypes = [vp]
+    L.dfe_band_ps_factor_bytes.restype = sz
+    L.dfe_band_ps_factor_bytes.argtypes = [vp, i64]
+    L.dfe_band_ps_workspace_bytes.restype = sz
+    L.dfe_band_ps_workspace_bytes.argtypes = [vp, i64]
+    L.dfe_band_ps_fwd.restype = ci
+    L.dfe_band_ps_fwd.argtypes = [vp, i64, vp, i64, vp, ci, vp, vp, i64, vp, vp, sz, vp]
+    L.dfe_band_ps_bwd.restype = ci
+    L.dfe_band_ps_bwd.argtypes = [vp, i64, vp, i64, vp, i64, vp, ci, vp, i64, vp, vp, sz, vp]
     L.dfe_heat_supported.restype = ci
     L.dfe_heat_supported.argtypes = [vp]
     L.dfe_heat_warps.restype = ci

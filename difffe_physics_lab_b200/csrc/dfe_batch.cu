@@ -481,9 +481,10 @@ __global__ void k_band_geom(const MeshDev M, double* __restrict__ geom) {
 // right-hand sides of the whole batch, (B, npad) row-major, rows >= n_free zero.
 // forward: one CTA per sample — f_b and the per-element terms (area/3) * (f_i+f_j+f_k)/3 (solver.py:143-145) in shared
 // memory, then every free row adds the terms of its adjacent elements in ascending element order and applies the
-// lifting in dict order (solver.py:165-169): the arithmetic of k_assemble / k_eliminate, bit for bit
+// lifting in dict order (solver.py:165-169): the arithmetic of k_assemble / k_eliminate, bit for bit.  Sample b reads its
+// matrix at vals_full + b * vstride (0: one matrix shared by the batch)
 __global__ void __launch_bounds__(BT) k_band_rhs_fwd(const MeshDev M, long long B, int npad, const double* __restrict__ f,
-                                                     long long ldf, const double* __restrict__ vals_full,
+                                                     long long ldf, const double* __restrict__ vals_full, long long vstride,
                                                      const double* __restrict__ geom, double* __restrict__ X) {
   extern __shared__ double sg[];
   double* sf = sg;               // [n_nodes]
@@ -510,7 +511,7 @@ __global__ void __launch_bounds__(BT) k_band_rhs_fwd(const MeshDev M, long long 
           v = __dadd_rn(v, M.dim == 1 ? __dmul_rn(geom[e], sf[node]) : st[e]);
         }
         for (int t = M.lift_ptr[r]; t < M.lift_ptr[r + 1]; ++t)
-          v = __dsub_rn(v, __dmul_rn(vals_full[M.lift_src[t]], M.lift_g[t]));   // solver.py:169
+          v = __dsub_rn(v, __dmul_rn(vals_full[b * vstride + M.lift_src[t]], M.lift_g[t]));   // solver.py:169
       }
       X[b * npad + r] = v;
     }
@@ -1400,6 +1401,44 @@ void dfe::band_frags(const dfe_mesh* m, const void* factor, const double** Ff, c
   *Bf = p.Bf;
 }
 
+void dfe::band_tables(const dfe_mesh* m, double* geom, double* geom2, cudaStream_t st) {
+  k_band_geom<<<nblk(m->dev.n_el, 128), 128, 0, st>>>(m->dev, geom);
+  k_band_tables<<<nblk(m->dev.n_el, 128), 128, 0, st>>>(m->dev, nullptr, 0, nullptr, geom2);
+}
+
+void dfe::band_rhs(const dfe_mesh* m, long long B, const double* f, long long ldf, const double* vals_full,
+                   long long vstride, const double* geom, double* X, cudaStream_t st) {
+  const size_t rsm = (static_cast<size_t>(m->dev.n_nodes) + m->dev.n_el) * sizeof(double);
+  cudaFuncSetAttribute(k_band_rhs_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(rsm));
+  long long rgrid = 8LL * m->sm_count;
+  if (rgrid > B) rgrid = B;
+  k_band_rhs_fwd<<<static_cast<unsigned>(rgrid), BT, rsm, st>>>(m->dev, B, band_npad(m), f, ldf, vals_full, vstride, geom, X);
+}
+
+int dfe::band_grad(const dfe_mesh* m, long long B, const double* X, const double* u, long long ldu, const double* geom,
+                   const double* geom2, int gk_per_elem, double* gk, double* gf, long long ldgf, cudaStream_t st) {
+  const int np = band_npad(m);
+  if (band_reg_fits(m)) {
+    const int nnp = (m->dev.n_nodes + 1) & ~1;
+    const size_t gsm2 = (4 * static_cast<size_t>(nnp) + m->dev.n_el + 4 + 2 * BNW) * sizeof(double);
+    cudaFuncSetAttribute(k_band_grad2, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(gsm2));
+    long long grid = 2LL * m->sm_count;
+    if (grid > B) grid = B;
+    k_band_grad2<<<static_cast<unsigned>(grid), BT, gsm2, st>>>(m->dev, B, np, X, u, ldu, geom2, gk, gk_per_elem, gf, ldgf, nnp);
+    return DFE_OK;
+  }
+  const size_t gsm = (2 * static_cast<size_t>(m->dev.n_nodes) + m->dev.n_el + 2 * BNW) * sizeof(double);
+  if (gsm > 200 * 1024) {
+    dfe::set_error("banded adjoint: mesh too large for the gradient kernel (%zu bytes of shared memory)", gsm);
+    return DFE_ERR_UNSUPPORTED;
+  }
+  cudaFuncSetAttribute(k_band_grad, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(gsm));
+  long long grid = 8LL * m->sm_count;
+  if (grid > B) grid = B;
+  k_band_grad<<<static_cast<unsigned>(grid), BT, gsm, st>>>(m->dev, B, np, X, u, ldu, geom, gk, gk_per_elem, gf, ldgf);
+  return DFE_OK;
+}
+
 // K_free = L L^T from the assembled matrix (dfe_assemble); `factor` holds dfe_band_factor_bytes(m) bytes.  The status
 // word (0 ok, 5 = a pivot <= 0: K_free is not SPD) is the int at the end of the buffer; *status_dev (optional, device)
 // receives a copy.  Asynchronous.
@@ -1476,11 +1515,7 @@ extern "C" int dfe_band_fwd(const dfe_mesh* m, int64_t B, const double* f, int64
         default: launch_rhs(k_band_rhs_fwd3<1, NST_F>, NST_F); break;
       }
     } else {
-      const size_t rsm = (static_cast<size_t>(m->dev.n_nodes) + m->dev.n_el) * sizeof(double);
-      cudaFuncSetAttribute(k_band_rhs_fwd, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(rsm));
-      long long rgrid = 8LL * m->sm_count;
-      if (rgrid > B) rgrid = B;
-      k_band_rhs_fwd<<<static_cast<unsigned>(rgrid), BT, rsm, st>>>(m->dev, B, np, f, ldf, vals_full, p.geom, X);
+      dfe::band_rhs(m, B, f, ldf, vals_full, 0, p.geom, X, st);
     }
     k_band_solve_mma<false, true><<<nblk(B, MMA_W * MMA_S), 32 * MMA_W, 0, st>>>(np, B, p.Ff, p.Bf, X, m->dev.free_nodes,
                                                                                  m->dev.n_free, nullptr, 0, u, ldu,
@@ -1518,7 +1553,6 @@ extern "C" int dfe_band_bwd(const dfe_mesh* m, int64_t B, const double* gbar, in
     double* X = static_cast<double*>(ws);
     k_band_solve_mma<true, false><<<nblk(B, MMA_W * MMA_S), 32 * MMA_W, 0, st>>>(np, B, p.Ff, p.Bf, X, m->dev.free_nodes,
                                                                                  m->dev.n_free, gbar, ldg, nullptr, 0, nullptr, nullptr, 0);
-    const size_t gsm = (2 * static_cast<size_t>(m->dev.n_nodes) + m->dev.n_el + 2 * BNW) * sizeof(double);
     if (kappa_mode == DFE_KAPPA_SCALAR && band_stencil_fits(m)) {
       const int nt = ((m->dev.n_nodes + SR - 1) / SR + 31) & ~31;
       double* gkpart = X + static_cast<size_t>(B) * np;
@@ -1545,26 +1579,11 @@ extern "C" int dfe_band_bwd(const dfe_mesh* m, int64_t B, const double* gbar, in
         }
       }
       k_band_gksum<<<nblk(B, 256), 256, 0, st>>>(B, nt / 32, gkpart, gkappa);
-    } else if (band_reg_fits(m)) {
-      const int nnp = (m->dev.n_nodes + 1) & ~1;
-      const size_t gsm2 = (4 * static_cast<size_t>(nnp) + m->dev.n_el + 4 + 2 * BNW) * sizeof(double);
-      cudaFuncSetAttribute(k_band_grad2, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(gsm2));
-      long long grid = 2LL * m->sm_count;
-      if (grid > B) grid = B;
-      k_band_grad2<<<static_cast<unsigned>(grid), BT, gsm2, st>>>(m->dev, B, np, X, u, ldu, p.geom2, gkappa,
-                                                                   kappa_mode == DFE_KAPPA_PER_ELEMENT, gf, ldgf, nnp);
-    } else if (gsm > 200 * 1024) {
-      dfe::set_error("dfe_band_bwd: mesh too large for the gradient kernel (%zu bytes of shared memory)", gsm);
-      rc = DFE_ERR_UNSUPPORTED;
     } else {
-      cudaFuncSetAttribute(k_band_grad, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(gsm));
-      long long grid = 8LL * m->sm_count;
-      if (grid > B) grid = B;
-      k_band_grad<<<static_cast<unsigned>(grid), BT, gsm, st>>>(m->dev, B, np, X, u, ldu, p.geom, gkappa,
-                                                                 kappa_mode == DFE_KAPPA_PER_ELEMENT, gf, ldgf);
+      rc = dfe::band_grad(m, B, X, u, ldu, p.geom, p.geom2, kappa_mode == DFE_KAPPA_PER_ELEMENT, gkappa, gf, ldgf, st);
     }
     cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) {
+    if (rc == DFE_OK && e != cudaSuccess) {
       dfe::set_error("dfe_band_bwd: kernel launch failed: %s", cudaGetErrorString(e));
       rc = DFE_ERR_CUDA;
     }

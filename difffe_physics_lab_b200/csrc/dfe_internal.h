@@ -76,6 +76,18 @@ int poison1d_launch(const dfe_mesh* m, double* out, long long ldo, long long B, 
 constexpr int BAND_FRAGD = 2048;
 void band_frags(const dfe_mesh* m, const void* factor, const double** Ff, const double** Bf);
 
+// pieces of the banded route (dfe_batch.cu) that the per-sample-kappa route (dfe_band_ps.cu) reuses, all asynchronous:
+//   band_tables  geom (8 * n_el) and geom2 (4 * n_el) per-element constants of a 2-D P1 mesh (k_band_geom, k_band_tables)
+//   band_rhs     X (B, npad) = lifted load of f in free numbering (k_band_rhs_fwd); sample b's matrix at
+//                vals_full + b * vstride
+//   band_grad    dL/dkappa (per element, or summed per sample) and dL/df (gf may be null) from lambda = X (k_band_grad2,
+//                else k_band_grad); DFE_ERR_UNSUPPORTED if neither fits
+void band_tables(const dfe_mesh* m, double* geom, double* geom2, cudaStream_t st);
+void band_rhs(const dfe_mesh* m, long long B, const double* f, long long ldf, const double* vals_full, long long vstride,
+              const double* geom, double* X, cudaStream_t st);
+int band_grad(const dfe_mesh* m, long long B, const double* X, const double* u, long long ldu, const double* geom,
+              const double* geom2, int gk_per_elem, double* gk, double* gf, long long ldgf, cudaStream_t st);
+
 }  // namespace dfe
 
 struct dfe_mesh {

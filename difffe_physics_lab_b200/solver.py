@@ -43,7 +43,7 @@ class KernelTimer:
     # kernels of libdfe_b200 launched per ABI call (default pipelined 1-D path: k1d_pipe_ck + k1d_pipe [+ k1d_pipe_gk]
     # + k1d_pipe_poison)
     KERNELS_PER_CALL = {"solve1d_fwd": 3, "solve1d_bwd": 4, "solve1d_bwd_misfit": 4, "batch_fwd": 1, "batch_bwd": 1, "band_factor": 1,
-                        "band_fwd": 3, "band_bwd": 3, "assemble": 1, "eliminate": 2, "pcg": 1, "scatter": 1,
+                        "band_fwd": 3, "band_bwd": 3, "band_ps_fwd": 7, "band_ps_bwd": 2, "assemble": 1, "eliminate": 2, "pcg": 1, "scatter": 1,
                         "gather": 1, "grad": 3, "mg_setup": 20, "mg_pcg": 1, "heat_fwd": 1, "heat_adj": 1,
                         "heat_grad": 2}
 
@@ -311,8 +311,15 @@ class _FESolve(torch.autograd.Function):
                 # many samples, one matrix: banded direct solver or one-CTA-per-sample PCG (config 5b)
                 if B >= int(opts.get("batch_min", 2)) and mode in (_native.KAPPA_SCALAR, _native.KAPPA_PER_ELEMENT):
                     ctx.batch = _batch_solver(L, nm, opts)
-                fwd = {"band": _band_forward, "pcg": _batch_forward, None: _general_forward}[ctx.batch]
-                saved_mats = fwd(L, nm, f, kappa, mode, u, opts)
+                # many samples, one matrix each: per-sample banded factorisations in batched kernels
+                elif (B >= int(opts.get("batch_min", 2)) and opts.get("batch_solver", "auto") in ("auto", "band")
+                      and L.dfe_band_ps_supported(nm.handle)):
+                    ctx.batch = "band_ps"
+                if ctx.batch == "band_ps":
+                    saved_mats = _band_ps_forward(L, nm, f, kappa, mode, u, opts, keep=any(ctx.needs_input_grad[:2]))
+                else:
+                    fwd = {"band": _band_forward, "pcg": _batch_forward, None: _general_forward}[ctx.batch]
+                    saved_mats = fwd(L, nm, f, kappa, mode, u, opts)
                 if out_host:
                     u_out = _to_host(u)
         ctx.mesh, ctx.mode, ctx.opts, ctx.fused, ctx.dev = mesh, mode, opts, fused, dev
@@ -380,6 +387,8 @@ class _FESolve(torch.autograd.Function):
                 gf = torch.empty_like(u) if need_f else None
                 if ctx.batch == "band":
                     _band_backward(L, nm, gbar, u, kappa, mode, ctx.mats, gf, gk, ctx.opts)
+                elif ctx.batch == "band_ps":
+                    _band_ps_backward(L, nm, gbar, u, mode, ctx.mats, gf, gk, ctx.opts)
                 elif ctx.batch == "pcg":
                     _batch_backward(L, nm, gbar, u, kappa, mode, ctx.mats, gf, gk, ctx.opts)
                 else:
@@ -520,6 +529,38 @@ def _band_backward(L, nm, gbar, u, kappa, mode, mats, gf, gk, opts):
                                      gk_b.data_ptr(), ws.data_ptr(), ws.numel(), st))
     opts["last_pcg_adjoint"] = [(0, 0.0)]
     gk.copy_(gk_b.sum(dim=0).reshape(gk.shape))   # torch.sum on CUDA is deterministic (no atomics)
+
+
+def _band_ps_forward(L, nm, f, kappa, mode, u, opts, keep):
+    """kappa (B, 1) or (B, n_el), half bandwidth <= 32: every sample's K_free(kappa_b) is assembled, factored and solved in
+    batched kernels (dfe_band_ps_fwd).  The factors are returned for the adjoint when ``keep`` (an input needs a gradient)."""
+    dev = f.device
+    B = f.shape[0]
+    st = _stream(dev)
+    factors = _ws(L.dfe_band_ps_factor_bytes(nm.handle, B), dev)
+    ws = _ws(L.dfe_band_ps_workspace_bytes(nm.handle, B), dev)
+    status = torch.empty(B, dtype=torch.int32, device=dev)
+    with _timed("band_ps_fwd", dev):
+        _native.check(L.dfe_band_ps_fwd(nm.handle, B, f.data_ptr(), f.stride(0), kappa.data_ptr(), mode, factors.data_ptr(),
+                                        u.data_ptr(), u.stride(0), status.data_ptr(), ws.data_ptr(), ws.numel(), st))
+    if int(status.max()) != 0:        # one synchronisation per call
+        b = int(torch.argmax(status))  # the first failing sample
+        raise _native.BreakdownError(_native.ERR_BREAKDOWN, f"dfe_band_ps_fwd: sample {b}: a pivot of the Cholesky "
+                                     "factorisation is <= 0: K_free(kappa_b) is not SPD — is kappa_b > 0?")
+    opts["last_pcg"] = [(0, 0.0)]     # direct solve: no iterations
+    return [("band_ps", factors)] if keep else None
+
+
+def _band_ps_backward(L, nm, gbar, u, mode, mats, gf, gk, opts):
+    dev = u.device
+    B = u.shape[0]
+    st = _stream(dev)
+    ws = _ws(L.dfe_band_ps_workspace_bytes(nm.handle, B), dev)
+    with _timed("band_ps_bwd", dev):
+        _native.check(L.dfe_band_ps_bwd(nm.handle, B, gbar.data_ptr(), gbar.stride(0), u.data_ptr(), u.stride(0),
+                                        mats[0][1].data_ptr(), mode, _ptr(gf), gf.stride(0) if gf is not None else nm.info.n_nodes,
+                                        gk.data_ptr(), ws.data_ptr(), ws.numel(), st))
+    opts["last_pcg_adjoint"] = [(0, 0.0)]
 
 
 def _batch_forward(L, nm, f, kappa, mode, u, opts):

@@ -251,6 +251,35 @@ int dfe_band_bwd(const dfe_mesh* m, int64_t B, const double* gbar, int64_t ldg, 
 int64_t dfe_band_npad(const dfe_mesh* m);
 int dfe_band_solve(const dfe_mesh* m, int64_t B, double* X, const void* factor, void* stream);
 
+/* ---------------------------------------------------------------- banded direct solver, one matrix per sample
+ * The same banded solve when every sample has its own conductivity: kappa[B] (DFE_KAPPA_PER_SAMPLE) or kappa[B * n_el]
+ * row-major (DFE_KAPPA_PER_SAMPLE_ELEMENT); any other mode gives DFE_ERR_INVALID.  Per sample: assembly of K(kappa_b)
+ * (bit-identical to dfe_assemble in the matching SCALAR / PER_ELEMENT mode), blocked banded Cholesky of K_free(kappa_b)
+ * (bit-identical to dfe_band_factor on that matrix), the lifted load, and two banded triangular solves.
+ *   dfe_band_ps_supported        1 for a 2-D P1 mesh with dfe_band_supported (the gradient kernels then fit)
+ *   dfe_band_ps_factor_bytes     (12 * n_el + B * npad * 33) * 8 bytes, npad = dfe_band_npad(m); 262 KB per sample at
+ *                                FEMesh.rectangle(32, 32) (npad 992), about 1.07 GB at B = 4096.  Layout, in doubles:
+ *                                  geom[8 * n_el] | geom2[4 * n_el]   per-element constants of the load / gradient kernels
+ *                                  then per sample b: invd[npad] | Lr[npad * 32]   (invd[i] = 1 / L_ii,
+ *                                  Lr[i * 32 + d - 1] = L[i][i - d]: the first npad * 33 doubles of a dfe_band_factor buffer)
+ *   dfe_band_ps_workspace_bytes  ws of both calls: B * (nnz_full + npad) doubles + npad * 33 int32
+ *   dfe_band_ps_fwd   fills `factors` and u (B, ldu); status[B] (device int32): 0 ok, 5 = a pivot failed the SPD test
+ *                     (pivot <= 1e-12 x its diagonal entry: K_free(kappa_b) is not SPD), sample by sample
+ *   dfe_band_ps_bwd   lambda_b = K_free(kappa_b)^{-1} gbar_b[free] with the factors of dfe_band_ps_fwd, then
+ *                     gkappa (same layout as kappa: -lambda_b^T K0_e u_b, per element or summed per sample) and
+ *                     gf = dL/df (B, ldgf; may be NULL)
+ *   Row strides ldf / ldu / ldg / ldgf are >= n_nodes (else DFE_ERR_INVALID); rows need only 8-byte alignment.  Both
+ *   calls are asynchronous on `stream`.
+ */
+int dfe_band_ps_supported(const dfe_mesh* m);
+size_t dfe_band_ps_factor_bytes(const dfe_mesh* m, int64_t B);
+size_t dfe_band_ps_workspace_bytes(const dfe_mesh* m, int64_t B);
+int dfe_band_ps_fwd(const dfe_mesh* m, int64_t B, const double* f, int64_t ldf, const double* kappa, int kappa_mode,
+                    void* factors, double* u, int64_t ldu, int32_t* status, void* ws, size_t ws_bytes, void* stream);
+int dfe_band_ps_bwd(const dfe_mesh* m, int64_t B, const double* gbar, int64_t ldg, const double* u, int64_t ldu,
+                    const void* factors, int kappa_mode, double* gf, int64_t ldgf, double* gkappa,
+                    void* ws, size_t ws_bytes, void* stream);
+
 /* ---------------------------------------------------------------- differentiable heat-equation rollouts
  * Backward Euler with the lumped mass, (M_L + dt K) u^{n+1} = M_L u^n + dt F, Dirichlet nodes held at the mesh's values,
  * for B states sharing one factor of A = M_L + dt K (dfe_band_factor), and its discrete adjoint.  In free numbering,
