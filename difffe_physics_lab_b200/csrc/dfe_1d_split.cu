@@ -550,9 +550,13 @@ __global__ void __launch_bounds__(ST, 2) k1d_pass2(const PS p) {
 constexpr int PR = 9;
 constexpr int PCH = PR * ST;   // 2304 nodes per chunk
 
+// Slots of elements that do not exist (element -1 of chunk 0, elements past the chunk) are never read: the row buffers
+// hold whatever the last bulk load or gradient staging left there — the neighbouring sample's kappa, a dL/dkappa of an
+// earlier sample — and an inf or NaN there would otherwise reach this sample through kdiv(k, 0, 0) = 0 * k.
+// e0: element n0-1+tb (kT[0]) exists; element n0+tb+j (kT[j+1]) exists iff j < nev.
 struct ChunkP {
   int n0, len, tb, nin, nst, nev, eA, ecnt, koff;
-  bool ownsL, ownsR;
+  bool ownsL, ownsR, e0;
 };
 __device__ __forceinline__ ChunkP make_chunk_pe(const PS& p, int c, int tid) {
   ChunkP k;
@@ -563,6 +567,7 @@ __device__ __forceinline__ ChunkP make_chunk_pe(const PS& p, int c, int tid) {
   k.nin = max(0, min(PR, min(k.len, p.nn - (p.bcR ? 1 : 0) - k.n0) - k.tb));
   k.nst = max(0, min(PR, k.len - k.tb));
   k.nev = max(0, min(PR, min(k.len, p.nn - 1 - k.n0) - k.tb));   // elements owned (right element of each node)
+  k.e0 = k.n0 + k.tb >= 1 && k.tb <= k.len && k.n0 + k.tb <= p.nn - 1;
   k.ownsL = p.bcL && c == 0 && tid == 0;
   k.ownsR = p.bcR && c == p.G - 1 && tid == (k.len - 1) / PR;
   // kappa elements held: e in [eA, eA+ecnt), slot j (element n0-1+j) lives at kS[2 + mk + j + koff]
@@ -648,7 +653,8 @@ __global__ void __launch_bounds__(ST, 2) k1d_pe_pass1(const PS p) {
         double v0 = BWD ? in : __dadd_rn(__dmul_rn(hp, in), __dmul_rn(hi, in));
         if (j == 0 && ck.ownsL) v0 = 0.0;
         v[j] = v0;
-        const double w = hi * (2.0 * __drcp_rn(kT[j + 1]));   // w_e = h_e/kappa_e (hs = h/2); 2 RN(1/k) == RN(2/k)
+        // w_e = h_e/kappa_e (hs = h/2); 2 RN(1/k) == RN(2/k)
+        const double w = (j < ck.nev) ? hi * (2.0 * __drcp_rn(kT[j + 1])) : 0.0;
         wv[j] = w;
         t.s += v0;
         t.w = fma(w, t.s, t.w);
@@ -660,10 +666,10 @@ __global__ void __launch_bounds__(ST, 2) k1d_pe_pass1(const PS p) {
     const Tri ex = cta_excl_scan_pe(t, wt, lane, warp, tot0);
     double S = ex.s, X = ex.x, W = ex.w;
     double a1 = 0, a2 = 0, a3 = 0, B1 = 0, B2 = 0, B3 = 0, Xt = 0;
-    double kp = kdiv(0.5 * kT[0], hsT[0], rhT[0]);
+    double kp = ck.e0 ? kdiv(0.5 * kT[0], hsT[0], rhT[0]) : 0.0;
 #pragma unroll
     for (int j = 0; j < PR; ++j) {
-      const double ki = kdiv(0.5 * kT[j + 1], hsT[j + 1], rhT[j + 1]);
+      const double ki = (j < ck.nev) ? kdiv(0.5 * kT[j + 1], hsT[j + 1], rhT[j + 1]) : 0.0;
       const double err = two_sum_err(kp, ki);
       kp = ki;
       S += v[j];
@@ -798,7 +804,7 @@ __global__ void __launch_bounds__(ST, 2) k1d_pe_pass2(const PS p) {
         double v0 = BWD ? in : __dadd_rn(__dmul_rn(hp, in), __dmul_rn(hi, in));
         if (j == 0 && ck.ownsL) v0 = 0.0;
         v[j] = v0;
-        const double ik = 2.0 * __drcp_rn(kT[j + 1]);   // == RN(2 / kappa_e)
+        const double ik = (j < ck.nev) ? 2.0 * __drcp_rn(kT[j + 1]) : 0.0;   // == RN(2 / kappa_e)
         ikv[j] = ik;
         const double w = hi * ik;   // w_e = h_e/kappa_e (hs = h/2)
         t.s += v0;
@@ -818,14 +824,14 @@ __global__ void __launch_bounds__(ST, 2) k1d_pe_pass2(const PS p) {
     Tri t1 = tri_id();
     {
       double S = ex.s, X = ex.x, W = ex.w;
-      double kp = kdiv(0.5 * kT[0], hsT[0], rhT[0]);
+      double kp = ck.e0 ? kdiv(0.5 * kT[0], hsT[0], rhT[0]) : 0.0;
 #pragma unroll
       for (int j = 0; j < PR; ++j) {
         S += v[j];
         const double x0 = fma(beta, X, alpha) - W;
         if (have_out) rin[mo + ck.tb + j] = x0;
         if (BWD) ge[j] = (j < ck.nev) ? (beta - S) * (uT[j + 1] - uT[j]) : 0.0;   // q0_e (u_{e+1}-u_e)
-        const double ki = kdiv(0.5 * kT[j + 1], hsT[j + 1], rhT[j + 1]);
+        const double ki = (j < ck.nev) ? kdiv(0.5 * kT[j + 1], hsT[j + 1], rhT[j + 1]) : 0.0;
         const double v1 = __dmul_rn(two_sum_err(kp, ki), x0);
         kp = ki;
         v[j] = v1;

@@ -28,6 +28,8 @@ What is restated, and where it comes from
   for the 1e-12 / 1e-9 parity bounds where the dense reference cannot run.
 * ``adjoint_and_grads``             autograd of solver.py:88-96, :139-145, :169
   + ``LinalgSolveExBackward0`` written in closed form (SURVEY §8a rows A7/A8).
+* ``forward_exact``/``grads_1d_exact``  1-D chains: the same solve and gradients kept in 50 digits until the
+  final rounding (dL/dkappa_e differences neighbouring values: at n_el ~ 1e5 the float64 version costs ~1e-12).
 * per-element kappa                 the reference loop with ``kappa`` replaced
   by ``kappa[e]`` at solver.py:88 / :139 (extension; the reference itself raises).
 """
@@ -241,8 +243,15 @@ def apply_bc(rowptr, col, vals, F, bc: Dict[int, float]):
 # --------------------------------------------------------------------------- solves
 def _thomas_decimal(a, d, c, b, prec=50):
     """Tridiagonal solve in ``prec``-digit decimal arithmetic (arbiter)."""
+    return np.array([float(v) for v in _thomas_decimal_exact(a, d, c, b, prec)])
+
+
+def _thomas_decimal_exact(a, d, c, b, prec=50):
+    """``_thomas_decimal`` without the final rounding: the ``prec``-digit solution as a list of Decimals."""
     getcontext().prec = prec
     n = len(d)
+    if n == 0:
+        return []
     a = [Decimal(float(v)) for v in a]
     d = [Decimal(float(v)) for v in d]
     c = [Decimal(float(v)) for v in c]
@@ -259,7 +268,7 @@ def _thomas_decimal(a, d, c, b, prec=50):
     x[-1] = bp[-1]
     for i in range(n - 2, -1, -1):
         x[i] = bp[i] - cp[i] * x[i + 1]
-    return np.array([float(v) for v in x])
+    return x
 
 
 def _is_tridiagonal(rowptr, col):
@@ -355,6 +364,60 @@ def adjoint_and_grads(nodes, elements, bc, kappa, u, gbar, exact=True):
         np.add.at(gf, el.ravel(), np.repeat(contrib, 3))
     assert gk.shape == (n_el,)
     return gk, gf, lam
+
+
+# ------------------------------------------------ 1-D gradients without float64 rounding
+def _tridiag_free(nodes, elements, bc, kappa, f):
+    """The float64 system K_free u_free = F_free of a 1-D chain as (free, lower, diagonal, upper, rhs)."""
+    import scipy.sparse as sp
+
+    rowptr, col, vals, F = assemble_csr(nodes, elements, kappa, f)
+    free, rp, cf, vf, Ff = apply_bc(rowptr, col, vals, F, bc)
+    assert _is_tridiagonal(rp, cf), "a 1-D chain has a tridiagonal K_free"
+    A = sp.csr_matrix((vf, cf, rp), shape=(len(free), len(free)))
+    lo = np.concatenate([[0.0], A.diagonal(-1)])
+    up = np.concatenate([A.diagonal(1), [0.0]])
+    return free, lo, A.diagonal(), up, Ff
+
+
+def forward_exact(nodes, elements, bc, kappa, f, prec=50):
+    """``forward`` on a 1-D chain, unrounded: the ``prec``-digit solution of the float64 system as a list of Decimals
+    (Dirichlet nodes hold their data exactly)."""
+    free, lo, d, up, rhs = _tridiag_free(nodes, elements, bc, kappa, f)
+    u = [Decimal(0)] * nodes.shape[0]
+    for k, g in bc.items():
+        u[k] = Decimal(float(g))
+    for i, v in zip(free, _thomas_decimal_exact(lo, d, up, rhs, prec)):
+        u[i] = v
+    return u
+
+
+def grads_1d_exact(nodes, elements, bc, kappa, u, gbar, prec=50):
+    """``adjoint_and_grads`` on a 1-D chain with every step after the float64 system in ``prec``-digit arithmetic.
+
+    ``u`` is a float64 vector (converted exactly: e.g. a kernel's stored solution) or the Decimal list of
+    ``forward_exact``.  Returns (gk, gf, lam): gk_e = -(lam_j - lam_i)(u_j - u_i)/h_e and
+    gf_i = sum_{e ∋ i} (h_e/2) lam_i, each formed from the unrounded lam and rounded once; lam is the ``prec``-digit adjoint
+    (list of Decimals, 0 on Dirichlet nodes).  The float64 ``adjoint_and_grads`` rounds lam and u first and differences the
+    rounded values: at n_el = 1e5 that alone moves gk by ~1e-12 relative (DESIGN.md §3.1b).
+    """
+    n = nodes.shape[0]
+    free, lo, d, up, rhs = _tridiag_free(nodes, elements, {k: 0.0 for k in bc}, kappa, np.zeros(n))
+    rhs = np.asarray(gbar, dtype=np.float64)[free]
+    getcontext().prec = prec
+    lam = [Decimal(0)] * n
+    for i, v in zip(free, _thomas_decimal_exact(lo, d, up, rhs, prec)):
+        lam[i] = v
+    ud = u if (len(u) and isinstance(u[0], Decimal)) else [Decimal(float(v)) for v in np.asarray(u, dtype=np.float64)]
+    h, _ = element_1d(nodes, elements, 1.0)
+    gk = np.empty(len(elements))
+    gf = [Decimal(0)] * n
+    for e, (i, j) in enumerate(elements.tolist()):
+        he = Decimal(float(h[e]))
+        gk[e] = float(-(lam[j] - lam[i]) * (ud[j] - ud[i]) / he)
+        gf[i] += he / 2 * lam[i]
+        gf[j] += he / 2 * lam[j]
+    return gk, np.array([float(v) for v in gf]), lam
 
 
 # ------------------------------------------------- reference Jacobi-PCG (2D timing)
