@@ -23,7 +23,8 @@ SOURCES = ["dfe_mesh.cu", "dfe_1d.cu", "dfe_1d_split.cu", "dfe_1d_pipe.cu", "dfe
            "dfe_batch.cu", "dfe_band_ps.cu", "dfe_heat.cu"]
 HEADERS = [PKG / "csrc" / "dfe_internal.h", PKG / "csrc" / "dfe_1d_common.cuh", PKG / "csrc" / "dfe_gridsync.cuh", PKG / "csrc" / "dfe_exact.cuh",
            PKG / "csrc" / "dfe_p2.cuh", PKG / "csrc" / "dfe_mg_kernel.cuh", PKG / "csrc" / "dfe_band_mma.cuh",
-           PKG / "csrc" / "dfe_assemble_row.cuh", ROOT / "include" / "dfe.h"]
+           PKG / "csrc" / "dfe_assemble_row.cuh", PKG / "csrc" / "dfe_band_ps_solve.cuh",
+           ROOT / "include" / "dfe.h"]
 
 OK, ERR_INVALID, ERR_CUDA, ERR_UNSUPPORTED, ERR_NOT_CONVERGED, ERR_BREAKDOWN, ERR_WORKSPACE = range(7)
 KAPPA_SCALAR, KAPPA_PER_SAMPLE, KAPPA_PER_ELEMENT, KAPPA_PER_SAMPLE_ELEMENT = range(4)
@@ -43,6 +44,8 @@ SYMBOLS = [
     "dfe_band_ps_supported", "dfe_band_ps_factor_bytes", "dfe_band_ps_workspace_bytes", "dfe_band_ps_fwd", "dfe_band_ps_bwd",
     "dfe_heat_supported", "dfe_heat_warps", "dfe_heat_grad_bytes", "dfe_heat_fwd", "dfe_heat_adj", "dfe_heat_grad",
     "dfe_heat_grad_sum",
+    "dfe_heat_ps_factor_bytes", "dfe_heat_ps_workspace_bytes", "dfe_heat_ps_setup", "dfe_heat_ps_fwd", "dfe_heat_ps_adj",
+    "dfe_heat_ps_grad", "dfe_heat_ps_grad_sum",
 ]
 
 
@@ -239,6 +242,20 @@ def lib() -> C.CDLL:
     L.dfe_heat_grad.argtypes = [vp, i64, i64, i64, i64, vp, i64, i64, vp, vp, sz, vp]
     L.dfe_heat_grad_sum.restype = ci
     L.dfe_heat_grad_sum.argtypes = [vp, i64, i64, dbl, ci, vp, vp, sz, vp]
+    L.dfe_heat_ps_factor_bytes.restype = sz
+    L.dfe_heat_ps_factor_bytes.argtypes = [vp, i64]
+    L.dfe_heat_ps_workspace_bytes.restype = sz
+    L.dfe_heat_ps_workspace_bytes.argtypes = [vp, i64]
+    L.dfe_heat_ps_setup.restype = ci
+    L.dfe_heat_ps_setup.argtypes = [vp, i64, vp, ci, dbl, vp, vp, vp, vp, vp, vp, sz, vp]
+    L.dfe_heat_ps_fwd.restype = ci
+    L.dfe_heat_ps_fwd.argtypes = [vp, i64, i64, vp, i64, vp, vp, vp, vp, vp, i64, i64, vp]
+    L.dfe_heat_ps_adj.restype = ci
+    L.dfe_heat_ps_adj.argtypes = [vp, i64, i64, i64, vp, i64, i64, i64, vp, vp, vp, vp, vp, vp]
+    L.dfe_heat_ps_grad.restype = ci
+    L.dfe_heat_ps_grad.argtypes = [vp, i64, i64, vp, vp, i64, i64, vp, vp, vp]
+    L.dfe_heat_ps_grad_sum.restype = ci
+    L.dfe_heat_ps_grad_sum.argtypes = [vp, i64, dbl, ci, vp, vp, vp]
     if L.dfe_abi_version() != 1:
         raise RuntimeError("libdfe_b200.so ABI version mismatch")
     _lib = L

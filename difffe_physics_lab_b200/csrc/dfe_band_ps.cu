@@ -8,6 +8,7 @@
 //                                  block rows are read straight from the sample's vals_full through the K_free pattern
 //   load          k_band_rhs_fwd   (dfe_batch.cu) with a per-sample vals_full stride for the lifting
 //   solve         k_bps_solve      L_b y = b, L_b^T x = y: one warp per sample, both sweeps, one read of L_b per sweep
+//                                  (bps_sweeps, dfe_band_ps_solve.cuh, shared with the per-sample heat rollout)
 //   gradients     k_band_grad2 / k_band_grad (dfe_batch.cu): they already write per-sample dL/dkappa and dL/df
 // Every reduction has a fixed order (no float atomics): the results are bit-reproducible and independent of B.
 #include "dfe_internal.h"
@@ -16,6 +17,7 @@ namespace {
 
 using dfe::MeshDev;
 #include "dfe_assemble_row.cuh"   // assemble_row: the per-sample matrices of dfe_assemble
+#include "dfe_band_ps_solve.cuh"  // bps_sweeps: both banded sweeps of one sample's factor by one warp
 
 constexpr int BW = 32;            // half bandwidth supported (as dfe_batch.cu)
 constexpr int FT = 128;           // threads per CTA of the factor kernel (one CTA per sample)
@@ -170,12 +172,10 @@ __global__ void __launch_bounds__(FT, 4) k_bps_factor(int n, int npad, const dou
   if (tid == 0) status[smp] = sbad ? 5 : 0;
 }
 
-// L_b y = b, L_b^T x = y for one right-hand side per factor: one warp per sample, lane a owns row 32k + a of block row k.
-// Per block row: the coupling to the previous (next) block row, 32 fmas per lane with the neighbour's solution broadcast
-// by shuffles, then the 32 dependent steps of the triangular diagonal block.  y stays in X between the sweeps (the lane
-// that wrote an entry reads it back).  GIN: the right-hand side is gathered from gsrc (B, ldg) through the free-node table
-// (the adjoint's gbar); SOUT: x is scattered into u (B, ldu) with the Dirichlet values (the forward solution); otherwise
-// both are in X (B, npad), free numbering.
+// L_b y = b, L_b^T x = y for one right-hand side per factor: one warp per sample, both sweeps of bps_sweeps
+// (dfe_band_ps_solve.cuh).  GIN: the right-hand side is gathered from gsrc (B, ldg) through the free-node table (the
+// adjoint's gbar); SOUT: x is scattered into u (B, ldu) with the Dirichlet values (the forward solution); otherwise both are
+// in X (B, npad), free numbering.
 template <bool GIN, bool SOUT>
 __global__ void __launch_bounds__(32 * SW_) k_bps_solve(const MeshDev M, long long B, int npad,
                                                         const double* __restrict__ fac, double* __restrict__ X,
@@ -185,62 +185,18 @@ __global__ void __launch_bounds__(32 * SW_) k_bps_solve(const MeshDev M, long lo
   const long long b = blockIdx.x * static_cast<long long>(SW_) + (threadIdx.x >> 5);
   if (b >= B) return;
   const double* invd = fac + b * (static_cast<long long>(npad) * (BW + 1));
-  const double* Lr = invd + npad;
   double* x = X + b * npad;
-  const int nb = npad >> 5, n = M.n_free;
-  double prev = 0.0;   // lane c: entry c of the solution of the block row just finished
-  for (int k = 0; k < nb; ++k) {
-    const int i = 32 * k + lane;
-    const double* Li = Lr + static_cast<size_t>(i) * BW;   // Li[d - 1] = L[i][i - d]
-    double acc;
-    if (GIN) acc = i < n ? gsrc[b * ldg + M.free_nodes[i]] : 0.0;
-    else acc = x[i];
-    if (k > 0) {
-#pragma unroll
-      for (int c = 0; c < 32; ++c) {   // L[i][32(k-1) + c], d = 32 + lane - c
-        const double yc = __shfl_sync(FULL, prev, c);
-        if (c >= lane) acc = fma(-Li[31 + lane - c], yc, acc);
-      }
-    }
-    const double inv = invd[i];
-    double y = 0.0;
-#pragma unroll
-    for (int j = 0; j < 32; ++j) {     // L[i][32k + j], d = lane - j
-      const double yj = __shfl_sync(FULL, acc * inv, j);
-      if (lane == j) y = yj;
-      if (lane > j) acc = fma(-Li[lane - j - 1], yj, acc);
-    }
-    x[i] = y;
-    prev = y;
-  }
-  prev = 0.0;
-  for (int k = nb - 1; k >= 0; --k) {
-    const int i = 32 * k + lane;
-    double acc = x[i];
-    if (k + 1 < nb) {
-      const double* Ln = Lr + static_cast<size_t>(32 * (k + 1)) * BW;
-#pragma unroll
-      for (int c = 0; c < 32; ++c) {   // L[32(k+1) + c][i], d = 32 + c - lane
-        const double xc = __shfl_sync(FULL, prev, c);
-        if (c <= lane) acc = fma(-Ln[c * BW + 31 + c - lane], xc, acc);
-      }
-    }
-    const double inv = invd[i];
-    const double* Lk = Lr + static_cast<size_t>(32 * k) * BW;
-    double xv = 0.0;
-#pragma unroll
-    for (int j = 31; j >= 0; --j) {    // L[32k + j][i], d = j - lane
-      const double xj = __shfl_sync(FULL, acc * inv, j);
-      if (lane == j) xv = xj;
-      if (lane < j) acc = fma(-Lk[j * BW + (j - lane) - 1], xj, acc);
-    }
-    if (SOUT) {
-      if (i < n) uout[b * ldu + M.free_nodes[i]] = xv;
-    } else {
-      x[i] = xv;
-    }
-    prev = xv;
-  }
+  const int n = M.n_free;
+  bps_sweeps(
+      invd, invd + npad, x, npad >> 5, lane,
+      [&](int i) { return GIN ? (i < n ? gsrc[b * ldg + M.free_nodes[i]] : 0.0) : x[i]; },
+      [&](int i, double xv) {
+        if (SOUT) {
+          if (i < n) uout[b * ldu + M.free_nodes[i]] = xv;
+        } else {
+          x[i] = xv;
+        }
+      });
   if (SOUT)
     for (int d = lane; d < M.n_dir; d += 32) uout[b * ldu + M.dir_idx[d]] = M.dir_val[d];   // solver.py:177-179
 }
@@ -271,6 +227,19 @@ int ps_enter(const dfe_mesh* m, const char* who, int* prev) {
 }
 
 }  // namespace
+
+void dfe::band_ps_assemble(const dfe_mesh* m, long long B, const double* kappa, int per_elem, double* vals,
+                           cudaStream_t st) {
+  const dim3 ag(nblk(m->dev.n_nodes, 128), static_cast<unsigned>(B < 65535 ? B : 65535));
+  k_bps_assemble<<<ag, 128, 0, st>>>(m->dev, B, kappa, per_elem, vals);
+}
+
+void dfe::band_ps_factor(const dfe_mesh* m, long long B, const double* vals, long long vstride, int* bidx, double* fac,
+                         int* status, cudaStream_t st) {
+  const int np = static_cast<int>(dfe_band_npad(m));
+  k_bps_bidx<<<nblk(np, 128), 128, 0, st>>>(m->dev, np, bidx);
+  k_bps_factor<<<static_cast<unsigned>(B), FT, 0, st>>>(m->dev.n_free, np, vals, vstride, bidx, fac, status);
+}
 
 extern "C" int dfe_band_ps_supported(const dfe_mesh* m) { return ps_fits(m) ? 1 : 0; }
 
@@ -311,10 +280,8 @@ extern "C" int dfe_band_ps_fwd(const dfe_mesh* m, int64_t B, const double* f, in
     double* X = vals + static_cast<size_t>(B) * m->dev.nnz_full;
     int* bidx = reinterpret_cast<int*>(X + static_cast<size_t>(B) * np);
     dfe::band_tables(m, geom, geom2, st);
-    k_bps_bidx<<<nblk(np, 128), 128, 0, st>>>(m->dev, np, bidx);
-    const dim3 ag(nblk(m->dev.n_nodes, 128), static_cast<unsigned>(B < 65535 ? B : 65535));
-    k_bps_assemble<<<ag, 128, 0, st>>>(m->dev, B, kappa, kappa_mode == DFE_KAPPA_PER_SAMPLE_ELEMENT, vals);
-    k_bps_factor<<<static_cast<unsigned>(B), FT, 0, st>>>(m->dev.n_free, np, vals, m->dev.nnz_full, bidx, fac, status);
+    dfe::band_ps_assemble(m, B, kappa, kappa_mode == DFE_KAPPA_PER_SAMPLE_ELEMENT, vals, st);
+    dfe::band_ps_factor(m, B, vals, m->dev.nnz_full, bidx, fac, status, st);
     dfe::band_rhs(m, B, f, ldf, vals, m->dev.nnz_full, geom, X, st);
     k_bps_solve<false, true><<<nblk(B, SW_), 32 * SW_, 0, st>>>(m->dev, B, np, fac, X, nullptr, 0, u, ldu);
     cudaError_t e = cudaGetLastError();

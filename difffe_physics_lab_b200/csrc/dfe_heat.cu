@@ -26,6 +26,18 @@
 //               kappa) in a fixed order.
 //
 // float64 throughout, no float atomics, every wait bounded.
+//
+// Per-sample conductivity (kappa (B, 1) or (B, n_el)): one A_b = M_L + dt K(kappa_b) and one factor per sample, so the
+// shared B operand of the tensor-core TRSM does not exist; the same recursions run with one warp per sample instead.
+// k_hps_shift   A_b = fl(dt K_b), then + M_L on the diagonal: the operations and order of timestepping._HeatOperator, so
+//               each A_b is bit-identical to its A (K_b from k_bps_assemble, the factor from k_bps_factor: dfe_band_ps.cu)
+// k_hps_cfree   c_b = fl(dt F_free) - (A_b g)_free, the lifting added in the mesh's fixed dict order (lift_ptr / lift_src)
+// k_hps_roll    the whole time loop (or one checkpoint segment) in ONE launch, one warp per sample: both sweeps of
+//               bps_sweeps per step with the right-hand side formed at load time (fma(m, x_n, c_b) forward,
+//               fma(m, lambda_{n+1}, gbar_n[free]) adjoint).  Warps never communicate: no barrier, no wait, no fault word.
+// k_hps_grad    gacc (B, n_el) += lam~^T K0_e u, one step at a time in DESCENDING step order (the order the adjoint
+//               produces them, within and across checkpoint segments): bit-identical with and without checkpointing, and
+//               independent of B.  k_hps_gsum scales by -dt (per element) or sums each sample's elements in a fixed order.
 #include "dfe_internal.h"
 
 namespace {
@@ -33,6 +45,7 @@ namespace {
 using dfe::MeshDev;
 #include "dfe_1d_common.cuh"   // mbarrier / 1-D TMA bulk copy wrappers
 #include "dfe_band_mma.cuh"     // block-row step of the tensor-core band solve and its fragment layout
+#include "dfe_band_ps_solve.cuh"  // bps_sweeps: both banded sweeps of one sample's factor by one warp
 
 constexpr double AREA_EPS = 1e-15;          // solver.py:120
 constexpr long long WAIT_POLLS = 1LL << 24; // try_wait polls before a fragment stage counts as lost (raises the fault word)
@@ -416,6 +429,203 @@ int roll_launch(const dfe_mesh* m, int warps, RollArgs a, const void* factor, cu
   return DFE_OK;
 }
 
+// ---------------------------------------------------------------------------------------------- per-sample conductivity
+constexpr int PSW = 4;   // warps per CTA of k_hps_roll (one warp per sample)
+
+// vals (B, nnz_full): K_b -> A_b = fl(dt K_b), then fl(A_b + mass) on the diagonal; thread (p, b) owns row p of sample b
+__global__ void k_hps_shift(const MeshDev M, long long B, double dt, const double* __restrict__ mass,
+                            double* __restrict__ vals) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= M.n_nodes) return;
+  for (long long b = blockIdx.y; b < B; b += gridDim.y) {
+    double* vb = vals + b * M.nnz_full;
+    for (int k = M.rowptr[p]; k < M.rowptr[p + 1]; ++k) {
+      const double v = __dmul_rn(dt, vb[k]);   // no contraction: two roundings, as float(dt) * vals; A[diag] += mass
+      vb[k] = M.col[k] == p ? __dadd_rn(v, mass[p]) : v;
+    }
+  }
+}
+
+// c (B, npad): c_b[r] = fl(dt F[node r]) - sum_k fl(A_b[lift_src[k]] g_k) in the mesh's dict order, zero for r >= n_free
+__global__ void k_hps_cfree(const MeshDev M, long long B, int npad, double dt, const double* __restrict__ load,
+                            const double* __restrict__ vals, double* __restrict__ c) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= npad) return;
+  for (long long b = blockIdx.y; b < B; b += gridDim.y) {
+    double v = 0.0;
+    if (r < M.n_free) {
+      const double* vb = vals + b * M.nnz_full;
+      double lift = 0.0;
+      for (int k = M.lift_ptr[r]; k < M.lift_ptr[r + 1]; ++k) lift = __dadd_rn(lift, __dmul_rn(vb[M.lift_src[k]], M.lift_g[k]));
+      v = __dsub_rn(__dmul_rn(dt, load ? load[M.free_nodes[r]] : 0.0), lift);
+    }
+    c[b * npad + r] = v;
+  }
+}
+
+struct PsRollArgs {
+  int npad, nfree, n_dir, nt;       // nt: time steps of this launch
+  long long B;
+  const double* fac;                // (B, npad * 33) per-sample factors of k_bps_factor
+  const int* fnode;
+  const int* dir_idx;
+  const double* dir_val;
+  const double* mf;                 // (npad) lumped mass on the free rows, zero-padded
+  const double* cf;                 // forward: (B, npad) c_b, zero-padded
+  double* X;                        // (B, npad) carry: x_n (forward) / lambda_{n+1} (adjoint); y between the two sweeps
+  const double* u0;                 // forward: (B, .) node-layout initial states, or null: X already holds x_0
+  long long ldu0;
+  double* traj;                     // forward: state after local step j at traj + b * ld_b + j * ld_t (node layout)
+  long long ld_b, ld_t;
+  const double* gbar;               // adjoint: dL/du_n at gbar + b * ldg_b + (n / gev - 1) * ldg_t when n % gev == 0
+  long long ldg_b, ldg_t;
+  int gev, n0;                      // adjoint: steps n0 + nt down to n0 + 1
+  double* lam;                      // adjoint: (nt, B, npad); slot j holds lambda_{n0 + 1 + j}
+  double* lsum;                     // adjoint: (B, npad) running sum of lambda_n
+};
+
+template <bool ADJ>
+__global__ void __launch_bounds__(32 * PSW) k_hps_roll(const PsRollArgs a) {
+  const int lane = threadIdx.x & 31;
+  const long long b = blockIdx.x * static_cast<long long>(PSW) + (threadIdx.x >> 5);
+  if (b >= a.B) return;
+  const int npad = a.npad, nb = npad >> 5, n = a.nfree;
+  const double* invd = a.fac + b * (static_cast<long long>(npad) * 33);
+  const double* Lr = invd + npad;
+  double* x = a.X + b * npad;
+  if (!ADJ && a.u0 != nullptr)   // x_0 = u0[free]: each lane the rows it owns in the sweeps
+    for (int i = lane; i < npad; i += 32) x[i] = i < n ? a.u0[b * a.ldu0 + a.fnode[i]] : 0.0;
+  for (int it = 0; it < a.nt; ++it) {
+    if (!ADJ) {
+      const double* cb = a.cf + b * npad;
+      double* urow = a.traj + b * a.ld_b + it * a.ld_t;
+      bps_sweeps(
+          invd, Lr, x, nb, lane, [&](int i) { return fma(a.mf[i], x[i], cb[i]); },
+          [&](int i, double xv) {
+            x[i] = xv;
+            if (i < n) urow[a.fnode[i]] = xv;
+          });
+      for (int d = lane; d < a.n_dir; d += 32) urow[a.dir_idx[d]] = a.dir_val[d];
+    } else {
+      const int step = a.n0 + a.nt - it;
+      const double* gs = (a.gbar != nullptr && step % a.gev == 0)
+                             ? a.gbar + b * a.ldg_b + static_cast<long long>(step / a.gev - 1) * a.ldg_t
+                             : nullptr;
+      double* lrow = a.lam + (static_cast<long long>(a.nt - 1 - it) * a.B + b) * npad;
+      double* srow = a.lsum + b * npad;
+      bps_sweeps(
+          invd, Lr, x, nb, lane,
+          [&](int i) { return fma(a.mf[i], x[i], (gs != nullptr && i < n) ? gs[a.fnode[i]] : 0.0); },
+          [&](int i, double xv) {
+            x[i] = xv;
+            lrow[i] = xv;
+            srow[i] += xv;
+          });
+    }
+  }
+}
+
+struct PsGradArgs {
+  int n_el, npad, n_seg;
+  long long B;
+  const double* u;      // state after local step j of sample b: u + b * ld_b + j * ld_t (node layout)
+  long long ld_b, ld_t;
+  const double* lam;    // (n_seg, B, npad)
+  const double* K0;     // (n_el, 6)
+  const int4* eidx;     // (n_el, 2)
+  double* gacc;         // (B, n_el) running sums
+};
+
+// thread (e, b): gacc[b][e] += lam~_j^T K0_e u_j for j = n_seg - 1 down to 0, one step at a time
+__global__ void k_hps_grad(const PsGradArgs a) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= a.n_el) return;
+  const int4 in = a.eidx[2 * e], ir = a.eidx[2 * e + 1];
+  const double2 k01 = *reinterpret_cast<const double2*>(a.K0 + 6 * static_cast<size_t>(e));
+  const double2 k23 = *reinterpret_cast<const double2*>(a.K0 + 6 * static_cast<size_t>(e) + 2);
+  const double2 k45 = *reinterpret_cast<const double2*>(a.K0 + 6 * static_cast<size_t>(e) + 4);
+  const int npad = a.npad;
+  for (long long b = blockIdx.y; b < a.B; b += gridDim.y) {
+    double acc = a.gacc[b * a.n_el + e];
+    for (int j = a.n_seg - 1; j >= 0; --j) {
+      const double* su = a.u + b * a.ld_b + j * a.ld_t;
+      const double* sl = a.lam + (j * a.B + b) * npad;
+      const double u0 = su[in.x], u1 = su[in.y], u2 = su[in.z];
+      const double ku0 = fma(k01.x, u0, fma(k01.y, u1, k23.x * u2));   // k00 u0 + k01 u1 + k02 u2
+      const double ku1 = fma(k01.y, u0, fma(k23.y, u1, k45.x * u2));   // k01 u0 + k11 u1 + k12 u2
+      const double ku2 = fma(k23.x, u0, fma(k45.x, u1, k45.y * u2));   // k02 u0 + k12 u1 + k22 u2
+      const double l0 = ir.x < npad ? sl[ir.x] : 0.0, l1 = ir.y < npad ? sl[ir.y] : 0.0, l2 = ir.z < npad ? sl[ir.z] : 0.0;
+      acc += fma(l0, ku0, fma(l1, ku1, l2 * ku2));
+    }
+    a.gacc[b * a.n_el + e] = acc;
+  }
+}
+
+// SUM = false: gk (B, n_el) = -dt gacc;  SUM = true: gk[b] = sum_e (-dt gacc[b][e]) by one CTA of 256 threads per sample in
+// a fixed order (the reduction of k_heat_sum1)
+template <bool SUM>
+__global__ void __launch_bounds__(256) k_hps_gsum(int n_el, long long B, double mdt, const double* __restrict__ gacc,
+                                                  double* __restrict__ gk) {
+  if (!SUM) {
+    const long long i = blockIdx.x * 256LL + threadIdx.x;
+    if (i < B * n_el) gk[i] = mdt * gacc[i];
+    return;
+  }
+  __shared__ double sh[256];
+  const double* g = gacc + static_cast<long long>(blockIdx.x) * n_el;
+  double s = 0.0;
+  for (int i = threadIdx.x; i < n_el; i += 256) s += mdt * g[i];
+  sh[threadIdx.x] = s;
+  __syncthreads();
+  for (int d = 128; d > 0; d >>= 1) {
+    if (threadIdx.x < d) sh[threadIdx.x] += sh[threadIdx.x + d];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) gk[blockIdx.x] = sh[0];
+}
+
+size_t hps_sample(const dfe_mesh* m) { return static_cast<size_t>(dfe_band_npad(m)) * 33; }   // doubles of one factor
+
+int hps_enter(const dfe_mesh* m, const char* who, int* prev) {
+  if (!m) {
+    dfe::set_error("%s: mesh is null", who);
+    return DFE_ERR_INVALID;
+  }
+  if (m->info.device < 0) {
+    dfe::set_error("%s: mesh handle is host-only; no CUDA device (this library has no CPU path)", who);
+    return DFE_ERR_CUDA;
+  }
+  if (!dfe_band_ps_supported(m)) {
+    dfe::set_error("%s: needs a 2-D P1 mesh whose K_free has half bandwidth <= 32 (dfe_band_ps_supported)", who);
+    return DFE_ERR_UNSUPPORTED;
+  }
+  DFE_CUDA_OK(cudaGetDevice(prev));
+  if (*prev != m->info.device) DFE_CUDA_OK(cudaSetDevice(m->info.device));
+  return DFE_OK;
+}
+
+int launch_status(const char* who) {
+  const cudaError_t e = cudaGetLastError();
+  if (e == cudaSuccess) return DFE_OK;
+  dfe::set_error("%s: kernel launch failed: %s", who, cudaGetErrorString(e));
+  return DFE_ERR_CUDA;
+}
+
+inline unsigned ygrid(long long B) { return static_cast<unsigned>(B < 65535 ? B : 65535); }
+
+template <bool ADJ>
+int hps_roll_launch(const dfe_mesh* m, PsRollArgs a, const void* factors, cudaStream_t st, const char* who) {
+  a.npad = static_cast<int>(dfe_band_npad(m));
+  a.nfree = m->dev.n_free;
+  a.n_dir = m->dev.n_dir;
+  a.fnode = m->dev.free_nodes;
+  a.dir_idx = m->dev.dir_idx;
+  a.dir_val = m->dev.dir_val;
+  a.fac = static_cast<const double*>(factors) + 10 * static_cast<size_t>(m->dev.n_el);
+  k_hps_roll<ADJ><<<nblk(a.B, PSW), 32 * PSW, 0, st>>>(a);
+  return launch_status(who);
+}
+
 }  // namespace
 
 extern "C" int dfe_heat_supported(const dfe_mesh* m) { return heat_fits(m) ? 1 : 0; }
@@ -560,6 +770,158 @@ extern "C" int dfe_heat_grad_sum(const dfe_mesh* m, int64_t B, int64_t n_total, 
       dfe::set_error("dfe_heat_grad_sum: kernel launch failed: %s", cudaGetErrorString(e));
       rc = DFE_ERR_CUDA;
     }
+  }
+  if (prev != m->info.device) cudaSetDevice(prev);
+  return rc;
+}
+
+// ---------------------------------------------------------------------------------------------- per-sample conductivity
+extern "C" size_t dfe_heat_ps_factor_bytes(const dfe_mesh* m, int64_t B) {
+  if (!dfe_band_ps_supported(m) || B < 1) return 0;
+  return (10 * static_cast<size_t>(m->dev.n_el) + static_cast<size_t>(B) * hps_sample(m)) * sizeof(double);
+}
+
+extern "C" size_t dfe_heat_ps_workspace_bytes(const dfe_mesh* m, int64_t B) {
+  if (!dfe_band_ps_supported(m) || B < 1) return 0;
+  // A (B, nnz_full) doubles | bidx (npad, 33) int32
+  return static_cast<size_t>(B) * m->dev.nnz_full * sizeof(double) + hps_sample(m) * sizeof(int);
+}
+
+extern "C" int dfe_heat_ps_setup(const dfe_mesh* m, int64_t B, const double* kappa, int kappa_mode, double dt,
+                                 const double* mass, const double* load, void* factors, double* c_free, int32_t* status,
+                                 void* ws, size_t ws_bytes, void* stream) {
+  int prev;
+  int rc = hps_enter(m, "dfe_heat_ps_setup", &prev);
+  if (rc) return rc;
+  if (!kappa || !mass || !factors || !c_free || !status || !ws || B < 1 || !al16(factors)) {
+    dfe::set_error("dfe_heat_ps_setup: null / invalid argument (factors must be 16-byte aligned)");
+    rc = DFE_ERR_INVALID;
+  } else if (kappa_mode != DFE_KAPPA_PER_SAMPLE && kappa_mode != DFE_KAPPA_PER_SAMPLE_ELEMENT) {
+    dfe::set_error("dfe_heat_ps_setup: kappa_mode must be PER_SAMPLE or PER_SAMPLE_ELEMENT");
+    rc = DFE_ERR_INVALID;
+  } else if (ws_bytes < dfe_heat_ps_workspace_bytes(m, B)) {
+    dfe::set_error("dfe_heat_ps_setup: workspace %zu bytes < required %zu", ws_bytes, dfe_heat_ps_workspace_bytes(m, B));
+    rc = DFE_ERR_WORKSPACE;
+  } else {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int np = static_cast<int>(dfe_band_npad(m)), ne = m->dev.n_el;
+    double* K0 = static_cast<double*>(factors);
+    double* fac = K0 + 10 * static_cast<size_t>(ne);
+    double* A = static_cast<double*>(ws);
+    int* bidx = reinterpret_cast<int*>(A + static_cast<size_t>(B) * m->dev.nnz_full);
+    k_heat_tables<<<nblk(ne, 128), 128, 0, st>>>(m->dev, np, K0, reinterpret_cast<int4*>(K0 + 6 * static_cast<size_t>(ne)));
+    dfe::band_ps_assemble(m, B, kappa, kappa_mode == DFE_KAPPA_PER_SAMPLE_ELEMENT, A, st);
+    k_hps_shift<<<dim3(nblk(m->dev.n_nodes, 128), ygrid(B)), 128, 0, st>>>(m->dev, B, dt, mass, A);
+    k_hps_cfree<<<dim3(nblk(np, 128), ygrid(B)), 128, 0, st>>>(m->dev, B, np, dt, load, A, c_free);
+    dfe::band_ps_factor(m, B, A, m->dev.nnz_full, bidx, fac, status, st);
+    rc = launch_status("dfe_heat_ps_setup");
+  }
+  if (prev != m->info.device) cudaSetDevice(prev);
+  return rc;
+}
+
+extern "C" int dfe_heat_ps_fwd(const dfe_mesh* m, int64_t B, int64_t n_steps, const double* u0, int64_t ldu0,
+                               const void* factors, const double* m_free, const double* c_free, double* X, double* traj,
+                               int64_t ld_b, int64_t ld_t, void* stream) {
+  int prev;
+  int rc = hps_enter(m, "dfe_heat_ps_fwd", &prev);
+  if (rc) return rc;
+  if (!factors || !m_free || !c_free || !X || !traj || B < 1 || n_steps < 1 || n_steps > (1LL << 30)) {
+    dfe::set_error("dfe_heat_ps_fwd: null / invalid argument");
+    rc = DFE_ERR_INVALID;
+  } else {
+    PsRollArgs a{};
+    a.B = B;
+    a.nt = static_cast<int>(n_steps);
+    a.mf = m_free;
+    a.cf = c_free;
+    a.X = X;
+    a.u0 = u0;
+    a.ldu0 = ldu0;
+    a.traj = traj;
+    a.ld_b = ld_b;
+    a.ld_t = ld_t;
+    rc = hps_roll_launch<false>(m, a, factors, static_cast<cudaStream_t>(stream), "dfe_heat_ps_fwd");
+  }
+  if (prev != m->info.device) cudaSetDevice(prev);
+  return rc;
+}
+
+extern "C" int dfe_heat_ps_adj(const dfe_mesh* m, int64_t B, int64_t n0, int64_t n_steps, const double* gbar,
+                               int64_t ldg_b, int64_t ldg_t, int64_t g_every, const void* factors, const double* m_free,
+                               double* X, double* lam, double* lam_sum, void* stream) {
+  int prev;
+  int rc = hps_enter(m, "dfe_heat_ps_adj", &prev);
+  if (rc) return rc;
+  if (!factors || !m_free || !X || !lam || !lam_sum || B < 1 || n0 < 0 || n_steps < 1 || n0 + n_steps > (1LL << 30) ||
+      (gbar && g_every < 1)) {
+    dfe::set_error("dfe_heat_ps_adj: null / invalid argument");
+    rc = DFE_ERR_INVALID;
+  } else {
+    PsRollArgs a{};
+    a.B = B;
+    a.nt = static_cast<int>(n_steps);
+    a.mf = m_free;
+    a.X = X;
+    a.gbar = gbar;
+    a.ldg_b = ldg_b;
+    a.ldg_t = ldg_t;
+    a.gev = gbar ? static_cast<int>(g_every) : 1;
+    a.n0 = static_cast<int>(n0);
+    a.lam = lam;
+    a.lsum = lam_sum;
+    rc = hps_roll_launch<true>(m, a, factors, static_cast<cudaStream_t>(stream), "dfe_heat_ps_adj");
+  }
+  if (prev != m->info.device) cudaSetDevice(prev);
+  return rc;
+}
+
+extern "C" int dfe_heat_ps_grad(const dfe_mesh* m, int64_t B, int64_t n_seg, const void* factors, const double* u,
+                                int64_t ld_b, int64_t ld_t, const double* lam, double* gacc, void* stream) {
+  int prev;
+  int rc = hps_enter(m, "dfe_heat_ps_grad", &prev);
+  if (rc) return rc;
+  if (!factors || !u || !lam || !gacc || B < 1 || n_seg < 1 || n_seg > (1LL << 30)) {
+    dfe::set_error("dfe_heat_ps_grad: null / invalid argument");
+    rc = DFE_ERR_INVALID;
+  } else {
+    const int ne = m->dev.n_el;
+    PsGradArgs a{};
+    a.n_el = ne;
+    a.npad = static_cast<int>(dfe_band_npad(m));
+    a.n_seg = static_cast<int>(n_seg);
+    a.B = B;
+    a.u = u;
+    a.ld_b = ld_b;
+    a.ld_t = ld_t;
+    a.lam = lam;
+    a.K0 = static_cast<const double*>(factors);
+    a.eidx = reinterpret_cast<const int4*>(a.K0 + 6 * static_cast<size_t>(ne));
+    a.gacc = gacc;
+    k_hps_grad<<<dim3(nblk(ne, 128), ygrid(B)), 128, 0, static_cast<cudaStream_t>(stream)>>>(a);
+    rc = launch_status("dfe_heat_ps_grad");
+  }
+  if (prev != m->info.device) cudaSetDevice(prev);
+  return rc;
+}
+
+extern "C" int dfe_heat_ps_grad_sum(const dfe_mesh* m, int64_t B, double dt, int kappa_mode, const double* gacc,
+                                    double* gkappa, void* stream) {
+  int prev;
+  int rc = hps_enter(m, "dfe_heat_ps_grad_sum", &prev);
+  if (rc) return rc;
+  if (!gacc || !gkappa || B < 1 || B > 0x7fffffffLL) {
+    dfe::set_error("dfe_heat_ps_grad_sum: null / invalid argument");
+    rc = DFE_ERR_INVALID;
+  } else if (kappa_mode != DFE_KAPPA_PER_SAMPLE && kappa_mode != DFE_KAPPA_PER_SAMPLE_ELEMENT) {
+    dfe::set_error("dfe_heat_ps_grad_sum: kappa_mode must be PER_SAMPLE or PER_SAMPLE_ELEMENT");
+    rc = DFE_ERR_INVALID;
+  } else {
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int ne = m->dev.n_el;
+    if (kappa_mode == DFE_KAPPA_PER_SAMPLE) k_hps_gsum<true><<<static_cast<unsigned>(B), 256, 0, st>>>(ne, B, -dt, gacc, gkappa);
+    else k_hps_gsum<false><<<nblk(B * ne, 256), 256, 0, st>>>(ne, B, -dt, gacc, gkappa);
+    rc = launch_status("dfe_heat_ps_grad_sum");
   }
   if (prev != m->info.device) cudaSetDevice(prev);
   return rc;

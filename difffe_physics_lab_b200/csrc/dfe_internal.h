@@ -88,6 +88,14 @@ void band_rhs(const dfe_mesh* m, long long B, const double* f, long long ldf, co
 int band_grad(const dfe_mesh* m, long long B, const double* X, const double* u, long long ldu, const double* geom,
               const double* geom2, int gk_per_elem, double* gk, double* gf, long long ldgf, cudaStream_t st);
 
+// pieces of the per-sample-kappa route (dfe_band_ps.cu) that the per-sample heat rollouts (dfe_heat.cu) reuse, asynchronous:
+//   band_ps_assemble  vals (B, nnz_full) = K(kappa_b) of every sample (k_bps_assemble); kappa[B] or kappa[B * n_el]
+//   band_ps_factor    fac (B, npad * 33) = the banded Cholesky factor of the matrix at vals + b * vstride, sample by
+//                     sample, and status[B] (k_bps_bidx into bidx (npad * 33 int32), k_bps_factor)
+void band_ps_assemble(const dfe_mesh* m, long long B, const double* kappa, int per_elem, double* vals, cudaStream_t st);
+void band_ps_factor(const dfe_mesh* m, long long B, const double* vals, long long vstride, int* bidx, double* fac,
+                    int* status, cudaStream_t st);
+
 }  // namespace dfe
 
 struct dfe_mesh {

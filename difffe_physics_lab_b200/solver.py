@@ -45,7 +45,8 @@ class KernelTimer:
     KERNELS_PER_CALL = {"solve1d_fwd": 3, "solve1d_bwd": 4, "solve1d_bwd_misfit": 4, "batch_fwd": 1, "batch_bwd": 1, "band_factor": 1,
                         "band_fwd": 3, "band_bwd": 3, "band_ps_fwd": 7, "band_ps_bwd": 2, "assemble": 1, "eliminate": 2, "pcg": 1, "scatter": 1,
                         "gather": 1, "grad": 3, "mg_setup": 20, "mg_pcg": 1, "heat_fwd": 1, "heat_adj": 1,
-                        "heat_grad": 2}
+                        "heat_grad": 2, "heat_ps_setup": 6, "heat_ps_fwd": 1, "heat_ps_adj": 1, "heat_ps_grad": 1,
+                        "heat_ps_grad_sum": 1}
 
     def __init__(self):
         self.events = []

@@ -12,7 +12,8 @@ states per step (block TRSM on the FP64 tensor cores).  Meshes: half bandwidth o
 
 ``DifferentiableHeatSolver`` runs the same scheme as a differentiable rollout: the whole time loop is one kernel launch
 (``dfe_heat_fwd``), and the backward is the discrete adjoint in time (``dfe_heat_adj``, ``dfe_heat_grad``) with optional
-checkpointing.  Gradients flow to ``u0``, ``kappa`` and ``f``.
+checkpointing.  Gradients flow to ``u0``, ``kappa`` and ``f``.  With one conductivity per sample (kappa ``(B, 1)`` or
+``(B, n_el)``) every sample has its own factor and the rollout runs one warp per sample (``dfe_heat_ps_*``).
 """
 from __future__ import annotations
 
@@ -111,8 +112,9 @@ class HeatStepper:
         return out
 
 
-def _heat_check_mesh(mesh: FEMesh, dev: torch.device):
-    """NotImplementedError (with the reason) for meshes the differentiable rollout does not take; returns the native mesh."""
+def _heat_check_mesh(mesh: FEMesh, dev: torch.device, per_sample: bool = False):
+    """NotImplementedError (with the reason) for meshes the differentiable rollout does not take; returns the native mesh.
+    ``per_sample``: the per-sample-kappa route, whose gradient kernel has no shared-memory bound (dfe_band_ps_supported)."""
     if mesh.dim != 2:
         raise NotImplementedError("DifferentiableHeatSolver supports 2-D meshes only (1-D meshes are not implemented)")
     if mesh.order != 1:
@@ -122,10 +124,16 @@ def _heat_check_mesh(mesh: FEMesh, dev: torch.device):
     if not L.dfe_band_supported(nm.handle):
         raise NotImplementedError("DifferentiableHeatSolver needs a mesh whose K_free has half bandwidth <= 32 "
                                   "(dfe_band_supported; e.g. rectangle(nx, ny) with nx <= 32)")
-    if not L.dfe_heat_supported(nm.handle):
+    if not per_sample and not L.dfe_heat_supported(nm.handle):
         raise NotImplementedError("mesh too large for the trajectory gradient kernel: the per-element sums and three "
                                   "(u, lambda) rows must fit 200 KB of shared memory (dfe_heat_supported)")
     return nm
+
+
+def _per_sample_kappa(kappa, n_el: int) -> bool:
+    """True for the 2-D kappa forms that give every sample its own conductivity.  (1, 1), (1, n_el) and (n_el, 1) keep the
+    shared meaning they had before per-sample kappa existed (the values are flattened)."""
+    return torch.is_tensor(kappa) and kappa.dim() == 2 and kappa.shape[0] > 1 and tuple(kappa.shape) != (n_el, 1)
 
 
 def _check_status(status: torch.Tensor, fault: torch.Tensor, who: str) -> None:
@@ -137,31 +145,159 @@ def _check_status(status: torch.Tensor, fault: torch.Tensor, who: str) -> None:
         raise _native.DfeError(_native.ERR_CUDA, f"{who}: a bounded wait inside a rollout kernel expired; outputs invalid")
 
 
+class _SharedRoute:
+    """kappa shared by the batch: one factor of A = M_L + dt K(kappa), the tensor-core rollout kernels (dfe_heat_*)."""
+
+    def __init__(self, mesh, kappa, dt, f, dev, B, warps):
+        self.op = op = _HeatOperator(mesh, kappa, dt, f, dev)
+        self.h, self.npad, self.free, self.mass_free = op.nm.handle, op.npad, op.free, op.mass_free
+        self.dt, self.warps, self.dev, self.B = dt, warps, dev, B
+        nf = op.free.numel()
+        self.mf = torch.zeros(self.npad, dtype=torch.float64, device=dev)
+        self.cf = torch.zeros(self.npad, dtype=torch.float64, device=dev)
+        self.mf[:nf], self.cf[:nf] = op.mass_free, op.rhs_const
+        self.fault = torch.zeros(1, dtype=torch.int32, device=dev)
+
+    def check(self, who):
+        _check_status(self.op.status, self.fault, who)
+
+    def fwd(self, src, X, traj, steps):
+        st = torch.cuda.current_stream(self.dev).cuda_stream
+        with _timed("heat_fwd", self.dev):
+            _native.check(_native.lib().dfe_heat_fwd(
+                self.h, self.B, steps, None if src is None else src.data_ptr(), traj.shape[-1], self.op.factor.data_ptr(),
+                self.mf.data_ptr(), self.cf.data_ptr(), X.data_ptr(), traj.data_ptr(), traj.stride(0), traj.stride(1),
+                self.warps, self.fault.data_ptr(), st))
+
+    def begin_backward(self, N):
+        self.N = N
+        self.fault = torch.zeros(1, dtype=torch.int32, device=self.dev)
+        self.gws = torch.empty(max(int(_native.lib().dfe_heat_grad_bytes(self.h, self.B, N)), 16), dtype=torch.uint8,
+                               device=self.dev)
+
+    def adj(self, n0, ln, gout, every, Xa, lam, lsum):
+        st = torch.cuda.current_stream(self.dev).cuda_stream
+        with _timed("heat_adj", self.dev):
+            _native.check(_native.lib().dfe_heat_adj(
+                self.h, self.B, n0, ln, gout.data_ptr(), gout.stride(0), gout.stride(1), every, self.op.factor.data_ptr(),
+                self.mf.data_ptr(), Xa.data_ptr(), lam.data_ptr(), lsum.data_ptr(), self.warps, self.fault.data_ptr(), st))
+
+    def grad(self, n0, ln, traj, lam):
+        st = torch.cuda.current_stream(self.dev).cuda_stream
+        with _timed("heat_grad", self.dev):
+            _native.check(_native.lib().dfe_heat_grad(self.h, self.B, n0, ln, self.N, traj.data_ptr(), traj.stride(0),
+                                                      traj.stride(1), lam.data_ptr(), self.gws.data_ptr(), self.gws.numel(), st))
+
+    def gkappa(self, kappa):
+        st = torch.cuda.current_stream(self.dev).cuda_stream
+        gk = torch.empty(kappa.numel(), dtype=torch.float64, device=self.dev)
+        mode = _native.KAPPA_SCALAR if kappa.numel() == 1 else _native.KAPPA_PER_ELEMENT
+        with _timed("heat_grad", self.dev):
+            _native.check(_native.lib().dfe_heat_grad_sum(self.h, self.B, self.N, self.dt, mode, gk.data_ptr(),
+                                                          self.gws.data_ptr(), self.gws.numel(), st))
+        return gk
+
+    def finish_backward(self, who):
+        _check_status(torch.zeros(1, dtype=torch.int32, device=self.dev), self.fault, who)
+
+
+class _PerSampleRoute:
+    """kappa (B, 1) or (B, n_el): one A_b = M_L + dt K(kappa_b) and one banded factor per sample (dfe_heat_ps_*), one
+    warp per sample in the rollout kernels.  The factors take npad * 33 doubles per sample."""
+
+    def __init__(self, mesh, kappa, dt, f, dev, B):
+        L = _native.lib()
+        nm = mesh._native(dev.index)
+        I = nm.info
+        self.h, self.npad, self.dt, self.dev, self.B = nm.handle, int(L.dfe_band_npad(nm.handle)), dt, dev, B
+        self.n_el = I.n_elements
+        self.mode = _native.KAPPA_PER_SAMPLE if kappa.shape[1] == 1 else _native.KAPPA_PER_SAMPLE_ELEMENT
+        st = torch.cuda.current_stream(dev).cuda_stream
+        one = torch.ones(1, dtype=torch.float64, device=dev)
+        vals = torch.empty(max(I.nnz_full, 1), dtype=torch.float64, device=dev)
+        mass = torch.empty(I.n_nodes, dtype=torch.float64, device=dev)   # M_L and F do not depend on kappa
+        _native.check(L.dfe_assemble(nm.handle, one.data_ptr(), _native.KAPPA_SCALAR,
+                                     torch.ones(I.n_nodes, dtype=torch.float64, device=dev).data_ptr(), vals.data_ptr(),
+                                     mass.data_ptr(), st))
+        load = None
+        if f is not None:
+            load = torch.empty(I.n_nodes, dtype=torch.float64, device=dev)
+            fs = f.to(device=dev, dtype=torch.float64).contiguous()
+            _native.check(L.dfe_assemble(nm.handle, one.data_ptr(), _native.KAPPA_SCALAR, fs.data_ptr(), vals.data_ptr(),
+                                         load.data_ptr(), st))
+        self.free = torch.as_tensor(np.asarray(mesh.free_nodes(), dtype=np.int64), device=dev)
+        self.mass_free = mass[self.free]
+        self.mf = torch.zeros(self.npad, dtype=torch.float64, device=dev)
+        self.mf[:self.free.numel()] = self.mass_free
+        self.factors = torch.empty(max(int(L.dfe_heat_ps_factor_bytes(nm.handle, B)), 16), dtype=torch.uint8, device=dev)
+        self.cf = torch.empty((B, self.npad), dtype=torch.float64, device=dev)
+        self.status = torch.empty(B, dtype=torch.int32, device=dev)
+        ws = torch.empty(max(int(L.dfe_heat_ps_workspace_bytes(nm.handle, B)), 16), dtype=torch.uint8, device=dev)
+        with _timed("heat_ps_setup", dev):
+            _native.check(L.dfe_heat_ps_setup(nm.handle, B, kappa.data_ptr(), self.mode, dt, mass.data_ptr(),
+                                              None if load is None else load.data_ptr(), self.factors.data_ptr(),
+                                              self.cf.data_ptr(), self.status.data_ptr(), ws.data_ptr(), ws.numel(), st))
+
+    def check(self, who):
+        bad = self.status.cpu().nonzero()                   # the one synchronisation of a forward call
+        if bad.numel():
+            raise _native.BreakdownError(_native.ERR_BREAKDOWN, f"{who}: sample {int(bad[0, 0])}: M_L + dt K(kappa_b) is "
+                                         "not positive definite (kappa_b <= 0?)")
+
+    def fwd(self, src, X, traj, steps):
+        st = torch.cuda.current_stream(self.dev).cuda_stream
+        with _timed("heat_ps_fwd", self.dev):
+            _native.check(_native.lib().dfe_heat_ps_fwd(
+                self.h, self.B, steps, None if src is None else src.data_ptr(), traj.shape[-1], self.factors.data_ptr(),
+                self.mf.data_ptr(), self.cf.data_ptr(), X.data_ptr(), traj.data_ptr(), traj.stride(0), traj.stride(1), st))
+
+    def begin_backward(self, N):
+        self.gacc = torch.zeros((self.B, self.n_el), dtype=torch.float64, device=self.dev)   # running sums, zeroed
+
+    def adj(self, n0, ln, gout, every, Xa, lam, lsum):
+        st = torch.cuda.current_stream(self.dev).cuda_stream
+        with _timed("heat_ps_adj", self.dev):
+            _native.check(_native.lib().dfe_heat_ps_adj(
+                self.h, self.B, n0, ln, gout.data_ptr(), gout.stride(0), gout.stride(1), every, self.factors.data_ptr(),
+                self.mf.data_ptr(), Xa.data_ptr(), lam.data_ptr(), lsum.data_ptr(), st))
+
+    def grad(self, n0, ln, traj, lam):
+        st = torch.cuda.current_stream(self.dev).cuda_stream
+        with _timed("heat_ps_grad", self.dev):
+            _native.check(_native.lib().dfe_heat_ps_grad(self.h, self.B, ln, self.factors.data_ptr(), traj.data_ptr(),
+                                                         traj.stride(0), traj.stride(1), lam.data_ptr(),
+                                                         self.gacc.data_ptr(), st))
+
+    def gkappa(self, kappa):
+        st = torch.cuda.current_stream(self.dev).cuda_stream
+        gk = torch.empty(kappa.shape[0] if self.mode == _native.KAPPA_PER_SAMPLE else kappa.shape, dtype=torch.float64,
+                         device=self.dev)
+        with _timed("heat_ps_grad_sum", self.dev):
+            _native.check(_native.lib().dfe_heat_ps_grad_sum(self.h, self.B, self.dt, self.mode, self.gacc.data_ptr(),
+                                                             gk.data_ptr(), st))
+        return gk
+
+    def finish_backward(self, who):
+        pass                                                # no waits inside the per-sample kernels: nothing to check
+
+
 class _HeatRollout(torch.autograd.Function):
-    """(u0 (B, n), kappa (1,) or (n_el,), f (n,) or None) -> the states after steps every, 2 every, ..., N: (B, N / every, n).
+    """(u0 (B, n), kappa, f (n,) or None) -> the states after steps every, 2 every, ..., N: (B, N / every, n).  kappa is
+    (1,) or (n_el,) (shared by the batch) or, with ``per_sample``, (B, 1) or (B, n_el).
 
     All tensors are float64 and contiguous on the solver's device."""
 
     @staticmethod
-    def forward(ctx, u0, kappa, f, solver, n_steps: int, every: int):
-        L = _native.lib()
+    def forward(ctx, u0, kappa, f, solver, n_steps: int, every: int, per_sample: bool = False):
         dev, mesh, dt, c = u0.device, solver.mesh, solver.dt, solver.checkpoint
         B, n, N = u0.shape[0], mesh.n_nodes, n_steps
-        st = torch.cuda.current_stream(dev).cuda_stream
-        op = _HeatOperator(mesh, kappa.detach(), dt, None if f is None else f.detach(), dev)
-        h, npad, nf = op.nm.handle, op.npad, op.free.numel()
-        mf = torch.zeros(npad, dtype=torch.float64, device=dev)
-        cf = torch.zeros(npad, dtype=torch.float64, device=dev)
-        mf[:nf], cf[:nf] = op.mass_free, op.rhs_const
-        fault = torch.zeros(1, dtype=torch.int32, device=dev)
-        X = torch.zeros((B, npad), dtype=torch.float64, device=dev)
-        w = solver._cta_warps
+        fd = None if f is None else f.detach()
+        rt = _PerSampleRoute(mesh, kappa.detach(), dt, fd, dev, B) if per_sample \
+            else _SharedRoute(mesh, kappa.detach(), dt, fd, dev, B, solver._cta_warps)
+        X = torch.zeros((B, rt.npad), dtype=torch.float64, device=dev)
 
         def roll(src, traj, steps):
-            with _timed("heat_fwd", dev):
-                _native.check(L.dfe_heat_fwd(h, B, steps, None if src is None else src.data_ptr(), n, op.factor.data_ptr(),
-                                             mf.data_ptr(), cf.data_ptr(), X.data_ptr(), traj.data_ptr(), traj.stride(0),
-                                             traj.stride(1), w, fault.data_ptr(), st))
+            rt.fwd(src, X, traj, steps)
 
         if c is None:                                       # every state kept: the trajectory is the saved state
             traj = torch.empty((B, N, n), dtype=torch.float64, device=dev)
@@ -181,8 +317,8 @@ class _HeatRollout(torch.autograd.Function):
                 if s + ln < N:
                     starts.append(seg[:, ln - 1].clone())
             saved = torch.stack(starts)
-        _check_status(op.status, fault, "DifferentiableHeatSolver")
-        ctx.op, ctx.mf, ctx.solver, ctx.N, ctx.every, ctx.kmode = op, mf, solver, N, every, kappa.numel()
+        rt.check("DifferentiableHeatSolver")
+        ctx.rt, ctx.solver, ctx.N, ctx.every = rt, solver, N, every
         ctx.need_f = f is not None
         ctx.save_for_backward(saved, kappa)
         return out
@@ -191,65 +327,49 @@ class _HeatRollout(torch.autograd.Function):
     def backward(ctx, gout):
         L = _native.lib()
         saved, kappa = ctx.saved_tensors
-        op, mf, solver, N, every = ctx.op, ctx.mf, ctx.solver, ctx.N, ctx.every
-        mesh, dt, c, w = solver.mesh, solver.dt, solver.checkpoint, solver._cta_warps
+        rt, solver, N, every = ctx.rt, ctx.solver, ctx.N, ctx.every
+        mesh, dt, c = solver.mesh, solver.dt, solver.checkpoint
         dev = saved.device
-        h, npad, nf, n = op.nm.handle, op.npad, op.free.numel(), mesh.n_nodes
+        h, npad, nf, n = rt.h, rt.npad, rt.free.numel(), mesh.n_nodes
         B = saved.shape[0] if c is None else saved.shape[1]
         st = torch.cuda.current_stream(dev).cuda_stream
         gout = gout.to(dtype=torch.float64).contiguous()
-        fault = torch.zeros(1, dtype=torch.int32, device=dev)
         Xa = torch.zeros((B, npad), dtype=torch.float64, device=dev)       # lambda_{n+1}, zero above step N
         lsum = torch.zeros((B, npad), dtype=torch.float64, device=dev)
-        gws = torch.empty(max(int(L.dfe_heat_grad_bytes(h, B, N)), 16), dtype=torch.uint8, device=dev)
+        rt.begin_backward(N)
 
         def adjoint(n0, ln, lam):
-            with _timed("heat_adj", dev):
-                _native.check(L.dfe_heat_adj(h, B, n0, ln, gout.data_ptr(), gout.stride(0), gout.stride(1), every,
-                                             op.factor.data_ptr(), mf.data_ptr(), Xa.data_ptr(), lam.data_ptr(),
-                                             lsum.data_ptr(), w, fault.data_ptr(), st))
-
-        def grad(n0, ln, traj, lam):
-            with _timed("heat_grad", dev):
-                _native.check(L.dfe_heat_grad(h, B, n0, ln, N, traj.data_ptr(), traj.stride(0), traj.stride(1),
-                                              lam.data_ptr(), gws.data_ptr(), gws.numel(), st))
+            rt.adj(n0, ln, gout, every, Xa, lam, lsum)
 
         if c is None:
             lam = torch.empty((N, B, npad), dtype=torch.float64, device=dev)
             adjoint(0, N, lam)
-            grad(0, N, saved, lam)
+            rt.grad(0, N, saved, lam)
         else:
-            cf = torch.zeros(npad, dtype=torch.float64, device=dev)
-            cf[:nf] = op.rhs_const
             Xs = torch.empty((B, npad), dtype=torch.float64, device=dev)
             seg = torch.empty((B, min(c, N), n), dtype=torch.float64, device=dev)
             lam = torch.empty((min(c, N), B, npad), dtype=torch.float64, device=dev)
             for i in reversed(range(saved.shape[0])):
                 s = i * c
                 ln = min(c, N - s)
-                with _timed("heat_fwd", dev):                 # recompute the segment's states from its first one
-                    _native.check(L.dfe_heat_fwd(h, B, ln, saved[i].data_ptr(), n, op.factor.data_ptr(), mf.data_ptr(),
-                                                 cf.data_ptr(), Xs.data_ptr(), seg.data_ptr(), seg.stride(0),
-                                                 seg.stride(1), w, fault.data_ptr(), st))
+                rt.fwd(saved[i], Xs, seg, ln)               # recompute the segment's states from its first one
                 adjoint(s, ln, lam)
-                grad(s, ln, seg, lam)
-        gk = torch.empty(ctx.kmode, dtype=torch.float64, device=dev)
-        mode = _native.KAPPA_SCALAR if ctx.kmode == 1 else _native.KAPPA_PER_ELEMENT
-        with _timed("heat_grad", dev):
-            _native.check(L.dfe_heat_grad_sum(h, B, N, dt, mode, gk.data_ptr(), gws.data_ptr(), gws.numel(), st))
+                rt.grad(s, ln, seg, lam)
+        gk = rt.gkappa(kappa)
         gu0 = torch.zeros((B, n), dtype=torch.float64, device=dev)
-        gu0[:, op.free] = op.mass_free * Xa[:, :nf]          # dL/du0[free] = m * lambda_1
+        gu0[:, rt.free] = rt.mass_free * Xa[:, :nf]          # dL/du0[free] = m * lambda_1
         gf = None
         if ctx.need_f:                                      # dL/df = W^T (dt sum_n sum_b lam~_n)
             lt = torch.zeros(n, dtype=torch.float64, device=dev)
-            lt[op.free] = dt * lsum[:, :nf].sum(0)
+            lt[rt.free] = dt * lsum[:, :nf].sum(0)
             gf = torch.empty(n, dtype=torch.float64, device=dev)
             scratch = torch.empty(mesh.n_elements, dtype=torch.float64, device=dev)
-            with _timed("grad", dev):
-                _native.check(L.dfe_grad(h, lt.data_ptr(), lt.data_ptr(), kappa.data_ptr(), _native.KAPPA_PER_ELEMENT,
+            kg = torch.ones(mesh.n_elements, dtype=torch.float64, device=dev) if isinstance(rt, _PerSampleRoute) else kappa
+            with _timed("grad", dev):                       # (gf does not depend on kappa; scratch takes dL/dkappa)
+                _native.check(L.dfe_grad(h, lt.data_ptr(), lt.data_ptr(), kg.data_ptr(), _native.KAPPA_PER_ELEMENT,
                                          scratch.data_ptr(), gf.data_ptr(), None, 0, st))
-        _check_status(torch.zeros(1, dtype=torch.int32, device=dev), fault, "DifferentiableHeatSolver.backward")
-        return gu0, gk.reshape(kappa.shape), gf, None, None, None
+        rt.finish_backward("DifferentiableHeatSolver.backward")
+        return gu0, gk.reshape(kappa.shape), gf, None, None, None, None
 
 
 class DifferentiableHeatSolver(nn.Module):
@@ -265,7 +385,15 @@ class DifferentiableHeatSolver(nn.Module):
     Parameters
     ----------
     mesh : FEMesh         2-D P1, ``K_free`` of half bandwidth <= 32 (``rectangle(nx, ny)``, nx <= 32)
-    kappa : number or tensor ``()`` / ``(1,)`` / ``(n_elements,)``, shared by the batch, differentiable
+    kappa : number or tensor, differentiable; ``kappa.grad`` has ``kappa``'s shape
+        ``()`` / ``(1,)`` / ``(n_elements,)``: shared by the batch (also ``(1, 1)``, ``(1, n_elements)`` and
+        ``(n_elements, 1)``, which are flattened);
+        ``(B, 1)`` / ``(B, n_elements)``: one scalar / one field per sample; ``u0`` must then be ``(B, n_nodes)`` with the
+        same B.  When B = n_elements, ``(B, 1)`` keeps its shared meaning: pass per-sample scalars as ``(B, n_elements)``
+        with constant rows.  Every sample gets its own ``M_L + dt K(kappa_b)`` and banded factor, ``npad * 33`` doubles
+        (262 KB at ``rectangle(32, 32)``, 1.07 GB at B = 4096) kept for the backward; a sample whose matrix is not SPD
+        raises ``BreakdownError`` naming the first such sample.  The trajectory and lambda buffers are those of the
+        shared route.
     dt : float            not differentiable
     f : None or ``(n_nodes,)`` source, shared by the batch, differentiable
     checkpoint : keyword-only, None (keep every state for the backward) or c: keep every c-th state and recompute each
@@ -285,7 +413,8 @@ class DifferentiableHeatSolver(nn.Module):
                                "(difffe_physics_lab_b200 has no CPU fallback)")
         if checkpoint is not None and int(checkpoint) < 1:
             raise ValueError(f"checkpoint must be None or >= 1, got {checkpoint}")
-        _heat_check_mesh(mesh, torch.device("cuda", torch.cuda.current_device()))
+        _heat_check_mesh(mesh, torch.device("cuda", torch.cuda.current_device()),
+                         per_sample=_per_sample_kappa(kappa, mesh.n_elements))
         self.mesh, self.dt = mesh, float(dt)
         self.checkpoint = None if checkpoint is None else int(checkpoint)
         self.kappa = torch.tensor(float(kappa), dtype=torch.float64) if isinstance(kappa, (int, float)) else kappa
@@ -301,19 +430,27 @@ class DifferentiableHeatSolver(nn.Module):
             raise ValueError(f"n_steps ({n_steps}) must be a positive multiple of every ({every})")
         if u0.dim() not in (1, 2) or u0.shape[-1] != mesh.n_nodes:
             raise ValueError(f"u0 must have shape (n_nodes,) or (B, n_nodes) with n_nodes={mesh.n_nodes}, got {tuple(u0.shape)}")
-        kap = torch.as_tensor(self.kappa, dtype=torch.float64).reshape(-1) if not torch.is_tensor(self.kappa) \
-            else self.kappa.to(dtype=torch.float64).reshape(-1)
-        if kap.numel() not in (1, mesh.n_elements):
-            raise ValueError(f"kappa must have 1 or n_elements={mesh.n_elements} entries, got {kap.numel()}")
+        per_sample = _per_sample_kappa(self.kappa, mesh.n_elements)
+        if per_sample:
+            ks = tuple(self.kappa.shape)
+            if u0.dim() != 2 or ks[0] != u0.shape[0] or ks[1] not in (1, mesh.n_elements):
+                raise ValueError(f"per-sample kappa must be (B, 1) or (B, n_elements={mesh.n_elements}) with u0 of shape "
+                                 f"(B, n_nodes); got kappa {ks} and u0 {tuple(u0.shape)}")
+            kap = self.kappa.to(dtype=torch.float64)
+        else:
+            kap = torch.as_tensor(self.kappa, dtype=torch.float64).reshape(-1) if not torch.is_tensor(self.kappa) \
+                else self.kappa.to(dtype=torch.float64).reshape(-1)
+            if kap.numel() not in (1, mesh.n_elements):
+                raise ValueError(f"kappa must have 1 or n_elements={mesh.n_elements} entries, got {kap.numel()}")
         if self.f is not None and tuple(self.f.shape) != (mesh.n_nodes,):
             raise ValueError(f"f must have shape ({mesh.n_nodes},), got {tuple(self.f.shape)}")
         dev = u0.device if u0.is_cuda else torch.device("cuda", torch.cuda.current_device())
-        _heat_check_mesh(mesh, dev)
+        _heat_check_mesh(mesh, dev, per_sample=per_sample)
         batched = u0.dim() == 2
         u = u0.to(device=dev, dtype=torch.float64).reshape(-1, mesh.n_nodes).contiguous()
         fd = None if self.f is None else self.f.to(device=dev, dtype=torch.float64).contiguous()
         with torch.cuda.device(dev):
-            U = _HeatRollout.apply(u, kap.to(dev).contiguous(), fd, self, n_steps, k)
+            U = _HeatRollout.apply(u, kap.to(dev).contiguous(), fd, self, n_steps, k, per_sample)
         if every is None:
             U = U[:, 0]
         if not batched:

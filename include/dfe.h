@@ -320,6 +320,49 @@ int dfe_heat_grad(const dfe_mesh* m, int64_t B, int64_t n0, int64_t n_seg, int64
 int dfe_heat_grad_sum(const dfe_mesh* m, int64_t B, int64_t n_total, double dt, int kappa_mode, double* gkappa, void* ws,
                       size_t ws_bytes, void* stream);
 
+/* ---------------------------------------------------------------- heat-equation rollouts, one conductivity per sample
+ * The rollouts above when every sample has its own conductivity: kappa[B] (DFE_KAPPA_PER_SAMPLE) or kappa[B * n_el]
+ * row-major (DFE_KAPPA_PER_SAMPLE_ELEMENT); any other mode gives DFE_ERR_INVALID.  Per sample b, in free numbering,
+ *   A_b = M_L + dt K(kappa_b),   c_b = dt F_free - (A_b g)_free
+ *   forward   A_b,ff x_{n+1} = m * x_n + c_b ;   adjoint   A_b,ff lambda_n = gbar_n + m * lambda_{n+1}
+ *   dL/dkappa_{b,e} = -dt sum_n lam~_{n,b}^T K0_e u_{n,b}   (PER_SAMPLE: summed over e in a fixed order)
+ * One warp per sample runs both banded sweeps of its own factor (no tensor cores: there is no shared B operand).
+ * Meshes: dfe_band_ps_supported (else DFE_ERR_UNSUPPORTED).
+ *   dfe_heat_ps_factor_bytes     (10 * n_el + B * npad * 33) * 8 bytes, npad = dfe_band_npad(m): 262 KB per sample at
+ *                                FEMesh.rectangle(32, 32), about 1.07 GB at B = 4096.  Layout, in doubles:
+ *                                  K0[6 * n_el] | element node / free-rank table[4 * n_el]   (per-element gradient tables)
+ *                                  then per sample b: invd[npad] | Lr[npad * 32]   (the layout of dfe_band_ps_factor_bytes)
+ *   dfe_heat_ps_workspace_bytes  ws of dfe_heat_ps_setup: B * nnz_full doubles (A_b on the pattern of K, left there on
+ *                                return) + npad * 33 int32
+ *   dfe_heat_ps_setup   mass / load (n_nodes): the lumped mass and the load vector F of the source (load may be NULL: no
+ *                       source), shared by the batch.  Assembles and factors every A_b (bit-identical to dfe_assemble,
+ *                       dt * K + mass on the diagonal with two roundings, and dfe_band_factor), fills `factors` (16-byte
+ *                       aligned) and c_free (B, npad), zero beyond n_free; status[B] (device int32): 0 ok, 5 = A_b not SPD.
+ *   dfe_heat_ps_fwd     as dfe_heat_fwd, with the factors and c_free (B, npad) of dfe_heat_ps_setup; m_free (npad).
+ *   dfe_heat_ps_adj     as dfe_heat_adj, with the factors of dfe_heat_ps_setup.
+ *   dfe_heat_ps_grad    gacc (B, n_el) += lam~_n^T K0_e u_n for the steps of one segment (u and lam as for dfe_heat_grad),
+ *                       added one step at a time from the last step down: call it for the segments in descending order
+ *                       on a zeroed gacc and the sums are bit-identical however the rollout was split, and independent of B.
+ *   dfe_heat_ps_grad_sum  gkappa = -dt gacc: (B, n_el) for PER_SAMPLE_ELEMENT, (B) summed per sample for PER_SAMPLE.
+ * Offsets into the factors, trajectory and lambda buffers are 64-bit.  The kernels never wait on each other's warps (no
+ * fault word).  All calls are asynchronous on `stream`.
+ */
+size_t dfe_heat_ps_factor_bytes(const dfe_mesh* m, int64_t B);
+size_t dfe_heat_ps_workspace_bytes(const dfe_mesh* m, int64_t B);
+int dfe_heat_ps_setup(const dfe_mesh* m, int64_t B, const double* kappa, int kappa_mode, double dt, const double* mass,
+                      const double* load, void* factors, double* c_free, int32_t* status, void* ws, size_t ws_bytes,
+                      void* stream);
+int dfe_heat_ps_fwd(const dfe_mesh* m, int64_t B, int64_t n_steps, const double* u0, int64_t ldu0, const void* factors,
+                    const double* m_free, const double* c_free, double* X, double* traj, int64_t ld_b, int64_t ld_t,
+                    void* stream);
+int dfe_heat_ps_adj(const dfe_mesh* m, int64_t B, int64_t n0, int64_t n_steps, const double* gbar, int64_t ldg_b,
+                    int64_t ldg_t, int64_t g_every, const void* factors, const double* m_free, double* X, double* lam,
+                    double* lam_sum, void* stream);
+int dfe_heat_ps_grad(const dfe_mesh* m, int64_t B, int64_t n_seg, const void* factors, const double* u, int64_t ld_b,
+                     int64_t ld_t, const double* lam, double* gacc, void* stream);
+int dfe_heat_ps_grad_sum(const dfe_mesh* m, int64_t B, double dt, int kappa_mode, const double* gacc, double* gkappa,
+                         void* stream);
+
 #ifdef __cplusplus
 }
 #endif
