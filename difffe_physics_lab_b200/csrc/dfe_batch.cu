@@ -114,6 +114,18 @@ __device__ __forceinline__ void block_sum2(double& a, double& b, double* sh, int
   b = y;
 }
 
+// block max of non-negative values (a max is exact in any order); every thread returns the same bits
+__device__ __forceinline__ double block_max(double a, double* sh, int lane, int warp) {
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) a = fmax(a, __shfl_xor_sync(0xffffffffu, a, d));
+  if (lane == 0) sh[warp] = a;
+  __syncthreads();
+  double x = sh[lane & (BNW - 1)];
+#pragma unroll
+  for (int d = BNW / 2; d > 0; d >>= 1) x = fmax(x, __shfl_xor_sync(0xffffffffu, x, d));
+  return x;
+}
+
 template <bool BWD, int RPT>
 __global__ void __launch_bounds__(BT, (RPT <= 4 ? 2 : 1)) k_batch(const BArgs A) {
   extern __shared__ __align__(16) unsigned char smem[];
@@ -148,7 +160,7 @@ __global__ void __launch_bounds__(BT, (RPT <= 4 ? 2 : 1)) k_batch(const BArgs A)
     const double* in = A.in + b * A.ldin;
     // ---- right-hand side
     double x[RPT], r[RPT], z[RPT], p[RPT], q[RPT];
-    double bb = 0.0, rz = 0.0;
+    double amax = 0.0;
 #pragma unroll
     for (int j = 0; j < RPT; ++j) {
       x[j] = r[j] = z[j] = p[j] = q[j] = 0.0;
@@ -162,6 +174,25 @@ __global__ void __launch_bounds__(BT, (RPT <= 4 ? 2 : 1)) k_batch(const BArgs A)
           for (int t = M.lift_ptr[row[j]]; t < M.lift_ptr[row[j] + 1]; ++t)
             Fr = __dsub_rn(Fr, __dmul_rn(A.vals_full[M.lift_src[t]], M.lift_g[t]));   // solver.py:169
         }
+        r[j] = Fr;
+        amax = fmax(amax, fabs(Fr));
+      }
+    }
+    // Solve for 2^sc * Fr with max |2^sc Fr| in [1, 2): the squares in ||Fr||^2, tol^2 ||Fr||^2 and p.q then neither
+    // underflow (|Fr| < ~2e-162 would give bb == 0, i.e. "converged" at x = 0; below ~1e-154 tol^2 bb underflows and the
+    // loop stops far above tol) nor overflow.  Scaling by a power of two is exact, so where no intermediate leaves the
+    // normal range the iterates are those of the unscaled solve, scaled.
+    amax = block_max(amax, sred + 2 * BNW, lane, warp);
+    int sc = 0;
+    if (amax > 0.0 && isfinite(amax)) {    // (0: nothing to solve; inf / NaN: reported as a breakdown below)
+      frexp(amax, &sc);
+      sc = 1 - sc;
+    }
+    double bb = 0.0, rz = 0.0;
+#pragma unroll
+    for (int j = 0; j < RPT; ++j) {
+      if (row[j] >= 0) {
+        const double Fr = ldexp(r[j], sc);
         r[j] = Fr;
         z[j] = dinv[j] * Fr;
         p[j] = z[j];
@@ -243,11 +274,11 @@ __global__ void __launch_bounds__(BT, (RPT <= 4 ? 2 : 1)) k_batch(const BArgs A)
       A.status[b] = status;
     }
     if (!BWD) {
-      // ---- u = 0; u[d] = g; u[free] = x   (solver.py:177-181)
+      // ---- u = 0; u[d] = g; u[free] = 2^-sc x   (solver.py:177-181)
       double* u = A.out + b * A.ldout;
 #pragma unroll
       for (int j = 0; j < RPT; ++j)
-        if (row[j] >= 0) u[M.free_nodes[row[j]]] = x[j];
+        if (row[j] >= 0) u[M.free_nodes[row[j]]] = ldexp(x[j], -sc);
       for (int i = tid; i < M.n_dir; i += BT) u[M.dir_idx[i]] = M.dir_val[i];
     } else {
       // ---- lambda on all nodes (0 on Dirichlet nodes), then the closed-form backward of the assembly (SURVEY A8)
@@ -256,7 +287,7 @@ __global__ void __launch_bounds__(BT, (RPT <= 4 ? 2 : 1)) k_batch(const BArgs A)
       __syncthreads();
 #pragma unroll
       for (int j = 0; j < RPT; ++j)
-        if (row[j] >= 0) slam[M.free_nodes[row[j]]] = x[j];
+        if (row[j] >= 0) slam[M.free_nodes[row[j]]] = ldexp(x[j], -sc);
       __syncthreads();
       const double* u = A.u + b * A.ldu;
       double gsum = 0.0, dummy = 0.0;
