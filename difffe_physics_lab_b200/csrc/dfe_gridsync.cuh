@@ -1,7 +1,8 @@
-// Grid-wide fixed-order sum of two doubles for a cooperative (co-resident) launch, fused with the grid barrier the
-// phases of a persistent solver need anyway.  Included inside an anonymous namespace by dfe_pcg.cu and dfe_mg.cu.
+// Grid-wide fixed-order reduction (a sum, or a max) of two doubles for a cooperative (co-resident) launch, fused with the
+// grid barrier the phases of a persistent solver need anyway.  Included inside an anonymous namespace by dfe_pcg.cu and
+// dfe_mg.cu.
 //
-// *Data-as-flag*: every CTA release-stores its two partial sums into its slot of the epoch's buffer (pre-set to an
+// *Data-as-flag*: every CTA release-stores its two partial results into its slot of the epoch's buffer (pre-set to an
 // all-ones sentinel), warp 0 of every CTA polls all G slots with relaxed loads and adds them in a fixed order
 // (lane-strided, then a butterfly), one acquire fence, one CTA barrier.  No atomic, no separate counter, no second
 // read of a partials array: one L2 round trip after the last CTA arrives.  Three buffers rotate; a CTA resets its own
@@ -28,27 +29,36 @@ __device__ __forceinline__ bool grid_aborted(const GridSync& gs) {
   return *reinterpret_cast<volatile int*>(gs.abort_flag) != 0;
 }
 
-// Sums of `v0` and `v1` over the whole grid; every thread of every CTA returns the same bits.  Doubles as the grid
-// barrier between phases (all global writes of every CTA before the call are visible after it).  `sh`: 2 * NW + 2 doubles.
-template <int NW>
-__device__ __forceinline__ void grid_sum2(const GridSync& gs, unsigned int& epoch, double& v0, double& v1, double* sh) {
+// The combine steps: a + b (fixed order, so bit-reproducible) and fmax (exact in any order; drops a NaN).
+struct SumOp {
+  __device__ __forceinline__ static double f(double a, double b) { return a + b; }
+};
+struct MaxOp {   // for non-negative values: 0 is the identity
+  __device__ __forceinline__ static double f(double a, double b) { return fmax(a, b); }
+};
+
+// Op::f-reductions of `v0` and `v1` over the whole grid; every thread of every CTA returns the same bits.  Doubles as the
+// grid barrier between phases (all global writes of every CTA before the call are visible after it).  `sh`: 2 * NW + 2
+// doubles.
+template <int NW, class Op>
+__device__ __forceinline__ void grid_reduce2(const GridSync& gs, unsigned int& epoch, double& v0, double& v1, double* sh) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int G = gridDim.x;
 #pragma unroll
   for (int d = 16; d > 0; d >>= 1) {
-    v0 += __shfl_xor_sync(0xffffffffu, v0, d);
-    v1 += __shfl_xor_sync(0xffffffffu, v1, d);
+    v0 = Op::f(v0, __shfl_xor_sync(0xffffffffu, v0, d));
+    v1 = Op::f(v1, __shfl_xor_sync(0xffffffffu, v1, d));
   }
   if (lane == 0) { sh[2 * warp] = v0; sh[2 * warp + 1] = v1; }
   __syncthreads();
   ++epoch;
   if (warp == 0) {
     double a = 0.0, b = 0.0;
-    for (int w = lane; w < NW; w += 32) { a += sh[2 * w]; b += sh[2 * w + 1]; }
+    for (int w = lane; w < NW; w += 32) { a = Op::f(a, sh[2 * w]); b = Op::f(b, sh[2 * w + 1]); }
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) {
-      a += __shfl_xor_sync(0xffffffffu, a, d);
-      b += __shfl_xor_sync(0xffffffffu, b, d);
+      a = Op::f(a, __shfl_xor_sync(0xffffffffu, a, d));
+      b = Op::f(b, __shfl_xor_sync(0xffffffffu, b, d));
     }
     double* cur = gs.slots + static_cast<size_t>(epoch % 3) * 2 * G;
     if (lane == 0) {
@@ -96,14 +106,14 @@ __device__ __forceinline__ void grid_sum2(const GridSync& gs, unsigned int& epoc
 #pragma unroll
       for (int k = 0; k < NSL; ++k)   // fixed order: slot index ascending within the lane
         if (i0 + 32 * k < G) {
-          sa += __longlong_as_double(static_cast<long long>(ua[k]));
-          sb += __longlong_as_double(static_cast<long long>(ub[k]));
+          sa = Op::f(sa, __longlong_as_double(static_cast<long long>(ua[k])));
+          sb = Op::f(sb, __longlong_as_double(static_cast<long long>(ub[k])));
         }
     }
 #pragma unroll
     for (int d = 16; d > 0; d >>= 1) {
-      sa += __shfl_xor_sync(0xffffffffu, sa, d);
-      sb += __shfl_xor_sync(0xffffffffu, sb, d);
+      sa = Op::f(sa, __shfl_xor_sync(0xffffffffu, sa, d));
+      sb = Op::f(sb, __shfl_xor_sync(0xffffffffu, sb, d));
     }
     // (the butterfly above made every lane's polls complete; one fence, then the CTA barrier, as a grid barrier does)
     __syncwarp();
@@ -116,6 +126,20 @@ __device__ __forceinline__ void grid_sum2(const GridSync& gs, unsigned int& epoc
   __syncthreads();
   v0 = sh[2 * NW];
   v1 = sh[2 * NW + 1];
+}
+
+// Sums of `v0` and `v1` over the whole grid (the reduction every solver phase ends with).
+template <int NW>
+__device__ __forceinline__ void grid_sum2(const GridSync& gs, unsigned int& epoch, double& v0, double& v1, double* sh) {
+  grid_reduce2<NW, SumOp>(gs, epoch, v0, v1, sh);
+}
+
+// Largest of the non-negative `v` over the whole grid; every thread of every CTA returns the same value.
+template <int NW>
+__device__ __forceinline__ double grid_max(const GridSync& gs, unsigned int& epoch, double v, double* sh) {
+  double unused = 0.0;
+  grid_reduce2<NW, MaxOp>(gs, epoch, v, unused, sh);
+  return v;
 }
 
 template <int NW>

@@ -23,7 +23,8 @@
 // Solve kernel: one 768-thread CTA per SM, every level's nodes split into contiguous per-CTA ranges; the phases of
 // the cycle (smooth / residual / restrict / prolong) and of CG (q = A p, vector updates) are separated by the
 // fixed-order grid reduction of dfe_gridsync.cuh, which doubles as the barrier: dot products are bit-reproducible,
-// no float atomics.  Stops at recursive ||r|| <= tol ||rhs||.
+// no float atomics.  Stops at recursive ||r|| <= tol ||rhs||, on the rhs scaled by the power of two that brings its largest
+// entry into [1, 2) (x is scaled back at the end; see k_pcg).
 #include <cmath>
 #include <cstdlib>
 #include <vector>
@@ -261,7 +262,8 @@ struct MgArgs {
   MgVec v[MG_MAXL];
   const double* rhs;
   double *x, *p0, *p1, *q;
-  double* out;          // [0] iterations, [1] relres, [2] status (0 ok, 4 not converged, 5 breakdown, 7 barrier timeout)
+  double* out;          // [0] iterations, [1] relres, [2] status (0 ok, 4 not converged, 5 breakdown, 7 barrier timeout),
+                        // [3] 1 if the breakdown is a non-finite rhs
   double* slots;
   int* abort_flag;
   double tol;
@@ -533,7 +535,7 @@ extern "C" int dfe_mg_pcg(const dfe_mesh* m, const void* hier, const double* rhs
       void* args[] = {&R};
       if (e == cudaSuccess)
         e = cudaLaunchCooperativeKernel(kern, dim3(static_cast<unsigned>(grid)), dim3(MT), args, smem, st);
-      double out[3] = {0, 0, 0};
+      double out[4] = {0, 0, 0, 0};
       if (e == cudaSuccess) e = cudaMemcpyAsync(out, R.out, sizeof out, cudaMemcpyDeviceToHost, st);
       if (e == cudaSuccess) e = cudaStreamSynchronize(st);
       if (e != cudaSuccess) {
@@ -546,6 +548,9 @@ extern "C" int dfe_mg_pcg(const dfe_mesh* m, const void* hier, const double* rhs
           dfe::set_error("dfe_mg_pcg: not converged after %lld iterations (relative residual %.3e, tol %.3e)",
                          static_cast<long long>(out[0]), out[1], tol);
           rc = DFE_ERR_NOT_CONVERGED;
+        } else if (out[2] == 5.0 && out[3] != 0.0) {
+          dfe::set_error("dfe_mg_pcg: breakdown at iteration 0: the right-hand side has a non-finite entry (inf or NaN)");
+          rc = DFE_ERR_BREAKDOWN;
         } else if (out[2] == 5.0) {
           dfe::set_error("dfe_mg_pcg: breakdown at iteration %lld (r^T M r <= 0, p^T K p <= 0 or non-finite)",
                          static_cast<long long>(out[0]));

@@ -197,22 +197,38 @@ __global__ void __launch_bounds__(MT, 1) k_mgpcg(const __grid_constant__ MgArgs 
     __syncthreads();
   }
 
-  // ---- init: x = 0, r = rhs, p buffers = 0
-  double bb = 0.0, zero = 0.0;
+  // ---- init: x = 0, p buffers = 0, amax = max |rhs_k|
+  double amax = 0.0;
   for (int k = lo0 + tid; k < hi0; k += MT) {
-    const double bi = A.rhs[k];
+    amax = fmax(amax, fabs(A.rhs[k]));
     A.x[k] = 0.0;
-    rcg[k] = bi;
     A.p0[k] = 0.0;
     A.p1[k] = 0.0;
+  }
+  amax = grid_max<MW>(gs, epoch, amax, sh);
+  // Solve for 2^sc rhs with max |2^sc rhs_k| in [1, 2), as k_pcg does: no square underflows or overflows, and since the
+  // V-cycle is linear too (smoothing, restriction, prolongation, the coarsest inverse), in-range inputs keep their bits.
+  int sc = 0;
+  if (amax > 0.0 && isfinite(amax)) {
+    frexp(amax, &sc);
+    sc = 1 - sc;
+  }
+  // ---- r = 2^sc rhs
+  double bb = 0.0, zero = 0.0;
+  for (int k = lo0 + tid; k < hi0; k += MT) {
+    const double bi = ldexp(A.rhs[k], sc);
+    rcg[k] = bi;
     bb = fma(bi, bi, bb);
   }
   grid_sum2<MW>(gs, epoch, bb, zero, sh);
   const double bnorm = sqrt(bb);
   double status = 0.0, relres = 0.0;
   long long it = 0;
-  if (!(bb > 0.0)) {
-    if (bb != 0.0) status = 5.0;      // rhs non-finite
+  // a non-finite rhs: amax = inf gives bb = inf (or NaN); fmax drops a NaN, but the sum does not
+  if (!isfinite(bb)) {
+    status = 5.0;
+  } else if (bb == 0.0) {
+    // rhs == 0 -> x = 0
   } else {
     double rz = 0.0, beta = 0.0;
     double* pold = A.p0;
@@ -289,10 +305,13 @@ __global__ void __launch_bounds__(MT, 1) k_mgpcg(const __grid_constant__ MgArgs 
       pnew = t;
     }
   }
+  // ---- x = 2^-sc x on this CTA's range of level 0 (the threads that last wrote it; nothing reads x after this)
+  for (int k = lo0 + tid; k < hi0; k += MT) A.x[k] = ldexp(A.x[k], -sc);
   if (blockIdx.x == 0 && tid == 0) {
     A.out[0] = static_cast<double>(it);
     A.out[1] = relres;
     A.out[2] = status;
+    A.out[3] = isfinite(bnorm) ? 0.0 : 1.0;
   }
 }
 

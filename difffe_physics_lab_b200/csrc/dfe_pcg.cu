@@ -12,7 +12,8 @@
 //   B  x += alpha p ; r -= alpha q ; z = D^{-1} r ; partial r.z and r.r
 // Dot products are reduced in a fixed order (lane-strided sum + xor-shuffle tree over the per-CTA
 // partials), identically on every CTA: results are bit-reproducible and no float atomics are used.
-// Stops when the recursive residual satisfies ||r||_2 <= tol ||rhs||_2.
+// Stops when the recursive residual satisfies ||r||_2 <= tol ||rhs||_2.  The solve runs on 2^sc rhs, the power of two that
+// brings max |rhs_i| into [1, 2), and scales x back at the end: exact, and no square underflows or overflows.
 #include <cstdlib>
 
 #include "dfe_internal.h"
@@ -38,7 +39,8 @@ struct PcgArgs {
   double* p1;
   double* q;
   double* part;   // [3 epochs][gridDim.x][2] exchange slots, pre-set to the sentinel
-  double* out;    // [0]=iterations, [1]=relres, [2]=status (0 ok, 4 not converged, 5 breakdown, 7 barrier timeout)
+  double* out;    // [0]=iterations, [1]=relres, [2]=status (0 ok, 4 not converged, 5 breakdown, 7 barrier timeout),
+                  // [3]=1 if the breakdown is a non-finite rhs
   int* abort_flag; // zeroed before the launch; raised by a grid barrier that waited longer than its bound
   double tol;
   long long maxit;
@@ -59,18 +61,36 @@ __global__ void __launch_bounds__(PT, 1) k_pcg(const PcgArgs A) {
   const int gw = s_lo + (threadIdx.x >> 5);
   constexpr int nwarps = PW;
 
-  // ---- init: x = 0, r = b, z = D^{-1} r, p buffers = 0
+  // ---- init: x = 0, p buffers = 0, amax = max |b_i|
+  double amax = 0.0;
+  for (int s = gw; s < s_hi; s += nwarps) {
+    const int i = 32 * s + lane;
+    if (i < A.n) {
+      amax = fmax(amax, fabs(A.b[i]));
+      A.x[i] = 0.0;
+      A.p0[i] = 0.0;
+      A.p1[i] = 0.0;
+    }
+  }
+  amax = grid_max<PW>(gs, epoch, amax, sh);
+  // Solve for 2^sc b with max |2^sc b_i| in [1, 2): ||b||^2, tol ||b|| and p.q then neither underflow (|b| < ~1e-162 gave
+  // bb == 0, i.e. "converged" at x = 0; below ~1e-154 the loop stopped far above tol) nor overflow (|b| ~ 1e155 overflowed
+  // p.q into a breakdown).  Where no intermediate leaves the normal range the iterates are those of the unscaled solve,
+  // scaled, so relres, the iteration count and (after the scale back below) x keep their bits.
+  int sc = 0;
+  if (amax > 0.0 && isfinite(amax)) {    // (0: nothing to solve; inf: reported as a breakdown below)
+    frexp(amax, &sc);
+    sc = 1 - sc;
+  }
+  // ---- r = 2^sc b, z = D^{-1} r
   double bb = 0.0, rz = 0.0;
   for (int s = gw; s < s_hi; s += nwarps) {
     const int i = 32 * s + lane;
     if (i < A.n) {
-      const double bi = A.b[i];
+      const double bi = ldexp(A.b[i], sc);
       const double zi = A.dinv[i] * bi;
-      A.x[i] = 0.0;
       A.r[i] = bi;
       A.z[i] = zi;
-      A.p0[i] = 0.0;
-      A.p1[i] = 0.0;
       bb = fma(bi, bi, bb);
       rz = fma(bi, zi, rz);
     }
@@ -79,9 +99,11 @@ __global__ void __launch_bounds__(PT, 1) k_pcg(const PcgArgs A) {
   const double bnorm = sqrt(bb);
   double status = 0.0, relres = 0.0;
   long long it = 0;
-  if (!(bb > 0.0)) {
-    // rhs == 0 -> x = 0 (or rhs non-finite -> breakdown)
-    if (bb != 0.0) status = 5.0;
+  // a non-finite rhs: amax = inf gives bb = inf (or NaN); fmax drops a NaN, but the sum does not
+  if (!isfinite(bb)) {
+    status = 5.0;
+  } else if (bb == 0.0) {
+    // rhs == 0 -> x = 0
   } else {
     double beta = 0.0;
     double* pold = A.p0;
@@ -201,10 +223,16 @@ __global__ void __launch_bounds__(PT, 1) k_pcg(const PcgArgs A) {
       pnew = t;
     }
   }
+  // ---- x = 2^-sc x on the rows of this CTA (the threads that last wrote them; nothing reads x after this)
+  for (int s = gw; s < s_hi; s += nwarps) {
+    const int i = 32 * s + lane;
+    if (i < A.n) __stcs(A.x + i, ldexp(__ldcs(A.x + i), -sc));
+  }
   if (blockIdx.x == 0 && threadIdx.x == 0) {
     A.out[0] = static_cast<double>(it);
     A.out[1] = relres;
     A.out[2] = status;
+    A.out[3] = isfinite(bnorm) ? 0.0 : 1.0;
   }
 }
 
@@ -304,7 +332,7 @@ extern "C" int dfe_pcg(const dfe_mesh* m, const double* sell_vals, const double*
       dfe::set_error("dfe_pcg: cooperative launch failed: %s", cudaGetErrorString(e));
       rc = DFE_ERR_CUDA;
     } else {
-      double out[3] = {0, 0, 0};
+      double out[4] = {0, 0, 0, 0};
       e = cudaMemcpyAsync(out, A.out, sizeof out, cudaMemcpyDeviceToHost, st);
       if (e == cudaSuccess) e = cudaStreamSynchronize(st);
       if (e != cudaSuccess) {
@@ -321,6 +349,9 @@ extern "C" int dfe_pcg(const dfe_mesh* m, const double* sell_vals, const double*
           dfe::set_error("dfe_pcg: a grid barrier waited longer than its bound (lost co-resident CTA?) at iteration %lld",
                          static_cast<long long>(out[0]));
           rc = DFE_ERR_CUDA;
+        } else if (out[2] == 5.0 && out[3] != 0.0) {
+          dfe::set_error("dfe_pcg: breakdown at iteration 0: the right-hand side has a non-finite entry (inf or NaN)");
+          rc = DFE_ERR_BREAKDOWN;
         } else if (out[2] == 5.0) {
           dfe::set_error("dfe_pcg: breakdown at iteration %lld (p^T K p <= 0 or non-finite): K_free is not SPD — "
                          "does the mesh have a Dirichlet node?",
