@@ -65,20 +65,22 @@ _EDGES = ((0, 1), (1, 2), (2, 0))
 
 
 def _shape_2d(lam, glam):
-    """P2 shape functions (6,) and gradients (6, 2) at barycentric point lam (3,), glam = grad lambda (3, 2)."""
+    """P2 shape functions (6,) and gradients (..., 6, 2) at barycentric point lam (3,), glam = grad lambda (..., 3, 2)."""
     N = np.empty(6)
-    G = np.empty((6, 2))
+    G = np.empty(glam.shape[:-2] + (6, 2))
     for i in range(3):
         N[i] = lam[i] * (2 * lam[i] - 1)
-        G[i] = (4 * lam[i] - 1) * glam[i]
+        G[..., i, :] = (4 * lam[i] - 1) * glam[..., i, :]
     for k, (i, j) in enumerate(_EDGES):
         N[3 + k] = 4 * lam[i] * lam[j]
-        G[3 + k] = 4 * (lam[i] * glam[j] + lam[j] * glam[i])
+        G[..., 3 + k, :] = 4 * (lam[i] * glam[..., j, :] + lam[j] * glam[..., i, :])
     return N, G
 
 
 def element_matrices(nodes, elements):
-    """(K0_e, M_e) for every element: stiffness at kappa = 1 and consistent mass, shapes (n_el, npe, npe)."""
+    """(K0_e, M_e) for every element: stiffness at kappa = 1 and consistent mass, shapes (n_el, npe, npe).  The
+    quadrature is applied to all elements at once (one pass per quadrature point), so meshes of 1e5 elements take a
+    fraction of a second."""
     nodes = np.asarray(nodes, dtype=np.float64)
     elements = np.asarray(elements, dtype=np.int64)
     ne, npe = elements.shape
@@ -87,27 +89,29 @@ def element_matrices(nodes, elements):
     if nodes.shape[1] == 1:
         assert npe == 3
         gp, gw = 0.5 * (_G3[0] + 1.0), 0.5 * _G3[1]
-        for e in range(ne):
-            h = nodes[elements[e, 1], 0] - nodes[elements[e, 0], 0]
-            for xi, w in zip(gp, gw):
-                N, dN = _shape_1d(xi)
-                K0[e] += w * np.outer(dN, dN) / h
-                M[e] += w * h * np.outer(N, N)
+        h = nodes[elements[:, 1], 0] - nodes[elements[:, 0], 0]
+        for xi, w in zip(gp, gw):
+            N, dN = _shape_1d(xi)
+            K0 += (w * np.outer(dN, dN))[None] / h[:, None, None]
+            M += w * h[:, None, None] * np.outer(N, N)[None]
     else:
         assert npe == 6
-        for e in range(ne):
-            P = nodes[elements[e, :3]]
-            J = np.array([[P[1, 0] - P[0, 0], P[2, 0] - P[0, 0]], [P[1, 1] - P[0, 1], P[2, 1] - P[0, 1]]])
-            det = J[0, 0] * J[1, 1] - J[0, 1] * J[1, 0]
-            area = 0.5 * abs(det)
-            if area < 1e-15:
-                continue
-            Jinv = np.linalg.inv(J)
-            glam = np.array([-(Jinv[0] + Jinv[1]), Jinv[0], Jinv[1]])   # gradients of lambda_0, lambda_1, lambda_2
-            for lam, w in zip(_TRI_PTS, _TRI_W):
-                N, G = _shape_2d(lam, glam)
-                K0[e] += w * area * (G @ G.T)
-                M[e] += w * area * np.outer(N, N)
+        P = nodes[elements[:, :3]]                                       # (ne, 3 vertices, 2)
+        J = np.stack((P[:, 1] - P[:, 0], P[:, 2] - P[:, 0]), axis=2)      # J[e] = [[x1-x0, x2-x0], [y1-y0, y2-y0]]
+        det = J[:, 0, 0] * J[:, 1, 1] - J[:, 0, 1] * J[:, 1, 0]
+        area = 0.5 * np.abs(det)
+        keep = ~(area < 1e-15)                                          # degenerate triangles contribute nothing
+        Jinv = np.linalg.inv(J[keep])                                   # rows: gradients of lambda_1, lambda_2
+        glam = np.stack((-(Jinv[:, 0] + Jinv[:, 1]), Jinv[:, 0], Jinv[:, 1]), axis=1)   # (nk, 3, 2)
+        a = area[keep][:, None, None]
+        Kk = np.zeros((len(glam), 6, 6))
+        Mk = np.zeros((len(glam), 6, 6))
+        for lam, w in zip(_TRI_PTS, _TRI_W):
+            N, G = _shape_2d(lam, glam)
+            Kk += w * a * np.einsum("eik,ejk->eij", G, G)
+            Mk += w * a * np.outer(N, N)[None]
+        K0[keep] = Kk
+        M[keep] = Mk
     return K0, M
 
 
