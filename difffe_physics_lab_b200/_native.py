@@ -46,6 +46,7 @@ SYMBOLS = [
     "dfe_heat_grad_sum",
     "dfe_heat_ps_factor_bytes", "dfe_heat_ps_workspace_bytes", "dfe_heat_ps_setup", "dfe_heat_ps_fwd", "dfe_heat_ps_adj",
     "dfe_heat_ps_grad", "dfe_heat_ps_grad_sum",
+    "dfe_heat_src_workspace_bytes", "dfe_heat_src_load", "dfe_heat_fwd_src", "dfe_heat_ps_fwd_src", "dfe_heat_src_grad",
 ]
 
 
@@ -256,6 +257,16 @@ def lib() -> C.CDLL:
     L.dfe_heat_ps_grad.argtypes = [vp, i64, i64, vp, vp, i64, i64, vp, vp, vp]
     L.dfe_heat_ps_grad_sum.restype = ci
     L.dfe_heat_ps_grad_sum.argtypes = [vp, i64, dbl, ci, vp, vp, vp]
+    L.dfe_heat_src_workspace_bytes.restype = sz
+    L.dfe_heat_src_workspace_bytes.argtypes = [vp]
+    L.dfe_heat_src_load.restype = ci
+    L.dfe_heat_src_load.argtypes = [vp, i64, i64, dbl, vp, i64, i64, vp, i64, vp, vp, sz, vp]
+    L.dfe_heat_fwd_src.restype = ci
+    L.dfe_heat_fwd_src.argtypes = [vp, i64, i64, vp, i64, vp, vp, vp, i64, i64, vp, vp, i64, i64, ci, vp, vp]
+    L.dfe_heat_ps_fwd_src.restype = ci
+    L.dfe_heat_ps_fwd_src.argtypes = [vp, i64, i64, vp, i64, vp, vp, vp, i64, i64, vp, vp, i64, i64, vp]
+    L.dfe_heat_src_grad.restype = ci
+    L.dfe_heat_src_grad.argtypes = [vp, i64, i64, dbl, vp, i64, i64, vp, i64, i64, vp, sz, vp]
     if L.dfe_abi_version() != 1:
         raise RuntimeError("libdfe_b200.so ABI version mismatch")
     _lib = L

@@ -6,6 +6,7 @@
 constexpr double AREA_EPS = 1e-15;  // solver.py:120
 
 #include "dfe_p2.cuh"   // closed-form P2 element matrices (roadmap extension, no upstream arithmetic)
+#include "dfe_exact.cuh"  // p1_load_term
 
 // vertices of P2 triangle e (the first three of its six nodes)
 __device__ __forceinline__ P2Tri p2_tri_of(const MeshDev& M, int e, int (&n)[6]) {
@@ -115,10 +116,7 @@ __device__ __forceinline__ void assemble_row(const MeshDev& M, int p, const doub
         add(M.adj_slot[3 * a + q], __ddiv_rn(num, den));
       }
       // F_p += area/3 * (f_i+f_j+f_k)/3   (:143-145)
-      if (LOAD) {
-        const double fc = __ddiv_rn(__dadd_rn(__dadd_rn(f[n[0]], f[n[1]]), f[n[2]]), 3.0);
-        Fp = __dadd_rn(Fp, __dmul_rn(__ddiv_rn(E.area, 3.0), fc));
-      }
+      if (LOAD) Fp = __dadd_rn(Fp, p1_load_term(__ddiv_rn(E.area, 3.0), f[n[0]], f[n[1]], f[n[2]]));
     }
   }
   if (LOAD) F[p] = Fp;

@@ -529,8 +529,7 @@ __global__ void __launch_bounds__(BT) k_band_rhs_fwd(const MeshDev M, long long 
       for (int e = tid; e < M.n_el; e += BT) {
         const double w = geom[e];
         const int n0 = M.elems[3 * e], n1 = M.elems[3 * e + 1], n2 = M.elems[3 * e + 2];
-        const double fc = __ddiv_rn(__dadd_rn(__dadd_rn(sf[n0], sf[n1]), sf[n2]), 3.0);
-        st[e] = w >= 0.0 ? __dmul_rn(w, fc) : 0.0;   // a skipped element adds nothing
+        st[e] = w >= 0.0 ? p1_load_term(w, sf[n0], sf[n1], sf[n2]) : 0.0;   // a skipped element adds nothing
       }
     __syncthreads();
     for (int r = tid; r < npad; r += BT) {

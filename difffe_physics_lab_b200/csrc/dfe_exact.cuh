@@ -19,3 +19,12 @@ __device__ __forceinline__ double div3(double a) {   // a / 3.0, correctly round
   constexpr double third = 0.333333333333333314829616256247;   // RN(1/3)
   return (a == 0.0 || mid_range(a)) ? div_markstein(a, 3.0, third) : __ddiv_rn(a, 3.0);
 }
+
+// The load term of one P1 triangle at node p (solver.py:143-145): fl(fl(area / 3) * fl(((f_i + f_j) + f_k) / 3)), with
+// area3 = fl(area / 3).  assemble_row, k_band_rhs_fwd and the heat-source kernels (dfe_heat.cu) all form F with this one
+// function; FAST takes the division by 3 through div3 (same bits, no division instruction).
+template <bool FAST = false>
+__device__ __forceinline__ double p1_load_term(double area3, double fi, double fj, double fk) {
+  const double s = __dadd_rn(__dadd_rn(fi, fj), fk);
+  return __dmul_rn(area3, FAST ? div3(s) : __ddiv_rn(s, 3.0));
+}

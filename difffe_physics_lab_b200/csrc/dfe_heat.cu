@@ -38,6 +38,10 @@
 // k_hps_grad    gacc (B, n_el) += lam~^T K0_e u, one step at a time in DESCENDING step order (the order the adjoint
 //               produces them, within and across checkpoint segments): bit-identical with and without checkpointing, and
 //               independent of B.  k_hps_gsum scales by -dt (per element) or sums each sample's elements in a fixed order.
+//
+// Sources per step and per sample: step j of a launch reads its own constant c_{j,b} = fl(c_b + fl(dt F_free(q_{j,b}))).
+// k_hsrc<false> forms those rows (F with the reference's arithmetic, p1_load_term), k_heat_roll<false, W, true> /
+// k_hps_roll<false, true> read them at c + j ldc_t + b ldc_b, and k_hsrc<true> maps lambda rows to dL/dq = W^T (dt lam~).
 #include "dfe_internal.h"
 
 namespace {
@@ -46,8 +50,8 @@ using dfe::MeshDev;
 #include "dfe_1d_common.cuh"   // mbarrier / 1-D TMA bulk copy wrappers
 #include "dfe_band_mma.cuh"     // block-row step of the tensor-core band solve and its fragment layout
 #include "dfe_band_ps_solve.cuh"  // bps_sweeps: both banded sweeps of one sample's factor by one warp
+#include "dfe_assemble_row.cuh"   // AREA_EPS, elem2d; p1_load_term and div3 (dfe_exact.cuh)
 
-constexpr double AREA_EPS = 1e-15;          // solver.py:120
 constexpr long long WAIT_POLLS = 1LL << 24; // try_wait polls before a fragment stage counts as lost (raises the fault word)
 constexpr int GT = 256;                     // threads of the gradient kernel
 constexpr int GNST = 3;                     // cp.async ring stages of the gradient kernel
@@ -75,6 +79,7 @@ struct RollArgs {
   double* lam;                      // adjoint: (nt, B, npad); slot j holds lambda_{n0 + 1 + j}
   double* lsum;                     // adjoint: (B, npad) running sum of lambda_n
   int* fault;                       // set to 1 when a fragment stage was lost
+  long long ldc_t, ldc_b;           // forward with SRC: step j of sample b reads its constant at cf + j * ldc_t + b * ldc_b
 };
 
 __device__ __forceinline__ bool mbar_wait_bounded(uint64_t* bar, uint32_t parity) {
@@ -92,8 +97,11 @@ __device__ __forceinline__ bool mbar_wait_bounded(uint64_t* bar, uint32_t parity
   return false;
 }
 
-template <bool ADJ, int W>
-__global__ void __launch_bounds__(32 * W, 16 / W) k_heat_roll(const RollArgs a) {
+// SRC (forward only): every step and sample reads its own constant c (a source that changes in time and / or per sample).
+// The per-sample read spills 8 bytes at 128 registers with W = 2; roll_warps picks W = 2 only when the grid of W = 4
+// would not cover the SMs (at most two CTAs of 64 threads per SM), so that instance is allowed 4 CTAs' worth of registers.
+template <bool ADJ, int W, bool SRC = false>
+__global__ void __launch_bounds__(32 * W, (SRC && W == 2) ? 4 : 16 / W) k_heat_roll(const RollArgs a) {
   __shared__ __align__(16) double stg[2][FRAGD];
   __shared__ uint64_t bar[2];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -133,13 +141,21 @@ __global__ void __launch_bounds__(32 * W, 16 / W) k_heat_roll(const RollArgs a) 
       }
     }
   }
-  // carry -> right-hand side in place: fma(m, x_n, c) (forward) / fma(m, lambda_{n+1}, gbar_n[free]) (adjoint)
-  auto form_rhs = [&](int kb, Blk& R) {
+  // carry -> right-hand side in place: fma(m, x_n, c) (forward) / fma(m, lambda_{n+1}, gbar_n[free]) (adjoint); step it
+  // of this launch (read by SRC only)
+  auto form_rhs = [&](int kb, Blk& R, int it) {
 #pragma unroll
     for (int nt = 0; nt < 4; ++nt) {
       const int c0 = 32 * kb + 8 * nt + 2 * q;
       const double2 mm = *reinterpret_cast<const double2*>(a.mf + c0);
-      if (!ADJ) {
+      if (SRC) {   // each of the lane's two samples reads its own row, as ld_block reads the carry
+#pragma unroll
+        for (int mt = 0; mt < 2; ++mt) {
+          const double2 cc = *reinterpret_cast<const double2*>(a.cf + it * a.ldc_t + sid[mt] * a.ldc_b + c0);
+          R[mt][nt][0] = fma(mm.x, R[mt][nt][0], cc.x);
+          R[mt][nt][1] = fma(mm.y, R[mt][nt][1], cc.y);
+        }
+      } else if (!ADJ) {
         const double2 cc = *reinterpret_cast<const double2*>(a.cf + c0);
 #pragma unroll
         for (int mt = 0; mt < 2; ++mt) {
@@ -167,7 +183,7 @@ __global__ void __launch_bounds__(32 * W, 16 / W) k_heat_roll(const RollArgs a) 
   Blk R, P = {}, acc;
   set_gbar(0);
   ld_block(row, 0, R);
-  form_rhs(0, R);
+  form_rhs(0, R, 0);
   bool lost = false;
   long long G = 0;   // stage counter over the whole rollout: fragment slot G & 1, barrier parity (G >> 1) & 1
   for (int it = 0; it < a.nt; ++it) {
@@ -188,7 +204,7 @@ __global__ void __launch_bounds__(32 * W, 16 / W) k_heat_roll(const RollArgs a) 
       if (step + 1 < nsub && knext != k) {
         if (step + 1 < nb) {
           ld_block(row, knext, R);
-          form_rhs(knext, R);
+          form_rhs(knext, R, it);
         } else {
           ld_block(row, knext, R);
         }
@@ -236,7 +252,7 @@ __global__ void __launch_bounds__(32 * W, 16 / W) k_heat_roll(const RollArgs a) 
     if (it + 1 < a.nt) {   // block 0 of the carry is in acc: the first right-hand side block of the next step, from registers
       set_gbar(it + 1);
       blk_copy(R, acc);
-      form_rhs(0, R);
+      form_rhs(0, R, it + 1);
     }
   }
   if (lost) atomicExch(a.fault, 1);
@@ -401,7 +417,7 @@ int heat_enter(const dfe_mesh* m, const char* who, int* prev) {
 }
 bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
-template <bool ADJ>
+template <bool ADJ, bool SRC = false>
 int roll_launch(const dfe_mesh* m, int warps, RollArgs a, const void* factor, cudaStream_t st, const char* who) {
   if (warps == 0) warps = roll_warps(m, a.B);
   if (warps != 2 && warps != 4 && warps != 8) {
@@ -417,9 +433,9 @@ int roll_launch(const dfe_mesh* m, int warps, RollArgs a, const void* factor, cu
   dfe::band_frags(m, factor, &a.Ff, &a.Bf);
   const unsigned grid = nblk(a.B, MMA_S * warps);
   switch (warps) {
-    case 8: k_heat_roll<ADJ, 8><<<grid, 256, 0, st>>>(a); break;
-    case 4: k_heat_roll<ADJ, 4><<<grid, 128, 0, st>>>(a); break;
-    default: k_heat_roll<ADJ, 2><<<grid, 64, 0, st>>>(a); break;
+    case 8: k_heat_roll<ADJ, 8, SRC><<<grid, 256, 0, st>>>(a); break;
+    case 4: k_heat_roll<ADJ, 4, SRC><<<grid, 128, 0, st>>>(a); break;
+    default: k_heat_roll<ADJ, 2, SRC><<<grid, 64, 0, st>>>(a); break;
   }
   const cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) {
@@ -482,9 +498,11 @@ struct PsRollArgs {
   int gev, n0;                      // adjoint: steps n0 + nt down to n0 + 1
   double* lam;                      // adjoint: (nt, B, npad); slot j holds lambda_{n0 + 1 + j}
   double* lsum;                     // adjoint: (B, npad) running sum of lambda_n
+  long long ldc_t, ldc_b;           // forward with SRC: step j of sample b reads its constant at cf + j * ldc_t + b * ldc_b
 };
 
-template <bool ADJ>
+// SRC (forward only): c_b read at cf + it * ldc_t + b * ldc_b in step it instead of cf + b * npad in every step
+template <bool ADJ, bool SRC = false>
 __global__ void __launch_bounds__(32 * PSW) k_hps_roll(const PsRollArgs a) {
   const int lane = threadIdx.x & 31;
   const long long b = blockIdx.x * static_cast<long long>(PSW) + (threadIdx.x >> 5);
@@ -495,9 +513,10 @@ __global__ void __launch_bounds__(32 * PSW) k_hps_roll(const PsRollArgs a) {
   double* x = a.X + b * npad;
   if (!ADJ && a.u0 != nullptr)   // x_0 = u0[free]: each lane the rows it owns in the sweeps
     for (int i = lane; i < npad; i += 32) x[i] = i < n ? a.u0[b * a.ldu0 + a.fnode[i]] : 0.0;
+  const double* cs = a.cf + b * a.ldc_b;   // SRC: this step's c_b, advanced by ldc_t per step
   for (int it = 0; it < a.nt; ++it) {
     if (!ADJ) {
-      const double* cb = a.cf + b * npad;
+      const double* cb = SRC ? cs : a.cf + b * npad;
       double* urow = a.traj + b * a.ld_b + it * a.ld_t;
       bps_sweeps(
           invd, Lr, x, nb, lane, [&](int i) { return fma(a.mf[i], x[i], cb[i]); },
@@ -506,6 +525,7 @@ __global__ void __launch_bounds__(32 * PSW) k_hps_roll(const PsRollArgs a) {
             if (i < n) urow[a.fnode[i]] = xv;
           });
       for (int d = lane; d < a.n_dir; d += 32) urow[a.dir_idx[d]] = a.dir_val[d];
+      if (SRC) cs += a.ldc_t;
     } else {
       const int step = a.n0 + a.nt - it;
       const double* gs = (a.gbar != nullptr && step % a.gev == 0)
@@ -613,7 +633,7 @@ int launch_status(const char* who) {
 
 inline unsigned ygrid(long long B) { return static_cast<unsigned>(B < 65535 ? B : 65535); }
 
-template <bool ADJ>
+template <bool ADJ, bool SRC = false>
 int hps_roll_launch(const dfe_mesh* m, PsRollArgs a, const void* factors, cudaStream_t st, const char* who) {
   a.npad = static_cast<int>(dfe_band_npad(m));
   a.nfree = m->dev.n_free;
@@ -622,8 +642,149 @@ int hps_roll_launch(const dfe_mesh* m, PsRollArgs a, const void* factors, cudaSt
   a.dir_idx = m->dev.dir_idx;
   a.dir_val = m->dev.dir_val;
   a.fac = static_cast<const double*>(factors) + 10 * static_cast<size_t>(m->dev.n_el);
-  k_hps_roll<ADJ><<<nblk(a.B, PSW), 32 * PSW, 0, st>>>(a);
+  k_hps_roll<ADJ, SRC><<<nblk(a.B, PSW), 32 * PSW, 0, st>>>(a);
   return launch_status(who);
+}
+
+
+// ---------------------------------------------------------------------------------------------- sources in time and per sample
+constexpr int SRT = 256;    // threads of the source kernels
+constexpr int SRNST = 4;    // cp.async ring stages of the source kernels
+
+struct SrcArgs {
+  int nn, npad, nfree, n_el, rowlen;   // rowlen: doubles of one ring stage
+  long long rows, nb;                  // rows = S * nb; row i is (step j = i / nb, sample b = i % nb)
+  double dt;
+  const double* in;                    // fwd: q row (node layout); grad: lambda row (free layout) at in + j * ldi_t + b * ldi_b
+  long long ldi_t, ldi_b;
+  const double* base;                  // fwd: c_base + b * ldbase (npad)
+  long long ldbase;
+  double* out;                         // fwd: c (S, nb, npad); grad: the node-layout row at out + j * ldo_t + b * ldo_b
+  long long ldo_t, ldo_b;
+  const int4* eidx;                    // (n_el, 2): node ids, free ranks (npad for a Dirichlet node: the zero slot)
+  const double* w;                     // (2, n_el): area / 3 (-1: degenerate element), area / 9 (0: degenerate)
+};
+
+// per element: node ids, free ranks and the two load weights, with the reference's area (elem2d)
+__global__ void k_hsrc_tables(const MeshDev M, int npad, int4* __restrict__ eidx, double* __restrict__ w) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= M.n_el) return;
+  int n[3];
+  const Elem2D E = elem2d(M, e, n);
+  const bool skip = E.area < AREA_EPS;
+  int rk[3];
+  for (int i = 0; i < 3; ++i) rk[i] = M.free_rank[n[i]] >= 0 ? M.free_rank[n[i]] : npad;
+  eidx[2 * e] = make_int4(n[0], n[1], n[2], 0);
+  eidx[2 * e + 1] = make_int4(rk[0], rk[1], rk[2], 0);
+  w[e] = skip ? -1.0 : __ddiv_rn(E.area, 3.0);
+  w[M.n_el + e] = skip ? 0.0 : E.area / 9.0;
+}
+
+// Many rows per CTA: the rows stream through a cp.async ring; per row the element terms go to shared memory (one per
+// element), then every output row adds the terms of its node's adjacent elements in ascending element order.
+//   GRAD = false   c[j, b, r] = fl(c_base_b[r] + fl(dt * F_free(q_{j,b})[r]))   F: the reference's load (p1_load_term)
+//   GRAD = true    out_{j,b}[p] = sum_{e∋p} area_e / 9 * ((l_i + l_j) + l_k),   l = dt * lambda~_{j,b}   (W^T, dfe_grad's gf)
+template <bool GRAD>
+__global__ void __launch_bounds__(SRT) k_hsrc(const MeshDev M, const SrcArgs a) {
+  extern __shared__ __align__(16) double ssm[];
+  double* st = ssm;                                   // [n_el] element terms
+  double* ring = ssm + ((a.n_el + 1) & ~1);           // [SRNST][rowlen]
+  const int tid = threadIdx.x;
+  const long long cnt = a.rows > blockIdx.x ? (a.rows - 1 - blockIdx.x) / gridDim.x + 1 : 0;
+  const int nin = GRAD ? a.npad : a.nn;
+  if (GRAD && tid < SRNST) ring[tid * a.rowlen + a.npad] = 0.0;   // lambda~ of a Dirichlet node
+  auto issue = [&](long long i) {
+    if (i < cnt) {
+      const long long row = blockIdx.x + i * gridDim.x, j = row / a.nb, b = row % a.nb;
+      const double* src = a.in + j * a.ldi_t + b * a.ldi_b;
+      double* dst = ring + (i % SRNST) * a.rowlen;
+      for (int t = tid; t < nin; t += SRT) cp_async8(dst + t, src + t);
+    }
+    cp_commit();   // an empty group past the end keeps the wait count uniform
+  };
+#pragma unroll
+  for (int i = 0; i < SRNST - 1; ++i) issue(i);
+  for (long long i = 0; i < cnt; ++i) {
+    cp_wait<SRNST - 2>();
+    __syncthreads();   // row i has landed for every thread; every thread is done with st and with the slot refilled next
+    issue(i + SRNST - 1);
+    const double* x = ring + (i % SRNST) * a.rowlen;
+    for (int e = tid; e < a.n_el; e += SRT) {
+      if (!GRAD) {
+        const int4 n = a.eidx[2 * e];
+        const double w3 = a.w[e];
+        st[e] = w3 >= 0.0 ? p1_load_term<true>(w3, x[n.x], x[n.y], x[n.z]) : 0.0;   // a skipped element adds nothing
+      } else {
+        const int4 r = a.eidx[2 * e + 1];
+        st[e] = a.w[a.n_el + e] * ((a.dt * x[r.x] + a.dt * x[r.y]) + a.dt * x[r.z]);
+      }
+    }
+    __syncthreads();
+    const long long row = blockIdx.x + i * gridDim.x, j = row / a.nb, b = row % a.nb;
+    if (!GRAD) {
+      double* o = a.out + row * a.npad;
+      const double* cb = a.base + b * a.ldbase;
+      for (int r = tid; r < a.npad; r += SRT) {
+        double v = 0.0;
+        if (r < a.nfree) {
+          const int node = M.free_nodes[r];
+          for (int k = M.adj_ptr[node]; k < M.adj_ptr[node + 1]; ++k) v = __dadd_rn(v, st[M.adj_elem[k]]);
+          v = __dadd_rn(cb[r], __dmul_rn(a.dt, v));
+        }
+        o[r] = v;
+      }
+    } else {
+      double* o = a.out + j * a.ldo_t + b * a.ldo_b;
+      for (int p = tid; p < a.nn; p += SRT) {
+        double v = 0.0;
+        for (int k = M.adj_ptr[p]; k < M.adj_ptr[p + 1]; ++k) v += st[M.adj_elem[k]];
+        o[p] = v;
+      }
+    }
+  }
+}
+
+size_t src_smem(const dfe_mesh* m, bool grad) {
+  const size_t rowlen = grad ? static_cast<size_t>(dfe_band_npad(m)) + 2 : (static_cast<size_t>(m->dev.n_nodes) + 1) & ~1ULL;
+  return (((static_cast<size_t>(m->dev.n_el) + 1) & ~1ULL) + SRNST * rowlen) * sizeof(double);
+}
+
+// validation and launch of k_hsrc<GRAD>: the tables are rebuilt into ws on every call (one small launch)
+int src_launch(const dfe_mesh* m, bool grad, SrcArgs a, void* ws, size_t ws_bytes, cudaStream_t st, const char* who) {
+  const size_t sm = src_smem(m, grad);
+  if (sm > GSMEM_MAX) {
+    dfe::set_error("%s: mesh too large for the source kernels: %zu bytes of shared memory > %zu", who, sm, GSMEM_MAX);
+    return DFE_ERR_UNSUPPORTED;
+  }
+  const size_t ne = static_cast<size_t>(m->dev.n_el);
+  if (ws_bytes < ne * (2 * sizeof(int4) + 2 * sizeof(double))) {
+    dfe::set_error("%s: workspace %zu bytes < required %zu", who, ws_bytes, ne * (2 * sizeof(int4) + 2 * sizeof(double)));
+    return DFE_ERR_WORKSPACE;
+  }
+  a.nn = m->dev.n_nodes;
+  a.npad = static_cast<int>(dfe_band_npad(m));
+  a.nfree = m->dev.n_free;
+  a.n_el = m->dev.n_el;
+  a.rowlen = static_cast<int>(grad ? a.npad + 2 : (a.nn + 1) & ~1);
+  int4* eidx = static_cast<int4*>(ws);
+  double* w = reinterpret_cast<double*>(eidx + 2 * ne);
+  a.eidx = eidx;
+  a.w = w;
+  k_hsrc_tables<<<nblk(a.n_el, 128), 128, 0, st>>>(m->dev, a.npad, eidx, w);
+  auto kern = grad ? k_hsrc<true> : k_hsrc<false>;
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(sm));
+  int per_sm = 0;
+  if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, SRT, sm);
+  if (e == cudaSuccess) {
+    const long long cap = static_cast<long long>(m->sm_count) * (per_sm > 0 ? per_sm : 1);
+    kern<<<static_cast<unsigned>(a.rows < cap ? a.rows : cap), SRT, sm, st>>>(m->dev, a);
+    e = cudaGetLastError();
+  }
+  if (e != cudaSuccess) {
+    dfe::set_error("%s: %s", who, cudaGetErrorString(e));
+    return DFE_ERR_CUDA;
+  }
+  return DFE_OK;
 }
 
 }  // namespace
@@ -922,6 +1083,127 @@ extern "C" int dfe_heat_ps_grad_sum(const dfe_mesh* m, int64_t B, double dt, int
     if (kappa_mode == DFE_KAPPA_PER_SAMPLE) k_hps_gsum<true><<<static_cast<unsigned>(B), 256, 0, st>>>(ne, B, -dt, gacc, gkappa);
     else k_hps_gsum<false><<<nblk(B * ne, 256), 256, 0, st>>>(ne, B, -dt, gacc, gkappa);
     rc = launch_status("dfe_heat_ps_grad_sum");
+  }
+  if (prev != m->info.device) cudaSetDevice(prev);
+  return rc;
+}
+
+// ---------------------------------------------------------------------------------------------- sources in time and per sample
+extern "C" size_t dfe_heat_src_workspace_bytes(const dfe_mesh* m) {
+  if (!dfe_band_ps_supported(m)) return 0;
+  return static_cast<size_t>(m->dev.n_el) * (2 * sizeof(int4) + 2 * sizeof(double));
+}
+
+extern "C" int dfe_heat_src_load(const dfe_mesh* m, int64_t n_steps, int64_t nb, double dt, const double* q, int64_t ldq_t,
+                                 int64_t ldq_b, const double* c_base, int64_t ldbase, double* c, void* ws, size_t ws_bytes,
+                                 void* stream) {
+  int prev;
+  int rc = hps_enter(m, "dfe_heat_src_load", &prev);
+  if (rc) return rc;
+  if (!q || !c_base || !c || !ws || n_steps < 1 || nb < 1 || ldq_t < 0 || ldq_b < 0 || ldbase < 0) {
+    dfe::set_error("dfe_heat_src_load: null / invalid argument");
+    rc = DFE_ERR_INVALID;
+  } else {
+    SrcArgs a{};
+    a.rows = n_steps * nb;
+    a.nb = nb;
+    a.dt = dt;
+    a.in = q;
+    a.ldi_t = ldq_t;
+    a.ldi_b = ldq_b;
+    a.base = c_base;
+    a.ldbase = ldbase;
+    a.out = c;
+    rc = src_launch(m, false, a, ws, ws_bytes, static_cast<cudaStream_t>(stream), "dfe_heat_src_load");
+  }
+  if (prev != m->info.device) cudaSetDevice(prev);
+  return rc;
+}
+
+extern "C" int dfe_heat_src_grad(const dfe_mesh* m, int64_t n_steps, int64_t nb, double dt, const double* lam,
+                                 int64_t ldl_t, int64_t ldl_b, double* g, int64_t ldg_t, int64_t ldg_b, void* ws,
+                                 size_t ws_bytes, void* stream) {
+  int prev;
+  int rc = hps_enter(m, "dfe_heat_src_grad", &prev);
+  if (rc) return rc;
+  if (!lam || !g || !ws || n_steps < 1 || nb < 1 || ldl_t < 0 || ldl_b < 0 || ldg_t < 0 || ldg_b < 0) {
+    dfe::set_error("dfe_heat_src_grad: null / invalid argument");
+    rc = DFE_ERR_INVALID;
+  } else {
+    SrcArgs a{};
+    a.rows = n_steps * nb;
+    a.nb = nb;
+    a.dt = dt;
+    a.in = lam;
+    a.ldi_t = ldl_t;
+    a.ldi_b = ldl_b;
+    a.out = g;
+    a.ldo_t = ldg_t;
+    a.ldo_b = ldg_b;
+    rc = src_launch(m, true, a, ws, ws_bytes, static_cast<cudaStream_t>(stream), "dfe_heat_src_grad");
+  }
+  if (prev != m->info.device) cudaSetDevice(prev);
+  return rc;
+}
+
+extern "C" int dfe_heat_fwd_src(const dfe_mesh* m, int64_t B, int64_t n_steps, const double* u0, int64_t ldu0,
+                                const void* factor, const double* m_free, const double* c, int64_t ldc_t, int64_t ldc_b,
+                                double* X, double* traj, int64_t ld_b, int64_t ld_t, int warps, int32_t* fault,
+                                void* stream) {
+  int prev;
+  int rc = heat_enter(m, "dfe_heat_fwd_src", &prev);
+  if (rc) return rc;
+  if (!factor || !m_free || !c || !X || !traj || !fault || B < 1 || n_steps < 1 || n_steps > (1LL << 30) ||
+      ldc_t < 0 || ldc_b < 0 || (ldc_t | ldc_b) & 1 || !al16(m_free) || !al16(c) || !al16(X)) {
+    dfe::set_error("dfe_heat_fwd_src: null / invalid argument (m_free, c and X must be 16-byte aligned, ldc_t and ldc_b "
+                   "even and >= 0)");
+    rc = DFE_ERR_INVALID;
+  } else {
+    RollArgs a{};
+    a.B = B;
+    a.nt = static_cast<int>(n_steps);
+    a.mf = m_free;
+    a.cf = c;
+    a.ldc_t = ldc_t;
+    a.ldc_b = ldc_b;
+    a.X = X;
+    a.u0 = u0;
+    a.ldu0 = ldu0;
+    a.traj = traj;
+    a.ld_b = ld_b;
+    a.ld_t = ld_t;
+    a.fault = fault;
+    rc = roll_launch<false, true>(m, warps, a, factor, static_cast<cudaStream_t>(stream), "dfe_heat_fwd_src");
+  }
+  if (prev != m->info.device) cudaSetDevice(prev);
+  return rc;
+}
+
+extern "C" int dfe_heat_ps_fwd_src(const dfe_mesh* m, int64_t B, int64_t n_steps, const double* u0, int64_t ldu0,
+                                   const void* factors, const double* m_free, const double* c, int64_t ldc_t,
+                                   int64_t ldc_b, double* X, double* traj, int64_t ld_b, int64_t ld_t, void* stream) {
+  int prev;
+  int rc = hps_enter(m, "dfe_heat_ps_fwd_src", &prev);
+  if (rc) return rc;
+  if (!factors || !m_free || !c || !X || !traj || B < 1 || n_steps < 1 || n_steps > (1LL << 30) || ldc_t < 0 ||
+      ldc_b < 0) {
+    dfe::set_error("dfe_heat_ps_fwd_src: null / invalid argument");
+    rc = DFE_ERR_INVALID;
+  } else {
+    PsRollArgs a{};
+    a.B = B;
+    a.nt = static_cast<int>(n_steps);
+    a.mf = m_free;
+    a.cf = c;
+    a.ldc_t = ldc_t;
+    a.ldc_b = ldc_b;
+    a.X = X;
+    a.u0 = u0;
+    a.ldu0 = ldu0;
+    a.traj = traj;
+    a.ld_b = ld_b;
+    a.ld_t = ld_t;
+    rc = hps_roll_launch<false, true>(m, a, factors, static_cast<cudaStream_t>(stream), "dfe_heat_ps_fwd_src");
   }
   if (prev != m->info.device) cudaSetDevice(prev);
   return rc;

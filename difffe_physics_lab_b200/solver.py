@@ -46,7 +46,7 @@ class KernelTimer:
                         "band_fwd": 3, "band_bwd": 3, "band_ps_fwd": 7, "band_ps_bwd": 2, "assemble": 1, "eliminate": 2, "pcg": 1, "scatter": 1,
                         "gather": 1, "grad": 3, "mg_setup": 20, "mg_pcg": 1, "heat_fwd": 1, "heat_adj": 1,
                         "heat_grad": 2, "heat_ps_setup": 6, "heat_ps_fwd": 1, "heat_ps_adj": 1, "heat_ps_grad": 1,
-                        "heat_ps_grad_sum": 1}
+                        "heat_ps_grad_sum": 1, "heat_src_load": 2, "heat_src_grad": 2}
 
     def __init__(self):
         self.events = []

@@ -13,7 +13,9 @@ states per step (block TRSM on the FP64 tensor cores).  Meshes: half bandwidth o
 ``DifferentiableHeatSolver`` runs the same scheme as a differentiable rollout: the whole time loop is one kernel launch
 (``dfe_heat_fwd``), and the backward is the discrete adjoint in time (``dfe_heat_adj``, ``dfe_heat_grad``) with optional
 checkpointing.  Gradients flow to ``u0``, ``kappa`` and ``f``.  With one conductivity per sample (kappa ``(B, 1)`` or
-``(B, n_el)``) every sample has its own factor and the rollout runs one warp per sample (``dfe_heat_ps_*``).
+``(B, n_el)``) every sample has its own factor and the rollout runs one warp per sample (``dfe_heat_ps_*``).  A source per
+sample (``f (B, n)``) or per step (``source``) enters through per-step constants formed by ``dfe_heat_src_load`` and read by
+the ``*_fwd_src`` rollouts; its gradient is ``dfe_heat_src_grad`` on the adjoint's lambda rows.
 """
 from __future__ import annotations
 
@@ -145,11 +147,37 @@ def _check_status(status: torch.Tensor, fault: torch.Tensor, who: str) -> None:
         raise _native.DfeError(_native.ERR_CUDA, f"{who}: a bounded wait inside a rollout kernel expired; outputs invalid")
 
 
+def _src_load(rt, n_steps, nb, q, ldq_t, ldq_b, base, ldbase, out=None):
+    """c (n_steps, nb, npad): row (j, b) = fl(base_b + fl(dt F_free(q_{j,b}))), q_{j,b} at q + j ldq_t + b ldq_b"""
+    if out is None:
+        out = torch.empty((n_steps, nb, rt.npad), dtype=torch.float64, device=rt.dev)
+    st = torch.cuda.current_stream(rt.dev).cuda_stream
+    with _timed("heat_src_load", rt.dev):
+        _native.check(_native.lib().dfe_heat_src_load(rt.h, n_steps, nb, rt.dt, q.data_ptr(), ldq_t, ldq_b, base.data_ptr(),
+                                                       ldbase, out.data_ptr(), rt.sws.data_ptr(), rt.sws.numel(), st))
+    return out
+
+
+def _src_grad(rt, n_steps, nb, lam, ldl_t, ldl_b, g, ldg_t, ldg_b):
+    """g row (j, b) at g + j ldg_t + b ldg_b = W^T (dt lam~_{j,b}), lam_{j,b} (free layout) at lam + j ldl_t + b ldl_b"""
+    st = torch.cuda.current_stream(rt.dev).cuda_stream
+    with _timed("heat_src_grad", rt.dev):
+        _native.check(_native.lib().dfe_heat_src_grad(rt.h, n_steps, nb, rt.dt, lam.data_ptr(), ldl_t, ldl_b, g.data_ptr(),
+                                                      ldg_t, ldg_b, rt.sws.data_ptr(), rt.sws.numel(), st))
+
+
+def _src_ws(h, dev):
+    return torch.empty(max(int(_native.lib().dfe_heat_src_workspace_bytes(h)), 16), dtype=torch.uint8, device=dev)
+
+
 class _SharedRoute:
-    """kappa shared by the batch: one factor of A = M_L + dt K(kappa), the tensor-core rollout kernels (dfe_heat_*)."""
+    """kappa shared by the batch: one factor of A = M_L + dt K(kappa), the tensor-core rollout kernels (dfe_heat_*).
+    With ``f (B, n)`` each sample's constant c_b (B, npad) is formed once from the lifting-only constant and read by
+    ``dfe_heat_fwd_src`` with a time stride of 0."""
 
     def __init__(self, mesh, kappa, dt, f, dev, B, warps):
-        self.op = op = _HeatOperator(mesh, kappa, dt, f, dev)
+        per_f = f is not None and f.dim() == 2
+        self.op = op = _HeatOperator(mesh, kappa, dt, None if per_f else f, dev)
         self.h, self.npad, self.free, self.mass_free = op.nm.handle, op.npad, op.free, op.mass_free
         self.dt, self.warps, self.dev, self.B = dt, warps, dev, B
         nf = op.free.numel()
@@ -157,17 +185,32 @@ class _SharedRoute:
         self.cf = torch.zeros(self.npad, dtype=torch.float64, device=dev)
         self.mf[:nf], self.cf[:nf] = op.mass_free, op.rhs_const
         self.fault = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.cB = None
+        if per_f:                                           # c_b = fl(fl(dt F_free(f_b)) - lift)
+            self.sws = _src_ws(self.h, dev)
+            self.cB = _src_load(self, 1, B, f, 0, f.stride(0), self.cf, 0)[0]
+        # the constant a per-step source adds to: per sample (B, npad) or shared (npad,), with its row stride
+        self.base, self.ldbase = (self.cf, 0) if self.cB is None else (self.cB, self.npad)
 
     def check(self, who):
         _check_status(self.op.status, self.fault, who)
 
-    def fwd(self, src, X, traj, steps):
+    def fwd(self, src, X, traj, steps, c=None):
+        """c: None, or (tensor, ldc_t, ldc_b): step j of sample b reads its constant at c + j ldc_t + b ldc_b"""
         st = torch.cuda.current_stream(self.dev).cuda_stream
+        if c is None and self.cB is not None:
+            c = (self.cB, 0, self.npad)
         with _timed("heat_fwd", self.dev):
-            _native.check(_native.lib().dfe_heat_fwd(
-                self.h, self.B, steps, None if src is None else src.data_ptr(), traj.shape[-1], self.op.factor.data_ptr(),
-                self.mf.data_ptr(), self.cf.data_ptr(), X.data_ptr(), traj.data_ptr(), traj.stride(0), traj.stride(1),
-                self.warps, self.fault.data_ptr(), st))
+            if c is None:
+                _native.check(_native.lib().dfe_heat_fwd(
+                    self.h, self.B, steps, None if src is None else src.data_ptr(), traj.shape[-1],
+                    self.op.factor.data_ptr(), self.mf.data_ptr(), self.cf.data_ptr(), X.data_ptr(), traj.data_ptr(),
+                    traj.stride(0), traj.stride(1), self.warps, self.fault.data_ptr(), st))
+            else:
+                _native.check(_native.lib().dfe_heat_fwd_src(
+                    self.h, self.B, steps, None if src is None else src.data_ptr(), traj.shape[-1],
+                    self.op.factor.data_ptr(), self.mf.data_ptr(), c[0].data_ptr(), c[1], c[2], X.data_ptr(),
+                    traj.data_ptr(), traj.stride(0), traj.stride(1), self.warps, self.fault.data_ptr(), st))
 
     def begin_backward(self, N):
         self.N = N
@@ -220,7 +263,8 @@ class _PerSampleRoute:
                                      torch.ones(I.n_nodes, dtype=torch.float64, device=dev).data_ptr(), vals.data_ptr(),
                                      mass.data_ptr(), st))
         load = None
-        if f is not None:
+        per_f = f is not None and f.dim() == 2
+        if f is not None and not per_f:
             load = torch.empty(I.n_nodes, dtype=torch.float64, device=dev)
             fs = f.to(device=dev, dtype=torch.float64).contiguous()
             _native.check(L.dfe_assemble(nm.handle, one.data_ptr(), _native.KAPPA_SCALAR, fs.data_ptr(), vals.data_ptr(),
@@ -237,6 +281,10 @@ class _PerSampleRoute:
             _native.check(L.dfe_heat_ps_setup(nm.handle, B, kappa.data_ptr(), self.mode, dt, mass.data_ptr(),
                                               None if load is None else load.data_ptr(), self.factors.data_ptr(),
                                               self.cf.data_ptr(), self.status.data_ptr(), ws.data_ptr(), ws.numel(), st))
+        if per_f:                                           # c_b += fl(dt F_free(f_b)), in place
+            self.sws = _src_ws(self.h, dev)
+            _src_load(self, 1, B, f, 0, f.stride(0), self.cf, self.npad, out=self.cf)
+        self.base, self.ldbase = self.cf, self.npad
 
     def check(self, who):
         bad = self.status.cpu().nonzero()                   # the one synchronisation of a forward call
@@ -244,12 +292,20 @@ class _PerSampleRoute:
             raise _native.BreakdownError(_native.ERR_BREAKDOWN, f"{who}: sample {int(bad[0, 0])}: M_L + dt K(kappa_b) is "
                                          "not positive definite (kappa_b <= 0?)")
 
-    def fwd(self, src, X, traj, steps):
+    def fwd(self, src, X, traj, steps, c=None):
+        """c: None, or (tensor, ldc_t, ldc_b): step j of sample b reads its constant at c + j ldc_t + b ldc_b"""
         st = torch.cuda.current_stream(self.dev).cuda_stream
         with _timed("heat_ps_fwd", self.dev):
-            _native.check(_native.lib().dfe_heat_ps_fwd(
-                self.h, self.B, steps, None if src is None else src.data_ptr(), traj.shape[-1], self.factors.data_ptr(),
-                self.mf.data_ptr(), self.cf.data_ptr(), X.data_ptr(), traj.data_ptr(), traj.stride(0), traj.stride(1), st))
+            if c is None:
+                _native.check(_native.lib().dfe_heat_ps_fwd(
+                    self.h, self.B, steps, None if src is None else src.data_ptr(), traj.shape[-1],
+                    self.factors.data_ptr(), self.mf.data_ptr(), self.cf.data_ptr(), X.data_ptr(), traj.data_ptr(),
+                    traj.stride(0), traj.stride(1), st))
+            else:
+                _native.check(_native.lib().dfe_heat_ps_fwd_src(
+                    self.h, self.B, steps, None if src is None else src.data_ptr(), traj.shape[-1],
+                    self.factors.data_ptr(), self.mf.data_ptr(), c[0].data_ptr(), c[1], c[2], X.data_ptr(),
+                    traj.data_ptr(), traj.stride(0), traj.stride(1), st))
 
     def begin_backward(self, N):
         self.gacc = torch.zeros((self.B, self.n_el), dtype=torch.float64, device=self.dev)   # running sums, zeroed
@@ -281,27 +337,71 @@ class _PerSampleRoute:
         pass                                                # no waits inside the per-sample kernels: nothing to check
 
 
+class _Source:
+    """A per-step source ``q``: ``(N, n)`` shared by the batch or ``(B, N, n)``.  Step n uses ``f + q[n]``: the constant of
+    a launch of steps s .. s + l - 1 is c (l, nb, npad) = fl(base_b + fl(dt F_free(q_{s+j,b}))) on the route's constant
+    without it (nb = 1 when both the source and that constant are shared by the batch)."""
+
+    def __init__(self, rt, q):
+        self.rt, self.q = rt, q
+        self.shared = q.dim() == 2
+        self.nb = 1 if self.shared and rt.ldbase == 0 else rt.B
+        if not hasattr(rt, "sws"):
+            rt.sws = _src_ws(rt.h, rt.dev)
+
+    def consts(self, s, l):
+        """(c, ldc_t, ldc_b) of the launch of steps s .. s + l - 1"""
+        rt, q, nb = self.rt, self.q, self.nb
+        qs = q[s] if self.shared else q[:, s]
+        c = _src_load(rt, l, nb, qs, q.stride(-2), 0 if self.shared else q.stride(0), rt.base, rt.ldbase)
+        return c, nb * rt.npad, rt.npad if nb > 1 else 0
+
+    def grad(self, g, s, l, lam):
+        """dL/dq at steps s .. s + l - 1 into g from lam (l, B, npad), whose slot j holds lambda_{s+1+j}: W^T (dt lam~), the
+        batch summed first (in torch's fixed order) for a shared source"""
+        rt, n = self.rt, self.q.shape[-1]
+        if self.shared:
+            ls = lam[:l].sum(1)
+            _src_grad(rt, l, 1, ls, rt.npad, 0, g[s], n, 0)
+        else:
+            _src_grad(rt, l, rt.B, lam, rt.B * rt.npad, rt.npad, g[:, s], n, g.stride(0))
+
+
+def _roll(rt, src, steps_per_launch, X, u0, traj, s, steps):
+    """steps s .. s + steps - 1 into traj[:, :steps], from u0 or (u0 None) from the carry X.  With a source the steps are
+    split into launches of at most ``steps_per_launch``: X carries the state across them exactly as across checkpoint
+    segments, so the split changes no bit."""
+    if src is None:
+        rt.fwd(u0, X, traj, steps)
+        return
+    for j in range(0, steps, steps_per_launch):
+        ln = min(steps_per_launch, steps - j)
+        rt.fwd(u0 if j == 0 else None, X, traj[:, j:], ln, src.consts(s + j, ln))
+
+
 class _HeatRollout(torch.autograd.Function):
-    """(u0 (B, n), kappa, f (n,) or None) -> the states after steps every, 2 every, ..., N: (B, N / every, n).  kappa is
-    (1,) or (n_el,) (shared by the batch) or, with ``per_sample``, (B, 1) or (B, n_el).
+    """(u0 (B, n), kappa, f (n,), (B, n) or None, source (N, n), (B, N, n) or None) -> the states after steps every,
+    2 every, ..., N: (B, N / every, n).  kappa is (1,) or (n_el,) (shared by the batch) or, with ``per_sample``, (B, 1) or
+    (B, n_el).
 
     All tensors are float64 and contiguous on the solver's device."""
 
     @staticmethod
-    def forward(ctx, u0, kappa, f, solver, n_steps: int, every: int, per_sample: bool = False):
+    def forward(ctx, u0, kappa, f, source, solver, n_steps: int, every: int, per_sample: bool = False):
         dev, mesh, dt, c = u0.device, solver.mesh, solver.dt, solver.checkpoint
         B, n, N = u0.shape[0], mesh.n_nodes, n_steps
         fd = None if f is None else f.detach()
         rt = _PerSampleRoute(mesh, kappa.detach(), dt, fd, dev, B) if per_sample \
             else _SharedRoute(mesh, kappa.detach(), dt, fd, dev, B, solver._cta_warps)
+        src = None if source is None else _Source(rt, source.detach())
         X = torch.zeros((B, rt.npad), dtype=torch.float64, device=dev)
 
-        def roll(src, traj, steps):
-            rt.fwd(src, X, traj, steps)
+        def roll(u_start, traj, s, steps):
+            _roll(rt, src, solver._src_steps, X, u_start, traj, s, steps)
 
         if c is None:                                       # every state kept: the trajectory is the saved state
             traj = torch.empty((B, N, n), dtype=torch.float64, device=dev)
-            roll(u0, traj, N)
+            roll(u0, traj, 0, N)
             out = traj if every == 1 else traj[:, every - 1::every].contiguous()
             saved = traj
         else:                                               # segments of c steps; only their first states are kept
@@ -310,7 +410,7 @@ class _HeatRollout(torch.autograd.Function):
             starts = [u0]
             for s in range(0, N, c):
                 ln = min(c, N - s)
-                roll(u0 if s == 0 else None, seg, ln)       # later segments continue from the carry X
+                roll(u0 if s == 0 else None, seg, s, ln)    # later segments continue from the carry X
                 first = (s // every + 1) * every            # first recorded step after s
                 if first <= s + ln:
                     out[:, first // every - 1:(s + ln) // every] = seg[:, first - s - 1:ln:every]
@@ -318,8 +418,9 @@ class _HeatRollout(torch.autograd.Function):
                     starts.append(seg[:, ln - 1].clone())
             saved = torch.stack(starts)
         rt.check("DifferentiableHeatSolver")
-        ctx.rt, ctx.solver, ctx.N, ctx.every = rt, solver, N, every
+        ctx.rt, ctx.src, ctx.solver, ctx.N, ctx.every = rt, src, solver, N, every
         ctx.need_f = f is not None
+        ctx.per_f = f is not None and f.dim() == 2
         ctx.save_for_backward(saved, kappa)
         return out
 
@@ -327,7 +428,7 @@ class _HeatRollout(torch.autograd.Function):
     def backward(ctx, gout):
         L = _native.lib()
         saved, kappa = ctx.saved_tensors
-        rt, solver, N, every = ctx.rt, ctx.solver, ctx.N, ctx.every
+        rt, src, solver, N, every = ctx.rt, ctx.src, ctx.solver, ctx.N, ctx.every
         mesh, dt, c = solver.mesh, solver.dt, solver.checkpoint
         dev = saved.device
         h, npad, nf, n = rt.h, rt.npad, rt.free.numel(), mesh.n_nodes
@@ -338,6 +439,9 @@ class _HeatRollout(torch.autograd.Function):
         lsum = torch.zeros((B, npad), dtype=torch.float64, device=dev)
         rt.begin_backward(N)
 
+        gsrc = None if src is None or not ctx.needs_input_grad[3] else \
+            torch.empty(src.q.shape, dtype=torch.float64, device=dev)
+
         def adjoint(n0, ln, lam):
             rt.adj(n0, ln, gout, every, Xa, lam, lsum)
 
@@ -345,6 +449,8 @@ class _HeatRollout(torch.autograd.Function):
             lam = torch.empty((N, B, npad), dtype=torch.float64, device=dev)
             adjoint(0, N, lam)
             rt.grad(0, N, saved, lam)
+            if gsrc is not None:
+                src.grad(gsrc, 0, N, lam)
         else:
             Xs = torch.empty((B, npad), dtype=torch.float64, device=dev)
             seg = torch.empty((B, min(c, N), n), dtype=torch.float64, device=dev)
@@ -352,14 +458,20 @@ class _HeatRollout(torch.autograd.Function):
             for i in reversed(range(saved.shape[0])):
                 s = i * c
                 ln = min(c, N - s)
-                rt.fwd(saved[i], Xs, seg, ln)               # recompute the segment's states from its first one
+                # recompute the segment's states from its first one
+                _roll(rt, src, solver._src_steps, Xs, saved[i], seg, s, ln)
                 adjoint(s, ln, lam)
                 rt.grad(s, ln, seg, lam)
+                if gsrc is not None:
+                    src.grad(gsrc, s, ln, lam)
         gk = rt.gkappa(kappa)
         gu0 = torch.zeros((B, n), dtype=torch.float64, device=dev)
         gu0[:, rt.free] = rt.mass_free * Xa[:, :nf]          # dL/du0[free] = m * lambda_1
         gf = None
-        if ctx.need_f:                                      # dL/df = W^T (dt sum_n sum_b lam~_n)
+        if ctx.need_f and ctx.per_f:                        # dL/df_b = W^T (dt sum_n lam~_{n,b})
+            gf = torch.empty((B, n), dtype=torch.float64, device=dev)
+            _src_grad(rt, 1, B, lsum, 0, npad, gf, 0, n)
+        elif ctx.need_f:                                    # dL/df = W^T (dt sum_n sum_b lam~_n)
             lt = torch.zeros(n, dtype=torch.float64, device=dev)
             lt[rt.free] = dt * lsum[:, :nf].sum(0)
             gf = torch.empty(n, dtype=torch.float64, device=dev)
@@ -369,7 +481,7 @@ class _HeatRollout(torch.autograd.Function):
                 _native.check(L.dfe_grad(h, lt.data_ptr(), lt.data_ptr(), kg.data_ptr(), _native.KAPPA_PER_ELEMENT,
                                          scratch.data_ptr(), gf.data_ptr(), None, 0, st))
         rt.finish_backward("DifferentiableHeatSolver.backward")
-        return gu0, gk.reshape(kappa.shape), gf, None, None, None, None
+        return gu0, gk.reshape(kappa.shape), gf, gsrc, None, None, None, None
 
 
 class DifferentiableHeatSolver(nn.Module):
@@ -377,9 +489,11 @@ class DifferentiableHeatSolver(nn.Module):
 
         (M_L + dt K(kappa)) u^{n+1} = M_L u^n + dt F(f),   Dirichlet nodes held at the mesh's values.
 
-    ``solver(u0, n_steps, every=None)`` returns the final state (``every=None``) or the states after steps ``every,
-    2 every, ..., n_steps`` as ``(B, n_steps // every, n_nodes)``; gradients flow to ``u0``, ``kappa`` and ``f`` through the
-    discrete adjoint.  Each call assembles ``K(kappa)``, factors ``M_L + dt K`` once and synchronises once (a failed
+    ``solver(u0, n_steps, every=None, *, source=None)`` returns the final state (``every=None``) or the states after steps
+    ``every, 2 every, ..., n_steps`` as ``(B, n_steps // every, n_nodes)``; gradients flow to ``u0``, ``kappa``, ``f`` and
+    ``source`` through the discrete adjoint.  ``source`` is ``(n_steps, n_nodes)`` (one source per step, shared by the
+    batch) or ``(B, n_steps, n_nodes)`` (per step and per sample, with ``u0`` of shape ``(B, n_nodes)``); step n (0-based,
+    u^n -> u^{n+1}) uses ``f + source[n]``, the backward-Euler evaluation of the source at t_{n+1}.  Each call assembles ``K(kappa)``, factors ``M_L + dt K`` once and synchronises once (a failed
     factorisation, e.g. ``kappa <= 0``, raises ``BreakdownError``).
 
     Parameters
@@ -395,7 +509,9 @@ class DifferentiableHeatSolver(nn.Module):
         raises ``BreakdownError`` naming the first such sample.  The trajectory and lambda buffers are those of the
         shared route.
     dt : float            not differentiable
-    f : None or ``(n_nodes,)`` source, shared by the batch, differentiable
+    f : None, ``(n_nodes,)`` (shared by the batch) or ``(B, n_nodes)`` (one per sample, with ``u0`` of shape
+        ``(B, n_nodes)``): a source constant in time, differentiable; ``f.grad`` has ``f``'s shape.  A per-step source goes
+        to the call (``source``).
     checkpoint : keyword-only, None (keep every state for the backward) or c: keep every c-th state and recompute each
         segment of c steps in the backward.  Gradients are bit-identical either way.
 
@@ -405,6 +521,10 @@ class DifferentiableHeatSolver(nn.Module):
 
     # warps per CTA of the rollout kernels; 0 lets the library choose from the batch size (results do not depend on it)
     _cta_warps = 0
+    # Steps per rollout launch with a per-step source (results do not depend on it).  A launch's constants take
+    # (steps, B, npad) doubles: 16 steps keep them at 16 carries (0.5 GB at B = 4096 on rectangle(32, 32)) against the
+    # (B, N, n_nodes) trajectory, while the launches it adds (one load kernel and one rollout per 16 steps) stay few.
+    _src_steps = 16
 
     def __init__(self, mesh: FEMesh, kappa, dt: float, f: torch.Tensor | None = None, *, checkpoint: int | None = None):
         super().__init__()
@@ -420,7 +540,8 @@ class DifferentiableHeatSolver(nn.Module):
         self.kappa = torch.tensor(float(kappa), dtype=torch.float64) if isinstance(kappa, (int, float)) else kappa
         self.f = f
 
-    def forward(self, u0: torch.Tensor, n_steps: int, every: int | None = None) -> torch.Tensor:
+    def forward(self, u0: torch.Tensor, n_steps: int, every: int | None = None, *,
+                source: torch.Tensor | None = None) -> torch.Tensor:
         mesh = self.mesh
         n_steps = int(n_steps)
         if n_steps < 1:
@@ -442,15 +563,21 @@ class DifferentiableHeatSolver(nn.Module):
                 else self.kappa.to(dtype=torch.float64).reshape(-1)
             if kap.numel() not in (1, mesh.n_elements):
                 raise ValueError(f"kappa must have 1 or n_elements={mesh.n_elements} entries, got {kap.numel()}")
-        if self.f is not None and tuple(self.f.shape) != (mesh.n_nodes,):
-            raise ValueError(f"f must have shape ({mesh.n_nodes},), got {tuple(self.f.shape)}")
+        n, Bu = mesh.n_nodes, (u0.shape[0] if u0.dim() == 2 else None)
+        if self.f is not None and tuple(self.f.shape) not in ((n,), (Bu, n)):
+            raise ValueError(f"f must have shape ({n},) or (B, {n}) with u0 of shape (B, n_nodes); got f "
+                             f"{tuple(self.f.shape)} and u0 {tuple(u0.shape)}")
+        if source is not None and tuple(source.shape) not in ((n_steps, n), (Bu, n_steps, n)):
+            raise ValueError(f"source must have shape (n_steps, n_nodes) = ({n_steps}, {n}) or (B, n_steps, n_nodes) with "
+                             f"u0 of shape (B, n_nodes); got source {tuple(source.shape)} and u0 {tuple(u0.shape)}")
         dev = u0.device if u0.is_cuda else torch.device("cuda", torch.cuda.current_device())
         _heat_check_mesh(mesh, dev, per_sample=per_sample)
         batched = u0.dim() == 2
         u = u0.to(device=dev, dtype=torch.float64).reshape(-1, mesh.n_nodes).contiguous()
         fd = None if self.f is None else self.f.to(device=dev, dtype=torch.float64).contiguous()
+        sd = None if source is None else source.to(device=dev, dtype=torch.float64).contiguous()
         with torch.cuda.device(dev):
-            U = _HeatRollout.apply(u, kap.to(dev).contiguous(), fd, self, n_steps, k, per_sample)
+            U = _HeatRollout.apply(u, kap.to(dev).contiguous(), fd, sd, self, n_steps, k, per_sample)
         if every is None:
             U = U[:, 0]
         if not batched:

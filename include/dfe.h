@@ -363,6 +363,43 @@ int dfe_heat_ps_grad(const dfe_mesh* m, int64_t B, int64_t n_seg, const void* fa
 int dfe_heat_ps_grad_sum(const dfe_mesh* m, int64_t B, double dt, int kappa_mode, const double* gacc, double* gkappa,
                          void* stream);
 
+/* ---------------------------------------------------------------- heat-equation rollouts with sources in time and per sample
+ * The rollouts above with a constant term per step and per sample.  Step j of a launch (u^n -> u^{n+1}) for sample b, in
+ * free numbering:
+ *   A_ff x_{n+1} = m * x_n + c_{j,b},   c_{j,b} = fl(c_base_b + fl(dt * F_free(q_{j,b})))
+ * F_free: the reference's load vector (per element fl(fl(area / 3) * fl(((q_i + q_j) + q_k) / 3)), added in ascending
+ * element order: the bits of dfe_assemble's F).  c_base is the route's constant without this source (c_free of
+ * _HeatOperator / dfe_heat_ps_setup, or a per-sample c_b formed by dfe_heat_src_load itself).  Meshes: dfe_band_ps_supported,
+ * and the element terms plus four input rows in 200 KB of shared memory (else DFE_ERR_UNSUPPORTED).
+ *   dfe_heat_src_workspace_bytes  ws of the two source kernels: 48 bytes per element (their per-element tables, rebuilt by
+ *                                 every call)
+ *   dfe_heat_src_load   c (n_steps, nb, npad), zero beyond n_free: row (j, b) from q at q + j * ldq_t + b * ldq_b (node
+ *                       layout, n_nodes) and c_base + b * ldbase (npad; ldbase 0: one base for every row).  c may equal
+ *                       c_base when n_steps = 1 and ldbase = npad (in place).
+ *   dfe_heat_fwd_src    dfe_heat_fwd, with step j of sample b reading c at c + j * ldc_t + b * ldc_b (npad; strides even
+ *                       and >= 0, c 16-byte aligned).  ldc_b = 0: one row for the batch; ldc_t = 0: constant in time.
+ *   dfe_heat_ps_fwd_src dfe_heat_ps_fwd, with c read as for dfe_heat_fwd_src.
+ *   dfe_heat_src_grad   g row (j, b) at g + j * ldg_t + b * ldg_b (node layout, n_nodes) = W^T (dt * lam~), lam~ the row at
+ *                       lam + j * ldl_t + b * ldl_b (free layout, npad) scattered with zeros on the Dirichlet nodes:
+ *                       g_p = sum_{e∋p} area_e / 9 * ((l_i + l_j) + l_k), l = dt * lam~ (dfe_grad's gf).  With lam slot
+ *                       j of dfe_heat_adj (lambda_{n0+1+j}) this is dL/dq at step n0 + j; with lam_sum it is dL/df_b of a
+ *                       per-sample constant source.  Non-zero on Dirichlet nodes in general.
+ * The Dirichlet and source-free behaviour is that of the calls above.  Offsets are 64-bit.  All calls are asynchronous on
+ * `stream`; a host-only handle gives DFE_ERR_CUDA and a null handle DFE_ERR_INVALID.
+ */
+size_t dfe_heat_src_workspace_bytes(const dfe_mesh* m);
+int dfe_heat_src_load(const dfe_mesh* m, int64_t n_steps, int64_t nb, double dt, const double* q, int64_t ldq_t,
+                      int64_t ldq_b, const double* c_base, int64_t ldbase, double* c, void* ws, size_t ws_bytes,
+                      void* stream);
+int dfe_heat_fwd_src(const dfe_mesh* m, int64_t B, int64_t n_steps, const double* u0, int64_t ldu0, const void* factor,
+                     const double* m_free, const double* c, int64_t ldc_t, int64_t ldc_b, double* X, double* traj,
+                     int64_t ld_b, int64_t ld_t, int warps, int32_t* fault, void* stream);
+int dfe_heat_ps_fwd_src(const dfe_mesh* m, int64_t B, int64_t n_steps, const double* u0, int64_t ldu0, const void* factors,
+                        const double* m_free, const double* c, int64_t ldc_t, int64_t ldc_b, double* X, double* traj,
+                        int64_t ld_b, int64_t ld_t, void* stream);
+int dfe_heat_src_grad(const dfe_mesh* m, int64_t n_steps, int64_t nb, double dt, const double* lam, int64_t ldl_t,
+                      int64_t ldl_b, double* g, int64_t ldg_t, int64_t ldg_b, void* ws, size_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
